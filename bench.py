@@ -2,12 +2,13 @@
 """Benchmark of the pattern-partition DP on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config auto|cfg3|cfg4|cfg5|n9m]
+                  [--dump-outputs DIR]
 
 --config auto (default):
   N = 1  : BASELINE config 3 — one full 9-mer DP (`NNNNANNNN`, 2 562 890 625 patterns) + backtrack.
            A step = count expansion (K2) + wave-front DP with fused scoring (K3+K4) + backtrack (K5), k-mer count
            tables already resident in HBM.  metric = pattern-scores/sec.  The same line carries, under `cv_grid`, the
-           45-job CV grid of config 4 on this one GPU (>= 5 timed steps): the N = 1 point of the N > 1 curve.
+           45-job CV grid of config 4 on this one GPU: the N = 1 point of the N > 1 curve.
   N > 1  : BASELINE config 4 — the 3x3 (alpha, penalty) grid x 5 folds = 45 single-fold DP jobs of the same size, dealt to
            the ranks by job, one all_gather (NCCL) of the per-job losses.  A step = fold count expansion + this rank's
            jobs + gather + selection, held-out fold tables already sampled.  metric = pattern-scores/sec over all jobs
@@ -24,7 +25,17 @@ Results are checked, not just timed: loss, partition and per-job CV losses are c
 (the oracle's full-size run) and the line carries "parity_checked".  A mismatch aborts the benchmark.
 
 Prints ONE JSON line on rank 0.  Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max
-over ranks.  Tables (>= 4 GB) are far larger than the 126 MB L2, so no explicit flush.
+over ranks.  Every GPU measurement of the line runs W warm-up steps, then K timed steps.  Tables (>= 4 GB) are far
+larger than the 126 MB L2, so no explicit flush.
+
+--dump-outputs DIR: after the timed steps rank 0 writes what the last timed step of each GPU measurement returned, as
+DIR/<name>.npy (float32 or float64), so that two builds can be compared output for output; the inputs are seeded and
+identical from run to run.  Single DP: loss (float32), partition (its pattern numbers, float64, exact below 2^53).
+CV grid: cv_losses (float32 [1, folds, alphas, penalties, (train, held-out)]), cv_selected (float64 [alpha, penalty,
+held-out loss]).  Sharded DP (N > 1): sharded_loss, sharded_partition.  A partition has at most one pattern per k-mer,
+so all of it stays far below 64 MB and is written whole.
+
+The benchmark compiles nothing and writes nothing into the tree: it loads the libraries __graft_entry__.build() made.
 """
 import argparse
 import hashlib
@@ -317,9 +328,6 @@ def run_reference(args, emit):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    from oracle import kp_oracle as O
-
-    O.build()
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     name = args.config if args.config != "auto" else ("cfg3" if world == 1 else "cfg4")
     threads = host_threads()
@@ -457,7 +465,7 @@ def bench_single(args, name, rank, world, local):
                 "d2h_bytes_per_step": int(4 + 8 * len(patnums) + 16)},
         "gpu_launches": int(launches), "clocks": clocks,
     }
-    return line
+    return line, {"loss": np.array([loss], dtype=np.float32), "partition": patnums.astype(np.float64)}
 
 
 def check_cv_against_golden(res, best):
@@ -478,15 +486,14 @@ def check_cv_against_golden(res, best):
     return out
 
 
-def bench_cv(args, rank, world, local, steps=None, warmup=None):
+def bench_cv(args, rank, world, local):
     import torch
 
     from kmerpapa_b200 import CV_tools, synthetic
     from kmerpapa_b200.algorithms import bottum_up_array_penalty_plus_pseudo_CV as cv
     from kmerpapa_b200.engine import get_plan
 
-    steps = args.steps if steps is None else steps
-    warmup = args.warmup if warmup is None else warmup
+    steps, warmup = args.steps, args.warmup
     dev = torch.device("cuda", local)
     kmers, pos, neg = synthetic.negbin_counts(CV_GEN_PAT, CV_DATA_SEED)
     codes = synthetic.codes_of(kmers)
@@ -529,12 +536,14 @@ def bench_cv(args, rank, world, local, steps=None, warmup=None):
            "selected": [best[0], best[1], float(best[2])], "parity_checked": bool(parity["checked"]), "parity": parity,
            "launches": int(launches), "clocks": clocks, "achieved_gbs_per_gpu": achieved, "frac_per_gpu": achieved / peak,
            "peak": peak, "peak_kind": peak_kind}
-    return out
+    return out, {"cv_losses": np.asarray(res, dtype=np.float32),
+                 "cv_selected": np.array([best[0], best[1], best[2]], dtype=np.float64)}
 
 
-def bench_sharded_dp(rank, world, local, reps=6):
+def bench_sharded_dp(args, rank, world, local):
     """Secondary N>1 measurement: ONE 9-mer DP (config 3) sharded over the ranks (kmerpapa_b200/sharded.py, replicated
-    mode: rows pushed to their readers over NVLink inside the DP kernel).  Device time, max over ranks, best of reps."""
+    mode: rows pushed to their readers over NVLink inside the DP kernel).  Device time, max over ranks, best of the
+    timed steps."""
     import torch
     import torch.distributed as dist
 
@@ -552,7 +561,7 @@ def bench_sharded_dp(rank, world, local, reps=6):
     sh = sharded.ShardedDP(plan, rank, world, replicate=True)
     sh.connect()
     ms = []
-    for _ in range(reps):
+    for _ in range(args.warmup + args.steps):
         sh.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -567,10 +576,12 @@ def bench_sharded_dp(rank, world, local, reps=6):
     top = float(sh.top_score())
     parity = check_single_against_golden("cfg3", np.float32(top), part)
     sh.close()
-    best = min(ms[1:])
-    return {"workload": "cfg3 single 9-mer DP sharded by the top high digit, replicated mode", "ms": best,
-            "pattern_scores_per_s": plan.npat / (best / 1e3), "partition_patterns": int(len(part)), "loss": top,
-            "parity_checked": bool(parity["checked"]), "reps_ms": [round(x, 3) for x in ms]}
+    ms = ms[args.warmup:]
+    best = min(ms)
+    return ({"workload": "cfg3 single 9-mer DP sharded by the top high digit, replicated mode", "ms": best,
+             "pattern_scores_per_s": plan.npat / (best / 1e3), "partition_patterns": int(len(part)), "loss": top,
+             "parity_checked": bool(parity["checked"]), "reps_ms": [round(x, 3) for x in ms]},
+            {"sharded_loss": np.array([top], dtype=np.float32), "sharded_partition": part.astype(np.float64)})
 
 
 def main():
@@ -580,12 +591,17 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="auto", choices=["auto", "cfg3", "cfg4", "cfg5", "n9m"])
-    ap.add_argument("--cv-steps", type=int, default=5, help="N=1: timed steps of the secondary CV-grid measurement")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-numba", action="store_true", help="skip the timing of the unmodified numba reference (about a minute)")
     ap.add_argument("--no-cv", action="store_true", help="N=1: skip the secondary CV-grid measurement")
     ap.add_argument("--no-sharded", action="store_true", help="N>1: skip the secondary sharded single-DP measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of each GPU measurement to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     # stdout carries exactly one JSON line: everything else that writes to file descriptor 1 (the NCCL banner,
     # stray prints of libraries) is sent to stderr for the duration of the run
     sys.stdout.flush()
@@ -598,21 +614,17 @@ def main():
     if args.impl == "reference":
         run_reference(args, emit)
         return
-    import __graft_entry__ as ge
-
     rank, world, local = dist_setup(args.gpus)
-    if rank == 0:
-        ge.build()
-    barrier_sync(world)
     name = args.config if args.config != "auto" else ("cfg3" if world == 1 else "cfg4")
     if name != "cfg4":
-        line = bench_single(args, name, rank, world, local)
+        line, outputs = bench_single(args, name, rank, world, local)
         if world == 1 and name == "cfg3" and not args.no_cv:
-            line["cv_grid"] = bench_cv(args, rank, world, local, steps=max(5, args.cv_steps), warmup=2)
+            line["cv_grid"], cv_outputs = bench_cv(args, rank, world, local)
             line["cv_grid"]["note"] = ("config 4 on this one GPU: the N = 1 point of the strong-scaling curve whose N > 1 points are "
                                        "the `value` of `bench.py --gpus N`")
+            outputs.update(cv_outputs)
     else:
-        cvres = bench_cv(args, rank, world, local)
+        cvres, outputs = bench_cv(args, rank, world, local)
         traffic, capture = load_traffic("cfg4_cv_job")
         line = {
             "metric": "pattern-scores/sec", "value": cvres["pattern_scores_per_s"], "unit": "patterns/s", "n_gpus": world,
@@ -631,11 +643,13 @@ def main():
             "cv_grid": cvres, "gpu_launches": cvres["launches"], "clocks": cvres["clocks"],
         }
         if not args.no_sharded and 1 < world <= 8:
-            line["sharded_single_dp"] = bench_sharded_dp(rank, world, local)
+            line["sharded_single_dp"], sharded_outputs = bench_sharded_dp(args, rank, world, local)
+            outputs.update(sharded_outputs)
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, key + ".npy"), arr)
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
-        from oracle import kp_oracle as O
-
-        O.build()
         threads = host_threads()
         r = cpu_single_sample(name, threads) if name != "cfg4" else cpu_cv_sample(threads)
         line["cpu_baseline"] = {

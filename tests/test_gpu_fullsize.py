@@ -254,3 +254,23 @@ def test_full_size_cv_job_matches_single_dp_on_train_counts():
     fM, fU = plan.expand(zM, zU, name="fs_fold_e")
     tr0, te0 = plan.cv_job(eM, eU, fM, fU, mc, 1.0, beta, 6.0)
     assert te0 == 0.0
+
+
+def test_bench_dump_outputs_reproduce_the_oracle_golden(tmp_path):
+    """bench.py --dump-outputs on config 5: the dumped loss and partition of the last timed step are the oracle's."""
+    import subprocess
+    import sys
+
+    from conftest import ROOT, free_gpu_memory
+
+    g = _golden("cfg5")
+    free_gpu_memory()   # the benchmark runs in a child process and needs its own tables
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "cfg5", "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout)["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["loss.npy", "partition.npy"]
+    loss, part = np.load(tmp_path / "loss.npy"), np.load(tmp_path / "partition.npy")
+    assert loss.dtype == np.float32 and loss.shape == (1,) and int(loss.view(np.uint32)[0]) == int(g["loss_bits"], 16)
+    assert part.dtype == np.float64 and len(part) == g["partition_patterns"]
+    assert hashlib.sha256(part.astype("<u8").tobytes()).hexdigest() == g["partition_sha256"]

@@ -372,3 +372,20 @@ def test_lattice_free_plan(eng):
     assert Mp.sum() == M.sum() and Up.sum() == U.sum()
     assert all(nm[0] != "N" for nm in names) and len(names) < 200      # the signal sits in position 0: it is always split
 
+
+def test_7mer_matches_the_recorded_numba_reference():
+    """bench.py's comparison with the unmodified numba reference (NNNMNNN, 34 M patterns), against that reference's
+    recorded result: same loss bits and the same partition, name for name."""
+    import importlib.util
+    import json
+    import os
+
+    from conftest import ROOT
+
+    nb = json.load(open(os.path.join(GOLDEN, "numba_NNNMNNN.json")))
+    spec = importlib.util.spec_from_file_location("kp_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert (bench.NUMBA_GEN_PAT, bench.NUMBA_SEED, bench.NUMBA_ALPHA, bench.NUMBA_PENALTY) == (
+        nb["gen_pat"], nb["seed"], nb["alpha"], nb["penalty"])
+    assert bench.gpu_matches_numba(nb, 0)
