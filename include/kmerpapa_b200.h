@@ -65,7 +65,7 @@ typedef struct kp_plan_info {
 } kp_plan_info;
 
 /* Return codes.  KP_ERR_CAPACITY: the workspace `cap` the caller passed was too small for the result (kp_backtrack,
- * kp_cv_heldout, kp_dp_cv_job, kp_shard_backtrack, kp_greedy): call again with a larger one.  Everything else is KP_ERR. */
+ * kp_cv_heldout, kp_dp_cv_job, kp_shard_backtrack, kp_shard_cv_heldout, kp_greedy): call again with a larger one.  Everything else is KP_ERR. */
 #define KP_OK 0
 #define KP_ERR 1
 #define KP_ERR_CAPACITY 2
@@ -194,7 +194,8 @@ const char *kp_dp_kernel_name(const kp_plan *plan);
  *
  *   kp_shard_create -> exchange pointers (kp_ipc_export / all_gather / kp_ipc_open, or directly within one
  *   process) -> kp_shard_set_peer for every other rank -> for wave in 0..nwaves-1: kp_shard_dp_wave, barrier ->
- *   kp_shard_backtrack / kp_shard_gather on any rank.
+ *   kp_shard_backtrack / kp_shard_gather on any rank.  A cross-validation job: kp_shard_cv_wave instead of
+ *   kp_shard_dp_wave, then kp_shard_cv_heldout on any rank.
  * ------------------------------------------------------------------------------------------------- */
 typedef struct kp_shard kp_shard;
 
@@ -230,6 +231,15 @@ int kp_ipc_close(int device, void *d_ptr);
  * All ranks must have finished wave w-1 before any rank starts wave w. */
 int kp_shard_dp_wave(kp_shard *shard, int wave, const int64_t *d_expM, const int64_t *d_expU, uint64_t max_count,
                      double alpha, double beta, double penalty, void *stream);
+/* kp_shard_dp_wave on train counts d_exp?tot - d_exp?test (one CV job, one wave); same rules as kp_shard_dp_wave */
+int kp_shard_cv_wave(kp_shard *shard, int wave, const int64_t *d_expMtot, const int64_t *d_expUtot,
+                     const int64_t *d_expMtest, const int64_t *d_expUtest, uint64_t max_count,
+                     double alpha, double beta_fold, double penalty, void *stream);
+/* after the last kp_shard_cv_wave on every rank: h_top[0] = train loss of `root`, h_top[1] = held-out loss of the
+ * best partition of `root` (kp_cv_heldout's definition), read through the shard view.  Synchronises. */
+int kp_shard_cv_heldout(kp_shard *shard, const int64_t *d_expMtot, const int64_t *d_expUtot, const int64_t *d_expMtest,
+                        const int64_t *d_expUtest, double alpha, double beta_fold, double penalty, uint64_t root,
+                        void *d_ws, uint64_t cap, float *h_top, void *stream);
 /* like kp_backtrack, over all shards (reads peers' memory); callable on any rank after the last wave */
 int kp_shard_backtrack(kp_shard *shard, void *d_ws, uint64_t cap, uint64_t root, uint64_t *h_patnums, uint64_t *n_out,
                        void *stream);

@@ -72,7 +72,9 @@ SYMBOLS = {
     "kp_ipc_open": (_int, [_int, _vp, ctypes.POINTER(_vp)]),
     "kp_ipc_close": (_int, [_int, _vp]),
     "kp_shard_dp_wave": (_int, [_vp, _int, _vp, _vp, _u64, _dbl, _dbl, _dbl, _vp]),
-    "kp_shard_backtrack": (_int, [_vp, _vp, _u64, _u64, _vp, ctypes.POINTER(_u64), _vp]),
+    "kp_shard_cv_wave": (_int, [_vp, _int, _vp, _vp, _vp, _vp, _u64, _dbl, _dbl, _dbl, _vp]),
+    "kp_shard_cv_heldout": (_int, [_vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _u64, _vp, _u64, _vp, _vp]),
+    "kp_shard_backtrack":(_int, [_vp, _vp, _u64, _u64, _vp, ctypes.POINTER(_u64), _vp]),
     "kp_shard_gather": (_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp]),
     "kp_greedy_ws_bytes": (_u64, [_u64]),
     "kp_greedy": (_int, [_vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _vp, _u64, _vp, _vp, _vp, ctypes.POINTER(_u64),

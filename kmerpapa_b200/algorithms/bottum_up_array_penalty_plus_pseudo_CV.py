@@ -10,6 +10,8 @@ and runs as an independent single-fold DP on the GPU (kp_dp_cv_job), with train 
 device as total - held-out.  Jobs are dealt to the ranks of torch.distributed (one process per GPU)
 in contiguous fold-major chunks and the per-job (train, held-out) losses of the general pattern are
 all-gathered (NCCL on GPUs); every rank then does the reference's float32 fold sum and selection.
+A general pattern whose CV tables do not fit one GPU is cross-validated with every job as one DP sharded over all
+ranks instead (ShardedFoldRunner, chosen by sharded_cv_runner).
 """
 import sys
 
@@ -173,6 +175,131 @@ class GpuFoldRunner:
         return self.plan.device
 
 
+class ShardedFoldRunner:
+    """GpuFoldRunner's run / begin_folds / set_fold / set_folds over ONE capacity-mode DP sharded over several shards, for a
+    general pattern whose CV tables do not fit one GPU: every job is a sharded CV job (ShardedDP.cv_job).  It is a
+    collective runner: every rank runs every job, so run_grid neither deals the jobs to the ranks nor gathers them.
+    It keeps the expanded held-out tables of one fold only (the jobs are fold-major: each fold is expanded once) and has
+    no pipelined interface.  `shards`: this process's connected shards, either one per rank of the NCCL group (connect())
+    or all shards of the DP in this process (connect_local(), see local())."""
+
+    collective = True
+
+    def __init__(self, shards, codes, pos, neg):
+        self.shards = list(shards)
+        self.plan = self.shards[0].plan
+        self.codes = codes
+        self.max_count = int(pos.sum()) + int(neg.sum())
+        kM, kU = self.plan.pack_counts(codes, pos, neg, name="cvtot_k")
+        self.tot = self.plan.expand(kM, kU, name="cvtot_e")
+        self.fold = None   # (f, expanded M, expanded U) of the resident fold
+
+    @classmethod
+    def local(cls, gen_pat, codes, pos, neg, world, device=None):
+        """`world` in-process shards on one GPU (the sharded CV without a process group)."""
+        from .. import sharded
+        from ..engine import get_plan
+
+        plan = get_plan(gen_pat, device)
+        shards = []
+        try:
+            for r in range(world):
+                shards.append(sharded.ShardedDP(plan, r, world, replicate=False))
+            for s in shards:
+                s.connect_local(shards)
+            return cls(shards, codes, pos, neg)
+        except BaseException:
+            for s in shards:
+                s.close()
+            raise
+
+    def set_folds(self, Mf, Uf):
+        self.Mf, self.Uf = Mf, Uf
+        self.fold = None
+
+    def begin_folds(self, nkmer, nfolds):
+        self.Mf = np.zeros((nkmer, nfolds), dtype=np.uint64)
+        self.Uf = np.zeros((nkmer, nfolds), dtype=np.uint64)
+        self.fold = None
+
+    def set_fold(self, f, M, U):
+        self.Mf[:, f], self.Uf[:, f] = M, U
+
+    def run(self, f, alpha, beta, penalty):
+        if self.fold is None or self.fold[0] != f:
+            err = None
+            try:
+                kM, kU = self.plan.pack_counts(self.codes, self.Mf[:, f], self.Uf[:, f], name="cvfold_k")
+                self.fold = (f,) + self.plan.expand(kM, kU, name="cvfold_e")
+            except Exception as e:   # noqa: BLE001 - raised on every rank by agree()
+                err = e
+            self.shards[0].agree(err, "ShardedFoldRunner: held-out tables")
+        return self.shards[0].cv_job(self.tot[0], self.tot[1], self.fold[1], self.fold[2], self.max_count, alpha, beta,
+                                     penalty)
+
+    def close(self):
+        """Release the shards (collective with peers in other processes: every rank calls it) and the CV buffers."""
+        self.fold = self.tot = None
+        for s in self.shards:
+            s.close()
+        self.shards = []
+        self.plan.release_buffers(prefix="cv")
+
+    @property
+    def device(self):
+        return self.plan.device
+
+
+def sharded_cv_runner(gen_pat, codes, pos, neg, nfolds):
+    """A ShardedFoldRunner over the ranks of the NCCL group when the CV tables GpuFoldRunner would allocate do not fit
+    one rank's GPU (or KP_SHARD_CV=1 asks for it) and every rank can hold its shard; else None: the jobs are dealt to
+    the ranks as usual.  The ranks agree on every decision through an all_reduce."""
+    import os
+
+    from .bottum_up_array_w_numba import _world, cv_buffer_bytes, fits_free_memory
+
+    rank, world = _world()
+    if world == 1:
+        return None
+    import torch
+    import torch.distributed as dist
+
+    from .. import sharded
+    from .._native import KpError
+    from ..engine import get_plan
+
+    plan = get_plan(gen_pat)
+    forced = os.environ.get("KP_SHARD_CV") == "1"
+    fits = torch.tensor([0 if forced else int(fits_free_memory(plan, cv_buffer_bytes(plan, nfolds), ("cv",)))],
+                        dtype=torch.int32, device=plan.device)
+    dist.all_reduce(fits, op=dist.ReduceOp.MIN)   # shard as soon as ONE rank cannot hold the CV
+    if int(fits.item()) == 1:
+        return None
+    torch.cuda.empty_cache()   # the shards are plain cudaMalloc allocations (CUDA IPC): give them torch's cached blocks
+    try:
+        sh = sharded.ShardedDP(plan, rank, world, replicate=False)
+    except KpError:
+        sh = None
+    ok = torch.tensor([0 if sh is None else 1], dtype=torch.int32, device=plan.device)
+    dist.all_reduce(ok, op=dist.ReduceOp.MIN)     # all ranks shard, or none does
+    if int(ok.item()) == 0:
+        if sh is not None:
+            sh.close()
+        return None
+    runner = err = None
+    try:
+        sh.connect()   # raises on every rank when one rank cannot map its peers
+        try:
+            runner = ShardedFoldRunner([sh], codes, pos, neg)
+        except Exception as e:   # noqa: BLE001 - e.g. no memory left for the count tables on this rank; raised by agree()
+            err = e
+        sh.agree(err, "ShardedFoldRunner")
+    except BaseException:
+        sh.close()     # collective: every rank is here
+        raise
+    return runner
+
+
 def run_grid(gen_pat, kmers, codes, pos, neg, alphas, penalties, nfolds, nit, seed, verbosity=0, runner=None,
              gather_device="auto", presampled=None, progress=None):
     """Core of the CV: returns float32 results [nit, nfolds, n_alpha, n_penalty, 2] (train, held-out).
@@ -180,6 +307,8 @@ def run_grid(gen_pat, kmers, codes, pos, neg, alphas, penalties, nfolds, nit, se
     progress(it, results_of_iteration): called once per iteration, in order — right after the iteration's jobs in
     a single process (the reference's interleaving of its stderr lines), after the gather when the jobs are sharded."""
     rank, world = dist_info()
+    if getattr(runner, "collective", False):   # every rank runs every job (one DP over all ranks): nothing to deal or gather
+        rank, world = 0, 1
     prng = np.random.RandomState(seed)
     if runner is None:
         runner = GpuFoldRunner(gen_pat, codes, pos, neg)
@@ -311,6 +440,12 @@ def pattern_partition_bottom_up(gen_pat, contextD, alphas, args, nmut, nunmut, p
                     if verbosity > 1:
                         print(f"test LL for each fold: {row}", file=sys.stderr)
 
-    results = run_grid(gen_pat, kmers, codes, pos, neg, alphas, penalties, nf, nit, args.seed, verbosity, progress=progress)
+    runner = sharded_cv_runner(gen_pat, codes, pos, neg, nf)   # None: the jobs are dealt to the ranks (or one GPU runs them)
+    try:
+        results = run_grid(gen_pat, kmers, codes, pos, neg, alphas, penalties, nf, nit, args.seed, verbosity, runner=runner,
+                           progress=progress)
+    finally:
+        if runner is not None:   # collective: every rank gets here, also when the grid raised (on all ranks alike)
+            runner.close()
     cvfile = args.CVfile if rank == 0 else None
     return select_best(alphas, penalties, results, nit, nf, len(gen_pat), cvfile)

@@ -47,16 +47,31 @@ def dp_buffer_bytes(plan):
             + int(info.backtrack_ws_bytes))
 
 
-def fits_one_gpu(plan):
-    """True when the DP's buffers fit in what is free on the plan's device right now, counting what the plan already
-    holds (its cached buffers are reused, not allocated again)."""
+def cv_buffer_bytes(plan, nfolds):
+    """Device bytes the unsharded cross-validation (GpuFoldRunner, pipelined jobs) allocates: two train tables and two
+    kept-whole masks in rotation, the expanded totals and the expanded held-out tables of every fold, the k-mer tables
+    of the totals and of one fold, and the backtrack workspace."""
+    info = plan.info
+    return (2 * (int(info.table_elems) * 4 + int(info.kept_elems) * 2) + (2 + 2 * int(nfolds)) * int(info.expanded_elems) * 8
+            + 4 * int(info.nkmer) * 8 + int(info.backtrack_ws_bytes))
+
+
+def fits_free_memory(plan, need, held_prefixes):
+    """True when `need` bytes fit in what is free on the plan's device right now, counting what the plan already holds in
+    the buffers whose names start with one of `held_prefixes` and the backtrack workspace (cached buffers are reused,
+    not allocated again)."""
     import torch
 
     free, _total = torch.cuda.mem_get_info(plan.device)
     held = sum(t.numel() * t.element_size() for name, t in plan._buf.items()
-               if name in ("best", "kept", "expM", "expU", "btws"))
+               if name.startswith(tuple(held_prefixes)) or name == "btws")
     reserve = 512 << 20   # allocator slack, CUDA context growth
-    return dp_buffer_bytes(plan) - held + reserve <= free + _cached_free(plan.device)
+    return need - held + reserve <= free + _cached_free(plan.device)
+
+
+def fits_one_gpu(plan):
+    """True when the single DP's buffers fit in what is free on the plan's device right now."""
+    return fits_free_memory(plan, dp_buffer_bytes(plan), ("best", "kept", "expM", "expU"))
 
 
 def _cached_free(device):

@@ -1127,15 +1127,17 @@ int kp_ipc_close(int device, void *d_ptr)
     return 0;
 }
 
-int kp_shard_dp_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_t *d_expU, uint64_t max_count, double alpha,
-                     double beta, double penalty, void *stream)
+// one wave of this rank's tiles on the counts d_expM - d_subM, d_expU - d_subU (d_sub*: null for none, as in dp_counts)
+static int shard_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_t *d_expU, const int64_t *d_subM,
+                      const int64_t *d_subU, uint64_t max_count, double alpha, double beta, double penalty, void *stream,
+                      const char *what)
 {
-    if (!s) return fail("kp_shard_dp_wave: null shard");
+    if (!s) return fail(std::string(what) + ": null shard");
     kp_plan *p = s->plan;
     const KpTables &t = p->host.t;
-    if (wave < 0 || wave >= (int)s->hl_off.size() - 1 || wave >= 64) return fail("kp_shard_dp_wave: bad wave");
+    if (wave < 0 || wave >= (int)s->hl_off.size() - 1 || wave >= 64) return fail(std::string(what) + ": bad wave");
     for (int r = 0; r < s->world; r++)
-        if (!s->view.best[r] || !s->view.flags[r]) return fail("kp_shard_dp_wave: a peer's shard has not been set");
+        if (!s->view.best[r] || !s->view.flags[r]) return fail(std::string(what) + ": a peer's shard has not been set");
     cudaStream_t st = (cudaStream_t)stream;
     KP_CUDA(cudaSetDevice(p->device));
     if (wave == 0) KP_CUDA(cudaMemsetAsync(s->d_counters, 0, sizeof(uint32_t) * 64, st));
@@ -1150,6 +1152,8 @@ int kp_shard_dp_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_t
     prm.rowtab = p->d_rowtab;
     prm.e0 = (const long long *)d_expM;
     prm.e1 = (const long long *)d_expU;
+    prm.s0 = (const long long *)d_subM;
+    prm.s1 = (const long long *)d_subU;
     prm.alpha = alpha; prm.beta = beta; prm.penalty = penalty;
     prm.best = s->d_best;
     prm.flags = s->d_kept;
@@ -1178,6 +1182,65 @@ int kp_shard_dp_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_t
     }
     p->launches++;
     KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int kp_shard_dp_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_t *d_expU, uint64_t max_count, double alpha,
+                     double beta, double penalty, void *stream)
+{
+    return shard_wave(s, wave, d_expM, d_expU, nullptr, nullptr, max_count, alpha, beta, penalty, stream, "kp_shard_dp_wave");
+}
+
+int kp_shard_cv_wave(kp_shard *s, int wave, const int64_t *d_expMtot, const int64_t *d_expUtot, const int64_t *d_expMtest,
+                     const int64_t *d_expUtest, uint64_t max_count, double alpha, double beta_fold, double penalty, void *stream)
+{
+    if (!d_expMtest || !d_expUtest) return fail("kp_shard_cv_wave: null held-out table");
+    return shard_wave(s, wave, d_expMtot, d_expUtot, d_expMtest, d_expUtest, max_count, alpha, beta_fold, penalty, stream,
+                      "kp_shard_cv_wave");
+}
+
+// kp_cv_heldout over the shard view: the backtrack reads the peers' tables, the leaf kernel this rank's (replicated) count
+// tables; the root's train loss comes from the same device gather as kp_shard_gather
+int kp_shard_cv_heldout(kp_shard *s, const int64_t *d_expMtot, const int64_t *d_expUtot, const int64_t *d_expMtest,
+                        const int64_t *d_expUtest, double alpha, double beta_fold, double penalty, uint64_t root, void *d_ws,
+                        uint64_t cap, float *h_top, void *stream)
+{
+    if (!s || !d_expMtot || !d_expUtot || !d_expMtest || !d_expUtest || !d_ws || !h_top)
+        return fail("kp_shard_cv_heldout: null argument");
+    kp_plan *p = s->plan;
+    if (p->host.t.total_level > 64) return fail("kp_shard_cv_heldout: more than 64 levels");
+    if (root == UINT64_MAX) root = p->host.npat - 1;
+    if (root >= p->host.npat) return fail("kp_shard_cv_heldout: root out of range");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    if (scratch_reserve(p, sizeof(float), st)) return 1;
+    float *d_rootval = (float *)p->d_scratch;
+    unsigned long long *sorted, *keys, *ctr;
+    float *vals;
+    if (backtrack_device(p, s->view, d_ws, cap, root, st, &sorted, &keys, &vals, &ctr)) return 1;
+    kp_cv_leaf_kernel<<<p->sm_count, 128, 0, st>>>(p->d_tab, p->d_rowtab, (const long long *)d_expMtot, (const long long *)d_expUtot,
+                                                   (const long long *)d_expMtest, (const long long *)d_expUtest, alpha, beta_fold,
+                                                   penalty, sorted, ctr, cap, vals);
+    kp_gather_kernel<<<1, 32, 0, st>>>(p->d_tab, p->d_rowtab, s->view, nullptr, root, 1, d_rootval);
+    p->launches += 2;
+    KP_CUDA(cudaGetLastError());
+    unsigned long long hc[2] = {0, 0};
+    int herr = 0;
+    float htrain = 0.f;
+    KP_CUDA(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(&herr, p->d_err, sizeof herr, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(&htrain, d_rootval, sizeof htrain, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    if (herr == 2) return fail("kp_shard_cv_heldout: the DP gave up waiting for a child tile (internal error)");
+    if (hc[1] || hc[0] > cap) return fail_capacity("kp_shard_cv_heldout: partition larger than the workspace capacity");
+    if (hc[0] == 0) return fail("kp_shard_cv_heldout: the backtrack produced no leaf (internal error)");
+    std::vector<unsigned long long> hk(hc[0]);
+    std::vector<float> hv(hc[0]);
+    KP_CUDA(cudaMemcpyAsync(hk.data(), keys, hc[0] * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(hv.data(), vals, hc[0] * 4, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    h_top[0] = htrain;
+    h_top[1] = tree_sum(hk.data(), hv.data(), 0, hc[0], 0);
     return 0;
 }
 

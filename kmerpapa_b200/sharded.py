@@ -48,6 +48,7 @@ class ShardedDP:
         self._opened = []
         self._group = None
         self._token = None
+        self._local = None
 
     def close_peers(self):
         """Unmap the peers' shards (CUDA IPC).  Local only; see close()."""
@@ -74,6 +75,7 @@ class ShardedDP:
 
             dist.barrier(group=self._group)
             self._token = None
+        self._local = None
         self.lib.kp_shard_destroy(self.handle)
         self.handle = None
 
@@ -88,7 +90,9 @@ class ShardedDP:
 
     # -- wiring --------------------------------------------------------------------------------------
     def connect_local(self, shards):
-        """All shards live in this process (possibly on one GPU): hand each other the raw device pointers."""
+        """All shards live in this process (possibly on one GPU): hand each other the raw device pointers.  cv_job on
+        any of them then runs the waves of all of them, in lock-step on one stream."""
+        self._local = list(shards)
         for other in shards:
             if other.rank != self.rank:
                 check(self.lib.kp_shard_set_peer(self.handle, other.rank, ctypes.c_void_p(other.info.d_best),
@@ -99,24 +103,35 @@ class ShardedDP:
         import torch.distributed as dist
 
         torch = _torch()
+        # collective from here on (close() included), and every rank learns whether all ranks succeeded (agree())
+        self._group = group
+        self._token = torch.zeros(1, dtype=torch.int32, device=self.plan.device)
         hb, hk = (ctypes.c_uint8 * 64)(), (ctypes.c_uint8 * 64)()
-        check(self.lib.kp_ipc_export(ctypes.c_void_p(self.info.d_best), hb), "kp_ipc_export")
-        check(self.lib.kp_ipc_export(ctypes.c_void_p(self.info.d_kept), hk), "kp_ipc_export")
+        err = None
+        try:
+            check(self.lib.kp_ipc_export(ctypes.c_void_p(self.info.d_best), hb), "kp_ipc_export")
+            check(self.lib.kp_ipc_export(ctypes.c_void_p(self.info.d_kept), hk), "kp_ipc_export")
+        except KpError as e:
+            err = e
+        self.agree(err, "kp_ipc_export")
         mine = (self.rank, bytes(hb), bytes(hk))
         everyone = [None] * self.world
         dist.all_gather_object(everyone, mine, group=group)
-        for r, b, k in everyone:
-            if r == self.rank:
-                continue
-            pb, pk = ctypes.c_void_p(), ctypes.c_void_p()
-            check(self.lib.kp_ipc_open(self.plan.device_index, (ctypes.c_uint8 * 64).from_buffer_copy(b), ctypes.byref(pb)),
-                  "kp_ipc_open")
-            check(self.lib.kp_ipc_open(self.plan.device_index, (ctypes.c_uint8 * 64).from_buffer_copy(k), ctypes.byref(pk)),
-                  "kp_ipc_open")
-            self._opened += [pb.value, pk.value]
-            check(self.lib.kp_shard_set_peer(self.handle, r, pb, pk), "kp_shard_set_peer")
-        self._group = group
-        self._token = torch.zeros(1, dtype=torch.int32, device=self.plan.device)
+        try:
+            for r, b, k in everyone:
+                if r == self.rank:
+                    continue
+                pb, pk = ctypes.c_void_p(), ctypes.c_void_p()
+                check(self.lib.kp_ipc_open(self.plan.device_index, (ctypes.c_uint8 * 64).from_buffer_copy(b),
+                                           ctypes.byref(pb)), "kp_ipc_open")
+                self._opened.append(pb.value)
+                check(self.lib.kp_ipc_open(self.plan.device_index, (ctypes.c_uint8 * 64).from_buffer_copy(k),
+                                           ctypes.byref(pk)), "kp_ipc_open")
+                self._opened.append(pk.value)
+                check(self.lib.kp_shard_set_peer(self.handle, r, pb, pk), "kp_shard_set_peer")
+        except KpError as e:
+            err = e
+        self.agree(err, "ShardedDP.connect")
 
     def barrier(self):
         """All ranks have finished the work they queued on their current streams (one tiny NCCL all_reduce)."""
@@ -124,6 +139,20 @@ class ShardedDP:
             import torch.distributed as dist
 
             dist.all_reduce(self._token, group=self._group)
+
+    def agree(self, err, what):
+        """Barrier that also tells every rank whether all ranks succeeded (MIN all_reduce of a success flag, read back).
+        err: this rank's exception or None.  Raises on every rank as soon as one rank failed, so that no rank is left
+        waiting in a collective the failed rank will never join."""
+        if self._token is not None:
+            import torch.distributed as dist
+
+            self._token.fill_(0 if err is not None else 1)
+            dist.all_reduce(self._token, op=dist.ReduceOp.MIN, group=self._group)
+            if int(self._token.item()) == 0 and err is None:
+                err = KpError(f"{what}: failed on another rank")
+        if err is not None:
+            raise err
 
     # -- the DP ----------------------------------------------------------------------------------------
     def wave(self, w, eM, eU, max_count, alpha, beta, penalty):
@@ -135,6 +164,55 @@ class ShardedDP:
         for w in range(self.nwaves):
             self.wave(w, eM, eU, max_count, alpha, beta, penalty)
             self.barrier()
+
+    # -- cross-validation jobs -------------------------------------------------------------------------
+    def cv_wave(self, w, eMtot, eUtot, eMte, eUte, max_count, alpha, beta, penalty):
+        check(self.lib.kp_shard_cv_wave(self.handle, int(w), eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(),
+                                        eUte.data_ptr(), int(max_count), float(alpha), float(beta), float(penalty),
+                                        self.plan._stream()), "kp_shard_cv_wave")
+
+    def cv_job(self, eMtot, eUtot, eMte, eUte, max_count, alpha, beta, penalty, root=None, cap=65536):
+        """One fold x alpha x penalty on the train counts total - held-out (PartitionPlan.cv_job over the shards): every
+        wave, then (np.float32 train loss, np.float32 held-out loss) of `root` (default: the general pattern).  With
+        in-process shards (connect_local) the waves of all of them run here, in lock-step on one stream; with one
+        process per rank (connect) every rank calls this with the same arguments and the ranks meet after every wave."""
+        job = (eMtot, eUtot, eMte, eUte, max_count, alpha, beta, penalty)
+        if self._local is not None:
+            for w in range(self.nwaves):
+                for s in self._local:
+                    s.cv_wave(w, *job)
+        else:
+            for w in range(self.nwaves):
+                err = None
+                try:
+                    self.cv_wave(w, *job)
+                except KpError as e:
+                    err = e
+                self.agree(err, f"kp_shard_cv_wave {w}")
+        err = res = None
+        try:
+            res = self.cv_heldout(eMtot, eUtot, eMte, eUte, alpha, beta, penalty, root, cap)
+        except KpError as e:
+            err = e
+        self.agree(err, "kp_shard_cv_heldout")   # no rank starts the next job's waves while a peer may still read its tables
+        return res
+
+    def cv_heldout(self, eMtot, eUtot, eMte, eUte, alpha, beta, penalty, root=None, cap=65536):
+        """(train, held-out) loss of `root` after the last wave of a CV job (this rank only, reads the peers' tables)."""
+        torch = _torch()
+        top = (ctypes.c_float * 2)()
+        while True:
+            ws = self.plan._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
+            rc = self.lib.kp_shard_cv_heldout(self.handle, eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(),
+                                              float(alpha), float(beta), float(penalty),
+                                              self.plan.TOP if root is None else int(root), ws.data_ptr(), cap,
+                                              ctypes.cast(top, ctypes.c_void_p), self.plan._stream())
+            if rc == 0:
+                return np.float32(top[0]), np.float32(top[1])
+            if rc == KP_ERR_CAPACITY and cap < self.plan.MAX_CAP:
+                cap *= 8
+                continue
+            raise KpError("kp_shard_cv_heldout: " + self.lib.kp_last_error().decode())
 
     def backtrack(self, cap=65536, root=None):
         torch = _torch()
