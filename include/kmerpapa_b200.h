@@ -272,6 +272,14 @@ int kp_debug_log(int device, const double *h_x, double *h_y, uint64_t n);
 /* Test hook: level-0 score of (M,U) pairs on the device (scipy xlogy/xlog1py restated). */
 int kp_debug_leaf_score(int device, const int64_t *h_M, const int64_t *h_U, uint64_t n, double alpha, double beta,
                         double penalty, double *h_out);
+/* Test hook: the three level >= 1 scoring paths of the DP kernels, item by item.  Item i has the per-base counts
+ * h_M[4i..4i+3], h_U[4i..4i+3] (>= 0; the pattern's counts are their sums), its own alpha, beta and penalty, and
+ * h_wide[i] = 1 for 64-bit on-chip counts, 0 for 32-bit (refused when the counts sum to 2^32 or more).  Outputs:
+ * h_lb = the score filter's float32 lower bound; h_ok, h_sf, h_rup, h_fast = kp_self_score_fast's verdict,
+ * RN_f32(s), "rounded up" bit and float64 estimate s~; h_exact = the exact float64 score.  Host buffers. */
+int kp_debug_self_score(int device, const int64_t *h_M, const int64_t *h_U, const double *h_alpha, const double *h_beta,
+                        const double *h_penalty, const uint8_t *h_wide, uint64_t n, float *h_lb, uint8_t *h_ok, float *h_sf,
+                        uint8_t *h_rup, double *h_fast, double *h_exact);
 
 #ifdef __cplusplus
 }

@@ -82,6 +82,7 @@ SYMBOLS = {
     "kp_kmer_fold_terms": (_int, [_int, _vp, _vp, _vp, _vp, _vp, _u64, _dbl, _vp, _vp]),
     "kp_debug_log": (_int, [_int, _vp, _vp, _u64]),
     "kp_debug_leaf_score": (_int, [_int, _vp, _vp, _u64, _dbl, _dbl, _dbl, _vp]),
+    "kp_debug_self_score": (_int, [_int, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -1421,4 +1421,49 @@ int kp_debug_leaf_score(int device, const int64_t *h_M, const int64_t *h_U, uint
     return 0;
 }
 
+int kp_debug_self_score(int device, const int64_t *h_M, const int64_t *h_U, const double *h_alpha, const double *h_beta,
+                        const double *h_penalty, const uint8_t *h_wide, uint64_t n, float *h_lb, uint8_t *h_ok, float *h_sf,
+                        uint8_t *h_rup, double *h_fast, double *h_exact)
+{
+    if (!h_M || !h_U || !h_alpha || !h_beta || !h_penalty || !h_wide || !h_lb || !h_ok || !h_sf || !h_rup || !h_fast || !h_exact)
+        return fail("kp_debug_self_score: null argument");
+    if (n == 0) return 0;
+    for (uint64_t i = 0; i < n; i++) {
+        uint64_t tot = 0;
+        for (int b = 0; b < 8; b++) {
+            const int64_t c = b < 4 ? h_M[4 * i + b] : h_U[4 * i + b - 4];
+            if (c < 0) return fail("kp_debug_self_score: negative count");
+            tot += (uint64_t)c;
+            if (tot >> 62) return fail("kp_debug_self_score: counts of an item sum to 2^62 or more");
+        }
+        if (!h_wide[i] && (tot >> 32)) return fail("kp_debug_self_score: narrow (32-bit) item whose counts sum to 2^32 or more");
+    }
+    KP_CUDA(cudaSetDevice(device));
+    // inputs: M, U (8 x 8 bytes), alpha, beta, penalty (3 x 8), wide (1); outputs: st, exact (2 x 8), lb, sf (2 x 4), ok, rup (2)
+    const size_t per = 8 * 8 + 3 * 8 + 1 + 2 * 8 + 2 * 4 + 2;
+    unsigned char *d = nullptr;
+    KP_CUDA(cudaMalloc(&d, n * per));
+    long long *dM = (long long *)d, *dU = dM + 4 * n;
+    double *da = (double *)(dU + 4 * n), *db = da + n, *dp = db + n, *dst = dp + n, *dex = dst + n;
+    float *dlb = (float *)(dex + n), *dsf = dlb + n;
+    unsigned char *dw = (unsigned char *)(dsf + n), *dok = dw + n, *drup = dok + n;
+    cudaMemcpy(dM, h_M, n * 32, cudaMemcpyHostToDevice);
+    cudaMemcpy(dU, h_U, n * 32, cudaMemcpyHostToDevice);
+    cudaMemcpy(da, h_alpha, n * 8, cudaMemcpyHostToDevice);
+    cudaMemcpy(db, h_beta, n * 8, cudaMemcpyHostToDevice);
+    cudaMemcpy(dp, h_penalty, n * 8, cudaMemcpyHostToDevice);
+    cudaError_t e = cudaMemcpy(dw, h_wide, n, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        kp_debug_self_score_kernel<<<296, 256>>>(dM, dU, da, db, dp, dw, n, dlb, dok, dsf, drup, dst, dex);
+        e = cudaGetLastError();
+    }
+    const void *src[6] = {dlb, dok, dsf, drup, dst, dex};
+    void *dst_h[6] = {h_lb, h_ok, h_sf, h_rup, h_fast, h_exact};
+    const size_t bytes[6] = {4, 1, 4, 1, 8, 8};
+    for (int k = 0; k < 6 && e == cudaSuccess; k++) e = cudaMemcpy(dst_h[k], src[k], n * bytes[k], cudaMemcpyDeviceToHost);
+    cudaFree(d);
+    if (e != cudaSuccess) return fail(std::string("kp_debug_self_score: ") + cudaGetErrorString(e));
+    return 0;
+}
+
 }  // extern "C"

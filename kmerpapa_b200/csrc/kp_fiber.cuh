@@ -177,7 +177,7 @@ __global__ void __launch_bounds__(KP_FIBER_THREADS, 1) kp_dp_fiber_kernel(const 
     for (int l = 0; l <= KP_FIBER_ROW_LEVELS; l++) lvl_start[l] = ft.lvl_start[l];
 
     const double alpha = p.alpha, beta = p.beta, penalty = p.penalty;
-    const float alpha_f = (float)alpha, ab_f = (float)(alpha + beta), penalty_f = (float)penalty;
+    const KpFilterK fk = kp_filter_consts(alpha, beta, penalty);
     const float INF = __int_as_float(0x7f800000);
     const uint32_t hwf = ft.hw;
     const int nhigh = tb.nhigh, fhi = ft.fhi;
@@ -360,7 +360,7 @@ __global__ void __launch_bounds__(KP_FIBER_THREADS, 1) kp_dp_fiber_kernel(const 
                             if ((kp_bm_c<R0>(2 * h) >> b) & 1) { Mf.x += mf[b]; Uf.x += uf[b]; }
                             if (2 * h + 1 < R0 && ((kp_bm_c<R0>(2 * h + 1) >> b) & 1)) { Mf.y += mf[b]; Uf.y += uf[b]; }
                         }
-                        const float2 lb = kp_score_lower_bound2(Mf, Uf, alpha_f, ab_f, penalty_f);
+                        const float2 lb = kp_score_lower_bound2(Mf, Uf, fk);
                         if (!(lb.x > v[2 * h])) need |= 1u << (2 * h);
                         if (2 * h + 1 < R0 && !(lb.y > v[2 * h + 1])) need |= 1u << (2 * h + 1);
                     }

@@ -112,9 +112,10 @@ __device__ __noinline__ double kp_self_score_exact_nl(C M, C U, double alpha, do
 #ifndef KP_FAST_INLINE
 #define KP_FAST_INLINE __forceinline__
 #endif
+// st (test hook only): receives s~; the DP kernels pass nothing and the store is compiled out.
 template <typename C>
 __device__ KP_FAST_INLINE bool kp_self_score_fast(C M, C U, double alpha, double beta, double penalty, const double2 *tab,
-                                                   const KpLogK &K, float &sf, bool &rup)
+                                                   const KpLogK &K, float &sf, bool &rup, double *st = nullptr)
 {
     const double Md = kp_cnt2d(M), Ud = kp_cnt2d(U), Sd = kp_cnt2d((C)(M + U));
     const double num = KP_ADD(Md, alpha), den = KP_ADD(KP_ADD(Sd, alpha), beta);
@@ -179,6 +180,7 @@ __device__ KP_FAST_INLINE bool kp_self_score_fast(C M, C U, double alpha, double
     const double fd = (double)flo;
     sf = flo;
     rup = fd > shi;
+    if (st) *st = sa;
     ok = ok && flo == fhi && (fd > shi || fd < slo) && sa < 0x1p120;   // NaN / inf / ambiguous: exact path
     return ok;
 }
@@ -248,23 +250,42 @@ __device__ __forceinline__ float kp_min3(float a, float b, float c)
     return r;
 }
 
+// Launch constants of the score filter, converted once per kernel (every caller of kp_score_lower_bound2 takes them from
+// here).  base = the margin's constant term: 0.01, plus 4e-4 |penalty| when penalty < 0.  The relative term rel |est| of
+// the margin only bounds the error when est = pen + t1 + t2 does not cancel, i.e. pen >= 0; with pen < 0 the error still
+// scales with t1 + t2 = est - pen <= |est| + |pen|, so rel (t1 + t2 + |pen|) <= rel |est| + 2 rel |pen| <= rel |est| +
+// 4e-4 |pen| for both values of rel, which also covers the rounding of penalty to float32.
+struct KpFilterK { float alpha, ab, penalty, base; };
+__device__ __forceinline__ KpFilterK kp_filter_consts(double alpha, double beta, double penalty)
+{
+    KpFilterK f;
+    f.alpha = (float)alpha;
+    f.ab = (float)(alpha + beta);
+    f.penalty = (float)penalty;
+    f.base = penalty >= 0.0 ? 0.01f : __fmaf_rn(4e-4f, (float)-penalty, 0.01f);
+    return f;
+}
+
 // Float32 lower bound of the self-score (w_numba.py:56-61) for the score filter, two patterns at a time with
-// the packed f32x2 instructions of sm_100 (FADD2/FMUL2/FFMA2).  Error budget of the estimate (both terms of s are >= 0:
-// no cancellation):
+// the packed f32x2 instructions of sm_100 (FADD2/FMUL2/FFMA2).  Error budget of the estimate (pen >= 0: both terms of s
+// are >= 0, no cancellation; pen < 0: see kp_filter_consts):
 //   counts -> float32 and their sums   <= 4 roundings of 2^-24 on M, U           (exact below 2^24)
 //   p = (M + a) / (M + U + a + b)      <= 2 roundings + __fdividef (2 ulp):  |dp| / p <= 2.4e-7 + conversions 3.6e-7 = 6e-7
 //   p < 2^-5 (the usual case):  ln p < -3.4, so  __logf  is in its RELATIVE regime (3 ulp) and the error of p adds
 //       6e-7 / 3.4 relative: 5.5e-7 of the first term; ln(1-p) by its series (truncation p^4/5 < 2e-7, three roundings) plus the
-//       error of p: 1e-6 of the second term; the final fma / mul / add: 2e-7.   Total < 1.5e-6 |s|;  bound used: 1e-5 |s| + 0.01.
+//       error of p: 1e-6 of the second term; the final fma / mul / add: 2e-7.   Total < 1.5e-6 |s|.  Not relative: s is the
+//       reference's float64 score, whose q = 1 - p is rounded by up to 2^-54, so its -2U ln q is off by up to U 2^-53 however
+//       small p is (for p < 2^-54 it is 0 instead of 2Up); with counts above 2^46 that exceeds 0.01.
+//       Bound used: 1e-5 |s| + 2^-52 (M + U) + 0.01.
 //   p >= 2^-5:  __logf has ABSOLUTE error 2^-21.4 = 3.6e-7 for arguments in [0.5, 2] (rates near 1, or 1-p above the series
 //       range), and the error of p enters ln p and ln(1-p) absolutely (up to 6e-7 / 0.5): together < 1.6e-6 per unit of count,
 //       times 2: bound used  2e-4 |s| + 4e-6 (M + U) + 0.01.
-// A NaN (p == 0, ...) never skips the exact score.
-__device__ __forceinline__ float2 kp_score_lower_bound2(float2 Mf, float2 Uf, float alpha, float ab, float penalty)
+// A NaN (p == 0, ...) never skips the exact score.  tests/test_gpu_score_bounds.py checks lb <= s at the edges.
+__device__ __forceinline__ float2 kp_score_lower_bound2(float2 Mf, float2 Uf, const KpFilterK &f)
 {
-    const float2 num = __fadd2_rn(Mf, make_float2(alpha, alpha));
+    const float2 num = __fadd2_rn(Mf, make_float2(f.alpha, f.alpha));
     const float2 cnt = __fadd2_rn(Mf, Uf);
-    const float2 den = __fadd2_rn(cnt, make_float2(ab, ab));
+    const float2 den = __fadd2_rn(cnt, make_float2(f.ab, f.ab));
     const float2 p = make_float2(__fdividef(num.x, den.x), __fdividef(num.y, den.y));
     const float2 lp = make_float2(__logf(p.x), __logf(p.y));
     // log(1-p) = -p (1 + p (1/2 + p (1/3 + p/4)))  for p < 2^-5
@@ -272,12 +293,12 @@ __device__ __forceinline__ float2 kp_score_lower_bound2(float2 Mf, float2 Uf, fl
     t = __ffma2_rn(p, t, make_float2(0.5f, 0.5f));
     t = __ffma2_rn(p, t, make_float2(1.0f, 1.0f));
     float2 l1 = __fmul2_rn(make_float2(-p.x, -p.y), t);
-    float2 rel = make_float2(1e-5f, 1e-5f), per = make_float2(0.f, 0.f);   // margin: relative only for small rates
+    float2 rel = make_float2(1e-5f, 1e-5f), per = make_float2(0x1p-52f, 0x1p-52f);   // margin of the small rates
     if (!(p.x < 0.03125f)) { l1.x = __logf(1.0f - p.x); rel.x = 2e-4f; per.x = 4e-6f; }
     if (!(p.y < 0.03125f)) { l1.y = __logf(1.0f - p.y); rel.y = 2e-4f; per.y = 4e-6f; }
     const float2 ll = __ffma2_rn(Mf, lp, __fmul2_rn(Uf, l1));                       // M log p + U log(1-p)  (<= 0)
-    const float2 est = __ffma2_rn(ll, make_float2(-2.0f, -2.0f), make_float2(penalty, penalty));
-    const float2 mar = __ffma2_rn(make_float2(fabsf(est.x), fabsf(est.y)), rel, __ffma2_rn(cnt, per, make_float2(0.01f, 0.01f)));
+    const float2 est = __ffma2_rn(ll, make_float2(-2.0f, -2.0f), make_float2(f.penalty, f.penalty));
+    const float2 mar = __ffma2_rn(make_float2(fabsf(est.x), fabsf(est.y)), rel, __ffma2_rn(cnt, per, make_float2(f.base, f.base)));
     return __fadd2_rn(est, make_float2(-mar.x, -mar.y));
 }
 
@@ -407,7 +428,7 @@ __global__ void KP_DP_BOUNDS kp_dp_rows_kernel(const KpDpParams p)
     uint32_t *hs2 = hs1 + maxhs;
     int *s_nhs = (int *)(hs2 + maxhs);
     const double alpha = p.alpha, beta = p.beta, penalty = p.penalty;
-    const float alpha_f = (float)alpha, ab_f = (float)(alpha + beta), penalty_f = (float)penalty;
+    const KpFilterK fk = kp_filter_consts(alpha, beta, penalty);
     const float INF = __int_as_float(0x7f800000);
     const float *tbase = p.best;
     unsigned long long pol_first;
@@ -738,7 +759,7 @@ __global__ void KP_DP_BOUNDS kp_dp_rows_kernel(const KpDpParams p)
                             if ((kp_bm_c<R0>(2 * h) >> b) & 1) { Mf.x += mf[b]; Uf.x += uf[b]; }
                             if (2 * h + 1 < R0 && ((kp_bm_c<R0>(2 * h + 1) >> b) & 1)) { Mf.y += mf[b]; Uf.y += uf[b]; }
                         }
-                        const float2 lb = kp_score_lower_bound2(Mf, Uf, alpha_f, ab_f, penalty_f);
+                        const float2 lb = kp_score_lower_bound2(Mf, Uf, fk);
                         if (!(lb.x > v[2 * h])) need |= 1u << (2 * h);
                         if (2 * h + 1 < R0 && !(lb.y > v[2 * h + 1])) need |= 1u << (2 * h + 1);
                     }
@@ -1587,4 +1608,50 @@ __global__ void kp_debug_leaf_kernel(const long long *M, const long long *U, uns
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n;
          i += (unsigned long long)gridDim.x * blockDim.x)
         out[i] = kp_leaf_score((unsigned long long)M[i], (unsigned long long)U[i], alpha, beta, penalty, tab);
+}
+
+// The three level >= 1 scoring paths of the DP kernels for one item: the score filter's lower bound (per-base counts
+// converted to float and summed in base order, as the kernels do), the fast score (ok, sf, rounded-up bit, s~) and the
+// exact score, in the count width C.  M, U: [n][4] per-base counts.
+template <typename C>
+__device__ void kp_debug_self_score_one(const long long *M, const long long *U, double alpha, double beta, double penalty,
+                                        const double2 *tab, float &lb, unsigned char &ok, float &sf, unsigned char &rup,
+                                        double &st, double &exact)
+{
+    C m[4], u[4], M_ = 0, U_ = 0;
+    float2 Mf = make_float2(0.f, 0.f), Uf = make_float2(0.f, 0.f);
+    for (int b = 0; b < 4; b++) {
+        m[b] = (C)M[b];
+        u[b] = (C)U[b];
+        M_ += m[b];
+        U_ += u[b];
+        Mf.x += (float)m[b];
+        Uf.x += (float)u[b];
+    }
+    Mf.y = Mf.x;
+    Uf.y = Uf.x;
+    lb = kp_score_lower_bound2(Mf, Uf, kp_filter_consts(alpha, beta, penalty)).x;
+    const KpLogK K = kp_logk_load();
+    bool r = false;
+    ok = kp_self_score_fast<C>(M_, U_, alpha, beta, penalty, tab, K, sf, r, &st);
+    rup = r;
+    exact = kp_self_score_exact_nl<C>(M_, U_, alpha, beta, penalty, tab);
+}
+
+__global__ void kp_debug_self_score_kernel(const long long *M, const long long *U, const double *alpha, const double *beta,
+                                           const double *penalty, const unsigned char *wide, unsigned long long n, float *lb,
+                                           unsigned char *ok, float *sf, unsigned char *rup, double *st, double *exact)
+{
+    __shared__ double2 tab[128];
+    for (int i = threadIdx.x; i < 128; i += blockDim.x) tab[i] = make_double2(kpc_logTab[2 * i], kpc_logTab[2 * i + 1]);
+    __syncthreads();
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        if (wide[i])
+            kp_debug_self_score_one<unsigned long long>(M + 4 * i, U + 4 * i, alpha[i], beta[i], penalty[i], tab, lb[i], ok[i],
+                                                        sf[i], rup[i], st[i], exact[i]);
+        else
+            kp_debug_self_score_one<unsigned int>(M + 4 * i, U + 4 * i, alpha[i], beta[i], penalty[i], tab, lb[i], ok[i], sf[i],
+                                                  rup[i], st[i], exact[i]);
+    }
 }

@@ -409,6 +409,13 @@ double kpo_leaf_score(double alpha, double beta, double penalty, uint64_t M, uin
     return -2.0 * (kpo_xlogy((double)M, p) + kpo_xlog1py((double)U, -p)) + penalty;
 }
 
+/* level >= 1 self-score of n items (w_numba.py:56-61), each with its own alpha, beta and penalty */
+void kpo_self_score_array(const double *alpha, const double *beta, const double *penalty, const uint64_t *M, const uint64_t *U,
+                          double *out, int64_t n)
+{
+    for (int64_t i = 0; i < n; i++) out[i] = self_score(alpha[i], beta[i], penalty[i], M[i], U[i], NULL, NULL);
+}
+
 /*
  * kmerM/kmerU: counts per k-mer in k-mer index order.  leaf_score: optional level-0 scores
  * (float32, k-mer index order) computed by the caller with scipy; NULL -> kpo_leaf_score().

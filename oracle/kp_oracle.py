@@ -49,6 +49,7 @@ def lib():
         L.kpo_num2pattern.argtypes = [ctypes.c_char_p, u64, ctypes.c_char_p]
         L.kpo_leaf_score.restype = dbl
         L.kpo_leaf_score.argtypes = [dbl, dbl, dbl, u64, u64]
+        L.kpo_self_score_array.argtypes = [vp, vp, vp, vp, vp, vp, i64]
         L.kpo_single_dp.argtypes = [ctypes.c_char_p, vp, vp, vp, dbl, dbl, dbl, vp, vp, vp, vp, cint]
         L.kpo_backtrack.restype = i64
         L.kpo_backtrack.argtypes = [ctypes.c_char_p, vp, vp, i64]

@@ -47,11 +47,11 @@ def _codes(gen_pat):
     return np.array([iupac.kmer_code(k) for k in iupac.matches(gen_pat)], dtype=np.uint64)
 
 
-@pytest.mark.parametrize("regime", ["dense", "sparse", "ties"])
+@pytest.mark.parametrize("regime", ["dense", "sparse", "ties", "negative_penalty"])
 @pytest.mark.parametrize("gen_pat", SHAPES)
 def test_fiber_kernel_against_oracle(oracle, monkeypatch, gen_pat, regime):
-    M, U = _counts(gen_pat, 77 + len(gen_pat), regime)
-    alpha, penalty = (0.8, 4.0) if regime != "ties" else (1.0, 0.5)
+    M, U = _counts(gen_pat, 77 + len(gen_pat), "dense" if regime == "negative_penalty" else regime)
+    alpha, penalty = {"ties": (1.0, 0.5), "negative_penalty": (10.0, -3.0)}.get(regime, (0.8, 4.0))
     mc = int(M.sum() + U.sum())
     mu = max(int(M.sum()), 1) / max(mc, 2)
     beta = alpha * (1.0 - mu) / mu

@@ -177,12 +177,13 @@ def test_random_against_oracle(eng, oracle, gen_pat, seed):
 
 
 @pytest.mark.parametrize("regime", ["rate_near_one", "half", "tiny_counts", "huge_counts", "zeros", "penalty_ties", "low_rates",
-                                    "kept_whole"])
+                                    "kept_whole", "negative_penalty"])
 @pytest.mark.parametrize("gen_pat", ["NNNNN", "NNMNNN", "NNNNNN"])
 def test_count_regimes_against_oracle(eng, oracle, gen_pat, regime):
     """Regimes that stress the score filter (a float32 bound decides whether the exact FP64 score is computed): rates
     near 1 (absolute error of the fast log), rates around 1/2, counts of a few units, counts near 2^31, mostly empty
-    tables, and penalties that make many self-scores tie with split sums.  Full table + split codes vs the oracle."""
+    tables, penalties that make many self-scores tie with split sums, and negative penalties (the filter's estimate
+    pen + t1 + t2 then cancels).  Full table + split codes vs the oracle."""
     import zlib
 
     rng = np.random.default_rng(zlib.crc32((gen_pat + regime).encode()))
@@ -207,14 +208,15 @@ def test_count_regimes_against_oracle(eng, oracle, gen_pat, regime):
     elif regime == "low_rates":     # the fast score path (kp_self_score_fast): rates on both sides of its 2^-8 switch, up to 2^-4
         U = rng.integers(10 ** 4, 10 ** 6, size=nk)
         M = rng.binomial(U, np.exp(rng.uniform(np.log(1e-6), np.log(0.07), size=nk)))
-    elif regime == "kept_whole":    # a penalty so large that every pattern is kept whole: every stored value is a self-score
+    elif regime in ("kept_whole", "negative_penalty"):   # kept_whole: a penalty so large that every pattern is kept whole
         U = 1 + rng.negative_binomial(2, 2 / (2 + 33000.0), size=nk)
         M = rng.binomial(U, np.minimum(0.5, 1e-3 * np.exp(rng.normal(0, 0.7, size=nk))))
     else:
         U = np.full(nk, 1000)
         M = np.full(nk, 10)
     U[0], M[0] = max(U[0], 5), max(M[0], 1)
-    grid = {"penalty_ties": ((1.0, 0.0), (1.0, 2.0)), "kept_whole": ((1.0, 1e6), (0.01, 3e3))}.get(regime, ((1.0, 4.0), (0.5, 0.0)))
+    grid = {"penalty_ties": ((1.0, 0.0), (1.0, 2.0)), "kept_whole": ((1.0, 1e6), (0.01, 3e3)),
+            "negative_penalty": ((1.0, -0.5), (10.0, -3.0))}.get(regime, ((1.0, 4.0), (0.5, 0.0)))
     for alpha, pen in grid:
         mu = M.sum() / (M.sum() + U.sum())
         beta = alpha * (1 - mu) / mu
@@ -226,9 +228,11 @@ def test_count_regimes_against_oracle(eng, oracle, gen_pat, regime):
 
 
 @pytest.mark.parametrize("gen_pat,seed", [("NNNNN", 21), ("RYNNANNKM", 22), ("VNNNH", 23), ("MMMMMMMMMM", 24),
-                                          ("RYNNNANRY", 25), ("BBDHVVB", 26), ("N", 27), ("ACGT", 28), ("NNNSNN", 29)])
+                                          ("RYNNNANRY", 25), ("BBDHVVB", 26), ("N", 27), ("ACGT", 28), ("NNNSNN", 29),
+                                          ("NNNNNN", 30)])
 def test_random_cv_job_against_oracle(eng, oracle, gen_pat, seed):
-    """One held-out fold on larger / oddly shaped general patterns: train and held-out tables, both widths."""
+    """One held-out fold on larger / oddly shaped general patterns: train and held-out tables, both widths.  Seed 30: a
+    negative penalty."""
     rng = np.random.default_rng(seed)
     _, nk, _ = oracle.plan_info(gen_pat)
     U = (1 + rng.negative_binomial(2, 2 / (2 + 800.0), size=nk)) * (rng.random(nk) < 0.9)
@@ -238,7 +242,7 @@ def test_random_cv_job_against_oracle(eng, oracle, gen_pat, seed):
         M = np.minimum(U, rng.choice([0, 1, 2, 4], size=nk))
         M[0], U[0] = 3, 50
     Mte, Ute = rng.binomial(M, 0.3), rng.binomial(U, 0.3)
-    alpha, pen = 1.0, 3.0
+    alpha, pen = (1.0, 3.0) if seed < 30 else (1.0, -2.0)
     mu = (M.sum() - Mte.sum()) / ((M.sum() - Mte.sum()) + (U.sum() - Ute.sum()))
     beta = alpha * (1 - mu) / mu
     plan = eng.get_plan(gen_pat)
