@@ -173,6 +173,30 @@ int kp_cv_heldout(kp_plan *plan, const float *d_train, const uint16_t *d_kept, c
 int kp_pattern_counts(kp_plan *plan, const int64_t *d_kmerM, const int64_t *d_kmerU, const uint64_t *h_patnums,
                       uint64_t n, int64_t *h_M, int64_t *h_U, void *stream);
 
+/*
+ * Scoring a fitted partition on k-mer counts (replaces the reference's papa.PatternPartition check, papa.py:53-107, and
+ * its get_loss on new data).  h_patnums[n]: the partition's patterns as dense pattern numbers of the plan's general
+ * pattern, in file order (1 <= n < 2^32 - 1).  Any plan works; a lite plan is enough.
+ *
+ * kp_partition_assign fills d_owner (uint32[nkmer]) with the index of the pattern that covers each k-mer
+ * (0xFFFFFFFF: none) and reports *h_conflict = 1 + the smallest k-mer index covered twice and *h_uncovered = 1 + the
+ * smallest k-mer index covered by no pattern, each 0 when there is none.  Members of the patterns are claimed in
+ * file order in chunks of nkmer; the first chunk that finds a k-mer claimed twice ends the pass, so *h_conflict is the
+ * smallest k-mer covered twice within the chunks up to it (all of them when the sizes sum to at most nkmer), and
+ * *h_uncovered is 0 then.  At most two chunks run.  Synchronises.
+ *
+ * kp_partition_score: per pattern, the counts M[q], U[q] of its k-mers in d_kmerM / d_kmerU (kp_pack_counts layout)
+ * and h_t[q] = xlogy(M, p) + xlog1py(U, -p) in float64 with p = h_rate[q] (bit for bit as scipy evaluates it).  Refused
+ * when the pattern sizes sum to more than nkmer.  d_kmer_rate (optional, double[nkmer]): the rate of each k-mer's
+ * owner in d_owner from kp_partition_assign (NaN where there is none).  Synchronises.  Every output is the same on
+ * every run.
+ */
+int kp_partition_assign(kp_plan *plan, const uint64_t *h_patnums, uint64_t n, uint32_t *d_owner, uint64_t *h_conflict,
+                        uint64_t *h_uncovered, void *stream);
+int kp_partition_score(kp_plan *plan, const uint64_t *h_patnums, const double *h_rate, uint64_t n, const int64_t *d_kmerM,
+                       const int64_t *d_kmerU, const uint32_t *d_owner, double *d_kmer_rate, int64_t *h_M, int64_t *h_U,
+                       double *h_t, void *stream);
+
 /* Where a dense pattern number lives in the device layout: element of a float table, element and bit of d_kept. */
 int kp_pattern_offset(const kp_plan *plan, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit);
 

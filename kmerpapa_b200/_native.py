@@ -60,7 +60,9 @@ SYMBOLS = {
     "kp_cv_job_finish": (_int, [_vp, _u64, _vp]),
     "kp_cv_heldout": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _u64, _vp, _u64, _vp, _vp]),
     "kp_pattern_counts": (_int, [_vp, _vp, _vp, _vp, _u64, _vp, _vp, _vp]),
-    "kp_pattern_offset": (_int, [_vp, _u64, ctypes.POINTER(_u64), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_uint32)]),
+    "kp_partition_assign": (_int, [_vp, _vp, _u64, _vp, ctypes.POINTER(_u64), ctypes.POINTER(_u64), _vp]),
+    "kp_partition_score": (_int, [_vp, _vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "kp_pattern_offset":(_int, [_vp, _u64, ctypes.POINTER(_u64), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_uint32)]),
     "kp_plan_launch_count": (_u64, [_vp]),
     "kp_dp_kernel_name": (_cp, [_vp]),
     "kp_shard_assignment": (_int, [_vp, _int, _vp, _vp]),

@@ -796,6 +796,132 @@ int kp_pattern_counts(kp_plan *p, const int64_t *d_kmerM, const int64_t *d_kmerU
 }
 
 // ===================================================================================================
+// Scoring a given partition.  Both entries lay out the partition in the plan's scratch: the uploaded pattern numbers,
+// their packed subsets, the member offsets (n + 1) and the scan's block sums; part_prepare returns the member total.
+// ===================================================================================================
+struct PartLayout {
+    unsigned long long *pat, *pm, *offs, *bsum;
+};
+
+static size_t part_bytes(uint64_t n) { return (3 * n + 1 + 1024) * 8; }   // the caller's own arrays follow
+
+static PartLayout part_layout(const kp_plan *p, uint64_t n)
+{
+    PartLayout L;
+    L.pat = (unsigned long long *)p->d_scratch;
+    L.pm = L.pat + n;
+    L.offs = L.pm + n;
+    L.bsum = L.offs + n + 1;
+    return L;
+}
+
+static int part_check(const kp_plan *p, const char *what, const uint64_t *h_patnums, uint64_t n)
+{
+    if (!p) return fail(std::string(what) + ": null plan");
+    if (!h_patnums || n == 0) return fail(std::string(what) + ": empty partition");
+    if (n >= KP_OWNER_EMPTY) return fail(std::string(what) + ": too many patterns (owners are uint32)");
+    for (uint64_t i = 0; i < n; i++)
+        if (h_patnums[i] >= p->host.npat) return fail(std::string(what) + ": pattern number out of range");
+    return 0;
+}
+
+// after scratch_reserve: upload the patterns and scan their sizes (synchronises to read the total)
+static int part_prepare(kp_plan *p, const uint64_t *h_patnums, uint64_t n, cudaStream_t st, uint64_t *total)
+{
+    const PartLayout L = part_layout(p, n);
+    KP_CUDA(cudaMemcpyAsync(L.pat, h_patnums, n * 8, cudaMemcpyHostToDevice, st));
+    const uint64_t nb = std::min<uint64_t>(1024, (n + 255) / 256), per = (n + nb - 1) / nb;
+    kp_part_prep_kernel<<<(unsigned)nb, 256, 0, st>>>(p->d_tab, L.pat, n, per, L.pm, L.bsum);
+    kp_part_scan_kernel<<<1, 256, 0, st>>>(L.bsum, (unsigned)nb, L.offs, n);
+    kp_part_offsets_kernel<<<(unsigned)nb, 256, 0, st>>>(p->d_tab, L.pm, n, per, L.bsum, L.offs);
+    p->launches += 3;
+    KP_CUDA(cudaGetLastError());
+    unsigned long long tot = 0;
+    KP_CUDA(cudaMemcpyAsync(&tot, L.offs + n, 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    *total = tot;
+    return 0;
+}
+
+int kp_partition_assign(kp_plan *p, const uint64_t *h_patnums, uint64_t n, uint32_t *d_owner, uint64_t *h_conflict,
+                        uint64_t *h_uncovered, void *stream)
+{
+    if (part_check(p, "kp_partition_assign", h_patnums, n)) return KP_ERR;
+    if (!d_owner || !h_conflict || !h_uncovered) return fail("kp_partition_assign: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    if (scratch_reserve(p, part_bytes(n) + 16, st)) return KP_ERR;
+    const PartLayout L = part_layout(p, n);
+    unsigned long long *d_res = L.bsum + 1024;
+    uint64_t total = 0;
+    if (part_prepare(p, h_patnums, n, st, &total)) return KP_ERR;
+    const uint64_t nkmer = p->host.nkmer;
+    KP_CUDA(cudaMemsetAsync(d_owner, 0xFF, nkmer * 4, st));
+    KP_CUDA(cudaMemsetAsync(d_res, 0xFF, 16, st));
+    const int grid = p->sm_count * 8;
+    unsigned long long res[2] = {~0ull, ~0ull};
+    // Chunks of nkmer members.  Past the first chunk a conflict is certain (more members than k-mers), so at most two
+    // chunks run before the loop stops, however much the file over-covers.
+    for (uint64_t lo = 0; lo < total; lo += nkmer) {
+        const uint64_t hi = std::min<uint64_t>(total, lo + nkmer);
+        kp_part_assign_kernel<<<grid, 256, 0, st>>>(p->d_tab, L.pm, L.offs, n, lo, hi, d_owner, d_res);
+        p->launches++;
+        KP_CUDA(cudaGetLastError());
+        if (hi == total) break;
+        KP_CUDA(cudaMemcpyAsync(res, d_res, 8, cudaMemcpyDeviceToHost, st));
+        KP_CUDA(cudaStreamSynchronize(st));
+        if (res[0] != ~0ull) break;
+    }
+    KP_CUDA(cudaMemcpyAsync(res, d_res, 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    if (res[0] == ~0ull) {   // the owner table is complete only when no chunk was cut short
+        kp_part_cover_kernel<<<grid_for(nkmer, 256, p->sm_count), 256, 0, st>>>(d_owner, nkmer, d_res);
+        p->launches++;
+        KP_CUDA(cudaGetLastError());
+        KP_CUDA(cudaMemcpyAsync(res, d_res, 16, cudaMemcpyDeviceToHost, st));
+        KP_CUDA(cudaStreamSynchronize(st));
+    }
+    *h_conflict = res[0] == ~0ull ? 0 : res[0] + 1;
+    *h_uncovered = res[0] != ~0ull || res[1] == ~0ull ? 0 : res[1] + 1;
+    return 0;
+}
+
+int kp_partition_score(kp_plan *p, const uint64_t *h_patnums, const double *h_rate, uint64_t n, const int64_t *d_kmerM,
+                       const int64_t *d_kmerU, const uint32_t *d_owner, double *d_kmer_rate, int64_t *h_M, int64_t *h_U,
+                       double *h_t, void *stream)
+{
+    if (part_check(p, "kp_partition_score", h_patnums, n)) return KP_ERR;
+    if (!h_rate || !d_kmerM || !d_kmerU || !h_M || !h_U || !h_t) return fail("kp_partition_score: null argument");
+    if (d_kmer_rate && !d_owner) return fail("kp_partition_score: the per-k-mer rates need the owner table");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    if (scratch_reserve(p, part_bytes(n) + 4 * n * 8, st)) return KP_ERR;
+    const PartLayout L = part_layout(p, n);
+    unsigned long long *d_M = (unsigned long long *)((unsigned char *)p->d_scratch + part_bytes(n)), *d_U = d_M + n;
+    double *d_rate = (double *)(d_U + n), *d_t = d_rate + n;
+    uint64_t total = 0;
+    if (part_prepare(p, h_patnums, n, st, &total)) return KP_ERR;
+    if (total > p->host.nkmer) return fail("kp_partition_score: the patterns have more members than there are k-mers (they overlap)");
+    KP_CUDA(cudaMemcpyAsync(d_rate, h_rate, n * 8, cudaMemcpyHostToDevice, st));
+    KP_CUDA(cudaMemsetAsync(d_M, 0, 2 * n * 8, st));
+    kp_part_counts_kernel<<<p->sm_count * 8, 256, 0, st>>>(p->d_tab, L.pm, L.offs, n, total, (const long long *)d_kmerM,
+                                                           (const long long *)d_kmerU, d_M, d_U);
+    kp_part_terms_kernel<<<grid_for(n, 256, p->sm_count), 256, 0, st>>>(d_M, d_U, d_rate, n, d_t);
+    p->launches += 2;
+    if (d_kmer_rate) {
+        kp_part_kmer_rate_kernel<<<grid_for(p->host.nkmer, 256, p->sm_count), 256, 0, st>>>(d_owner, d_rate, n, p->host.nkmer,
+                                                                                           d_kmer_rate);
+        p->launches++;
+    }
+    KP_CUDA(cudaGetLastError());
+    KP_CUDA(cudaMemcpyAsync(h_M, d_M, n * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h_U, d_U, n * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h_t, d_t, n * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// ===================================================================================================
 // One DP sharded over the GPUs of a node (SURVEY 8f.3).  The score table is split by the digit of the top high
 // position; every rank runs the same waves on its own tiles and reads the children that live on a peer straight
 // from the peer's memory (NVLink) inside the DP kernel.  The caller puts a barrier between the waves.

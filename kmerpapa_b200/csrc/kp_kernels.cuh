@@ -1570,6 +1570,269 @@ __global__ void __launch_bounds__(256) kp_pattern_counts_kernel(const KpTables *
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Scoring a given partition (kp_partition_assign / kp_partition_score).  The partition's patterns, in file order,
+// are flattened into one member space: pattern q owns members [offs[q], offs[q + 1]) (offs = exclusive prefix sum of
+// the pattern sizes), and member j of a pattern is the k-mer of mixed-radix digit j over its positions (position 0
+// fastest, the bases of a position in A, C, G, T order).  Work is spread over members, not patterns, so a pattern that
+// covers half of the k-mers costs the same per k-mer as many one-k-mer patterns.  A pattern is held as its nucleotide
+// subsets packed 4 bits per effective position ("pm").  Every output is an integer atomic, a min-reduction or a
+// per-pattern float64 expression: the results are the same on every run.
+// ---------------------------------------------------------------------------------------------------
+#define KP_OWNER_EMPTY 0xFFFFFFFFu
+#define KP_PART_ITERS 16   // 32-member steps of one warp range (a warp range is 512 consecutive members)
+
+// k-mer index contribution of the r-th base (A, C, G, T order) of subset m at effective position e
+__device__ __forceinline__ void kp_part_offsets_init(const KpTables &tb, uint32_t (*s_off)[16][4])
+{
+    for (int x = threadIdx.x; x < KP_MAXPOS * 16; x += blockDim.x) {
+        const int e = x >> 4, m = x & 15;
+        int r = 0;
+        for (int b = 0; b < 4; b++)
+            if ((m >> b) & 1) s_off[e][m][r++] = (uint32_t)tb.mask_digit[e][1u << b] * tb.kw[e];
+    }
+}
+
+// k-mer index of member j of the pattern with packed subsets pm
+__device__ __forceinline__ uint32_t kp_part_kidx(const uint32_t (*s_off)[16][4], unsigned long long pm, int npos, uint32_t j)
+{
+    uint32_t kidx = 0;
+    for (int e = 0; e < npos; e++) {
+        const uint32_t m = (uint32_t)(pm >> (4 * e)) & 15u, nb = __popc(m);
+        const uint32_t q = nb == 3 ? __umulhi(j, 0xAAAAAAABu) >> 1 : j >> (nb >> 1);   // j / nb for nb in 1..4
+        kidx += s_off[e][m][j - q * nb];
+        j = q;
+    }
+    return kidx;
+}
+
+// largest q in [lo, hi] with offs[q] <= i (offs[lo] <= i)
+__device__ __forceinline__ unsigned long long kp_part_find(const unsigned long long *offs, unsigned long long lo,
+                                                           unsigned long long hi, unsigned long long i)
+{
+    while (lo < hi) {
+        const unsigned long long mid = lo + (hi - lo + 1) / 2;
+        if (offs[mid] <= i) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// exclusive scan of one value per thread over a 256-thread block; total = the block's sum
+__device__ __forceinline__ unsigned long long kp_block_scan256(unsigned long long v, unsigned long long *s8,
+                                                               unsigned long long &total)
+{
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    unsigned long long x = v;
+    for (int d = 1; d < 32; d <<= 1) {
+        const unsigned long long y = __shfl_up_sync(0xFFFFFFFFu, x, d);
+        if (lane >= d) x += y;
+    }
+    if (lane == 31) s8[w] = x;
+    __syncthreads();
+    unsigned long long pre = 0, tot = 0;
+    for (int i = 0; i < 8; i++) {
+        const unsigned long long s = s8[i];
+        if (i < w) pre += s;
+        tot += s;
+    }
+    __syncthreads();
+    total = tot;
+    return pre + x - v;
+}
+
+// scan pass 1: packed subsets and size of every pattern; block b sums the sizes of patterns [b * per, (b + 1) * per)
+__global__ void __launch_bounds__(256) kp_part_prep_kernel(const KpTables *tab, const unsigned long long *patnums,
+                                                           unsigned long long n, unsigned long long per,
+                                                           unsigned long long *pm, unsigned long long *bsum)
+{
+    const KpTables &tb = *tab;
+    __shared__ unsigned long long s8[8];
+    const unsigned long long lo = blockIdx.x * per, hi = min(n, lo + per);
+    unsigned long long acc = 0;
+    for (unsigned long long q = lo + threadIdx.x; q < hi; q += blockDim.x) {
+        unsigned long long x = patnums[q], packed = 0, size = 1;
+        for (int e = 0; e < tb.npos; e++) {
+            const uint32_t m = tb.digit_mask[e][x % tb.radix[e]];
+            x /= tb.radix[e];
+            packed |= (unsigned long long)m << (4 * e);
+            size *= (unsigned long long)__popc(m);
+        }
+        pm[q] = packed;
+        acc += size;
+    }
+    unsigned long long total;
+    kp_block_scan256(acc, s8, total);
+    if (threadIdx.x == 0) bsum[blockIdx.x] = total;
+}
+
+// scan pass 2 (one block): bsum[0..nb) -> exclusive prefix sums; offs[n] = total members
+__global__ void __launch_bounds__(256) kp_part_scan_kernel(unsigned long long *bsum, unsigned int nb, unsigned long long *offs,
+                                                           unsigned long long n)
+{
+    __shared__ unsigned long long s8[8];
+    unsigned long long carry = 0;
+    for (unsigned int base = 0; base < nb; base += blockDim.x) {
+        const unsigned int b = base + threadIdx.x;
+        const unsigned long long v = b < nb ? bsum[b] : 0;
+        unsigned long long total;
+        const unsigned long long ex = kp_block_scan256(v, s8, total);
+        if (b < nb) bsum[b] = carry + ex;
+        carry += total;
+    }
+    if (threadIdx.x == 0) offs[n] = carry;
+}
+
+// scan pass 3: offs[q] = members of the patterns before q
+__global__ void __launch_bounds__(256) kp_part_offsets_kernel(const KpTables *tab, const unsigned long long *pm,
+                                                              unsigned long long n, unsigned long long per,
+                                                              const unsigned long long *bsum, unsigned long long *offs)
+{
+    const int npos = tab->npos;
+    __shared__ unsigned long long s8[8];
+    const unsigned long long lo = blockIdx.x * per, hi = min(n, lo + per);
+    unsigned long long carry = bsum[blockIdx.x];
+    for (unsigned long long base = lo; base < hi; base += blockDim.x) {
+        const unsigned long long q = base + threadIdx.x;
+        unsigned long long size = 0;
+        if (q < hi) {
+            size = 1;
+            for (int e = 0; e < npos; e++) size *= (unsigned long long)__popc((uint32_t)(pm[q] >> (4 * e)) & 15u);
+        }
+        unsigned long long total;
+        const unsigned long long ex = kp_block_scan256(size, s8, total);
+        if (q < hi) offs[q] = carry + ex;
+        carry += total;
+    }
+}
+
+// Assign: members [lo, hi) claim their k-mer, owner[kidx] = q, with a compare-and-swap on an all-empty table.  A
+// failed swap means the k-mer is covered twice: result[0] = min of such k-mers.  Warp w takes the 512 members from
+// lo + 512 w on; lane l of step s has member base + 32 s + l, so consecutive lanes hold consecutive members and a
+// step's patterns lie within 32 of the previous step's last one.
+__global__ void __launch_bounds__(256) kp_part_assign_kernel(const KpTables *tab, const unsigned long long *pm,
+                                                             const unsigned long long *offs, unsigned long long n,
+                                                             unsigned long long lo, unsigned long long hi, uint32_t *owner,
+                                                             unsigned long long *result)
+{
+    __shared__ uint32_t s_off[KP_MAXPOS][16][4];
+    kp_part_offsets_init(*tab, s_off);
+    __syncthreads();
+    const int npos = tab->npos, lane = threadIdx.x & 31;
+    const unsigned long long warp = (blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x) >> 5;
+    const unsigned long long nwarp = (gridDim.x * (unsigned long long)blockDim.x) >> 5, span = 32ull * KP_PART_ITERS;
+    unsigned long long conflict = ~0ull;
+    for (unsigned long long wbase = lo + warp * span; wbase < hi; wbase += nwarp * span) {
+        unsigned long long qlo = kp_part_find(offs, 0, n - 1, wbase);
+        for (int s = 0; s < KP_PART_ITERS && wbase + 32ull * s < hi; s++) {
+            const unsigned long long i = wbase + 32ull * s + lane;
+            const unsigned long long q = kp_part_find(offs, qlo, min(qlo + 32, n - 1), i);
+            if (i < hi) {
+                const uint32_t kidx = kp_part_kidx(s_off, pm[q], npos, (uint32_t)(i - offs[q]));
+                if (atomicCAS(owner + kidx, KP_OWNER_EMPTY, (uint32_t)q) != KP_OWNER_EMPTY)
+                    conflict = min(conflict, (unsigned long long)kidx);
+            }
+            qlo = __shfl_sync(0xFFFFFFFFu, q, 31);
+        }
+    }
+    if (conflict != ~0ull) atomicMin(result, conflict);
+}
+
+// Cover: result[1] = smallest k-mer index nobody owns
+__global__ void __launch_bounds__(256) kp_part_cover_kernel(const uint32_t *owner, unsigned long long nkmer,
+                                                            unsigned long long *result)
+{
+    uint32_t first = 0xFFFFFFFFu;
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < nkmer;
+         i += (unsigned long long)gridDim.x * blockDim.x)
+        if (owner[i] == KP_OWNER_EMPTY) { first = (uint32_t)i; break; }   // later i of this thread are larger
+    first = __reduce_min_sync(0xFFFFFFFFu, first);
+    if ((threadIdx.x & 31) == 0 && first != 0xFFFFFFFFu) atomicMin(result + 1, (unsigned long long)first);
+}
+
+// Score, counts: (M, U) of every pattern = sums of the k-mer counts of its members (outM / outU zeroed).  Same walk as
+// the assign kernel; each step's 32 counts are summed per run of equal patterns by a segmented warp reduction.  The
+// run that reaches lane 31 is carried into the next step, so a pattern spanning a warp range costs one atomic per
+// range, not one per step.
+__global__ void __launch_bounds__(256) kp_part_counts_kernel(const KpTables *tab, const unsigned long long *pm,
+                                                             const unsigned long long *offs, unsigned long long n,
+                                                             unsigned long long total, const long long *kmerM,
+                                                             const long long *kmerU, unsigned long long *outM,
+                                                             unsigned long long *outU)
+{
+    __shared__ uint32_t s_off[KP_MAXPOS][16][4];
+    kp_part_offsets_init(*tab, s_off);
+    __syncthreads();
+    const int npos = tab->npos, lane = threadIdx.x & 31;
+    const unsigned long long warp = (blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x) >> 5;
+    const unsigned long long nwarp = (gridDim.x * (unsigned long long)blockDim.x) >> 5, span = 32ull * KP_PART_ITERS;
+    for (unsigned long long wbase = warp * span; wbase < total; wbase += nwarp * span) {
+        unsigned long long qlo = kp_part_find(offs, 0, n - 1, wbase);
+        unsigned long long cq = ~0ull, cM = 0, cU = 0;   // carried run (the same in every lane)
+        for (int s = 0; s < KP_PART_ITERS && wbase + 32ull * s < total; s++) {
+            const unsigned long long i = wbase + 32ull * s + lane;
+            const unsigned long long q = kp_part_find(offs, qlo, min(qlo + 32, n - 1), i);
+            unsigned long long m = 0, u = 0;
+            if (i < total) {
+                const uint32_t kidx = kp_part_kidx(s_off, pm[q], npos, (uint32_t)(i - offs[q]));
+                m = (unsigned long long)kmerM[kidx];
+                u = (unsigned long long)kmerU[kidx];
+            }
+            // after step d a lane holds the sum of its run's next 2d lanes: the first lane of each run holds the run
+            for (int d = 1; d < 32; d <<= 1) {
+                const unsigned long long om = __shfl_down_sync(0xFFFFFFFFu, m, d), ou = __shfl_down_sync(0xFFFFFFFFu, u, d);
+                const unsigned long long oq = __shfl_down_sync(0xFFFFFFFFu, q, d);
+                if (lane + d < 32 && oq == q) { m += om; u += ou; }
+            }
+            const unsigned long long qprev = __shfl_up_sync(0xFFFFFFFFu, q, 1);
+            const bool head = lane == 0 || qprev != q;
+            const unsigned long long q0 = __shfl_sync(0xFFFFFFFFu, q, 0), q31 = __shfl_sync(0xFFFFFFFFu, q, 31);
+            const int hl = __ffs(__ballot_sync(0xFFFFFFFFu, q == q31)) - 1;
+            const unsigned long long lm = __shfl_sync(0xFFFFFFFFu, m, hl), lu = __shfl_sync(0xFFFFFFFFu, u, hl);
+            if (head && q != q31) {   // a finished run; the carry continues in it only when it starts at lane 0
+                if (q == cq) { m += cM; u += cU; }
+                atomicAdd(outM + q, m);
+                atomicAdd(outU + q, u);
+            }
+            if (cq == q31) {          // the whole step continues the carried run
+                cM += lm;
+                cU += lu;
+            } else {
+                if (lane == 0 && cq != ~0ull && cq != q0) { atomicAdd(outM + cq, cM); atomicAdd(outU + cq, cU); }
+                cq = q31;
+                cM = lm;
+                cU = lu;
+            }
+            qlo = q31;
+        }
+        if (lane == 0 && cq != ~0ull) { atomicAdd(outM + cq, cM); atomicAdd(outU + cq, cU); }
+    }
+}
+
+// Score, terms: t[q] = xlogy(M, p) + xlog1py(U, -p) in float64 (score_utils.get_loss's summand, scipy-exact)
+__global__ void kp_part_terms_kernel(const unsigned long long *M, const unsigned long long *U, const double *rate,
+                                     unsigned long long n, double *t)
+{
+    __shared__ double2 tab[128];
+    for (int i = threadIdx.x; i < 128; i += blockDim.x) tab[i] = make_double2(kpc_logTab[2 * i], kpc_logTab[2 * i + 1]);
+    __syncthreads();
+    for (unsigned long long q = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; q < n;
+         q += (unsigned long long)gridDim.x * blockDim.x) {
+        const double p = rate[q];
+        t[q] = KP_ADD(kp_xlogy((double)M[q], p, tab), kp_xlog1py((double)U[q], -p, tab));
+    }
+}
+
+// rate of every k-mer: the rate of the pattern that owns it (NaN for a k-mer without an owner)
+__global__ void kp_part_kmer_rate_kernel(const uint32_t *owner, const double *rate, unsigned long long n,
+                                         unsigned long long nkmer, double *out)
+{
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < nkmer;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        const uint32_t o = owner[i];
+        out[i] = o < n ? rate[o] : __longlong_as_double(0x7ff8000000000000LL);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
 // test hooks
 // ---------------------------------------------------------------------------------------------------
 __global__ void kp_debug_log_kernel(const double *x, double *y, unsigned long long n)

@@ -259,6 +259,39 @@ class PartitionPlan:
                                          M.ctypes.data, U.ctypes.data, self._stream()), "kp_pattern_counts")
         return M, U
 
+    # -- scoring a given partition ---------------------------------------------------------------
+    def partition_assign(self, patnums, name="part"):
+        """Owner of every k-mer for a partition given as dense pattern numbers (file order).  Returns (owner, conflict,
+        uncovered): the uint32 owner table (int32 tensor, -1 = none) and the smallest k-mer index covered twice / by no
+        pattern, None when there is none (kp_partition_assign)."""
+        torch = _torch()
+        patnums = np.ascontiguousarray(patnums, dtype=np.uint64)
+        owner = self._buffer(name + "_owner", self.nkmer, torch.int32)
+        conflict, uncovered = ctypes.c_uint64(0), ctypes.c_uint64(0)
+        check(self.lib.kp_partition_assign(self.handle, patnums.ctypes.data, patnums.size, owner.data_ptr(),
+                                           ctypes.byref(conflict), ctypes.byref(uncovered), self._stream()),
+              "kp_partition_assign")
+        return (owner[: self.nkmer], conflict.value - 1 if conflict.value else None,
+                uncovered.value - 1 if uncovered.value else None)
+
+    def partition_score(self, patnums, rates, kM, kU, owner=None, name="part"):
+        """(M, U, t) per pattern on the k-mer tables kM / kU: int64 counts and the float64 terms
+        xlogy(M, p) + xlog1py(U, -p) (kp_partition_score).  With the owner table of partition_assign, also the float64
+        rate of every k-mer (device tensor) as a fourth value."""
+        torch = _torch()
+        patnums = np.ascontiguousarray(patnums, dtype=np.uint64)
+        rates = np.ascontiguousarray(rates, dtype=np.float64)
+        if rates.shape != patnums.shape:
+            raise ValueError("one rate per pattern")
+        n = patnums.size
+        M, U, t = np.empty(n, dtype=np.int64), np.empty(n, dtype=np.int64), np.empty(n, dtype=np.float64)
+        kmer_rate = self._buffer(name + "_rate", self.nkmer, torch.float64) if owner is not None else None
+        check(self.lib.kp_partition_score(self.handle, patnums.ctypes.data, rates.ctypes.data, n, kM.data_ptr(), kU.data_ptr(),
+                                          owner.data_ptr() if owner is not None else None,
+                                          kmer_rate.data_ptr() if owner is not None else None,
+                                          M.ctypes.data, U.ctypes.data, t.ctypes.data, self._stream()), "kp_partition_score")
+        return (M, U, t) if owner is None else (M, U, t, kmer_rate[: self.nkmer])
+
     # -- dense views (tests, exports) ------------------------------------------------------------
     def gather(self, table, first=0, n=None):
         """float32 values of patterns first..first+n-1 (dense numbering) from a device table."""

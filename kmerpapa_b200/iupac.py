@@ -36,6 +36,16 @@ def matches(pattern):
     return out
 
 
+def kmer_of_index(pattern, idx):
+    """matches(pattern)[idx] without the list: the k-mer index is mixed radix over the positions, first fastest."""
+    out = []
+    for ch in pattern:
+        bases = CODE[ch]
+        out.append(bases[idx % len(bases)])
+        idx //= len(bases)
+    return "".join(out)
+
+
 def lca_pattern(kmers):
     """Smallest pattern covering all the given k-mers."""
     k = len(kmers[0])
