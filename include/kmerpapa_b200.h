@@ -197,6 +197,37 @@ int kp_partition_score(kp_plan *plan, const uint64_t *h_patnums, const double *h
                        const int64_t *d_kmerU, const uint32_t *d_owner, double *d_kmer_rate, int64_t *h_M, int64_t *h_U,
                        double *h_t, void *stream);
 
+/* Applying a partition along sequences (DESIGN §4c; kmerpapa_b200/apply_partition.py).  Position i of a record of
+ * length rec_len has the window seq[i - c, i - c + k), c = k / 2.  The window is a context when it lies in the record
+ * and all its bytes are A, C, G or T (either case).  It matches when every base lies in the general pattern's letter at
+ * its position; its k-mer index is kp_pack_counts'.  With both != 0 (odd k only) the reverse complement of the window is
+ * looked up too, and the position's rate is p_fwd + p_rev (one float64 addition; a side that does not match adds 0).
+ *
+ * kp_kmer_rates: d_kmer_rate (double[nkmer]) = h_rate of each k-mer's owner in d_owner from kp_partition_assign (NaN
+ * where there is none).  Synchronises.
+ *
+ * kp_seq_scan: one pass over the positions [pos0, pos1) of a record; pos0 is a multiple of the piece size 65536.
+ * d_seq holds the record bytes [seq_base, seq_base + seq_len), 16-byte aligned and readable up to the next multiple of
+ * 16 bytes; it must hold every window of the positions that lies in the record.  Without d_tasks, block b sums piece
+ * pos0 / 65536 + b of the record (its positions in [pos0, pos1)): d_sum[b] = its float64 rate sum by a fixed tree and
+ * d_n[b] = its matching (position, strand) pairs.  Optionally d_track[i - pos0] = RN_f32(rate of position i), NaN where i
+ * has no context; and d_counts[kidx] (int64[nkmer], not zeroed here) += 1 per match of a position i whose bit
+ * i - pos0 is set in d_count_mask (uint32 words; NULL: every position).  With d_tasks (uint32[ntask][3]: piece of the
+ * record, lo, hi), entry t gives in d_sum[t], d_n[t] the same sums restricted to positions piece * 65536 + [lo, hi),
+ * through the same tree with zeros elsewhere: where a task covers the whole piece its sum is the piece's sum, bit for
+ * bit; tracks and counts are refused there.  Does not synchronise.
+ *
+ * kp_region_sums: for region r = d_regions[4r..4r+3] = (first piece pa, last piece pb, task of pa or -1, task of pb or
+ * -1), d_sum[r] / d_n[r] = the left-to-right float64 / int64 sums over the pieces pa..pb of the task sums d_task_sum /
+ * d_task_n where a task is given and of the piece sums d_piece_sum / d_piece_n elsewhere.  Does not synchronise.
+ * Every output is the same on every run and for every split of a record into calls. */
+int kp_kmer_rates(kp_plan *plan, const uint32_t *d_owner, const double *h_rate, uint64_t n, double *d_kmer_rate, void *stream);
+int kp_seq_scan(kp_plan *plan, const uint8_t *d_seq, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0,
+                uint64_t pos1, int both, const double *d_kmer_rate, const uint32_t *d_tasks, uint64_t ntask, double *d_sum,
+                int64_t *d_n, float *d_track, const uint32_t *d_count_mask, int64_t *d_counts, void *stream);
+int kp_region_sums(kp_plan *plan, const double *d_piece_sum, const int64_t *d_piece_n, const double *d_task_sum,
+                   const int64_t *d_task_n, const int64_t *d_regions, uint64_t n, double *d_sum, int64_t *d_n, void *stream);
+
 /* Where a dense pattern number lives in the device layout: element of a float table, element and bit of d_kept. */
 int kp_pattern_offset(const kp_plan *plan, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit);
 

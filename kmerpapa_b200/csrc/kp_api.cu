@@ -922,6 +922,87 @@ int kp_partition_score(kp_plan *p, const uint64_t *h_patnums, const double *h_ra
 }
 
 // ===================================================================================================
+// Applying a partition along sequences (DESIGN §4c).  Nothing here synchronises: the caller overlaps the next chunk's
+// upload with the scan.
+// ===================================================================================================
+int kp_kmer_rates(kp_plan *p, const uint32_t *d_owner, const double *h_rate, uint64_t n, double *d_kmer_rate, void *stream)
+{
+    if (!p) return fail("kp_kmer_rates: null plan");
+    if (!d_owner || !h_rate || !d_kmer_rate || n == 0) return fail("kp_kmer_rates: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    if (scratch_reserve(p, n * 8, st)) return KP_ERR;
+    double *d_rate = (double *)p->d_scratch;
+    KP_CUDA(cudaMemcpyAsync(d_rate, h_rate, n * 8, cudaMemcpyHostToDevice, st));
+    kp_part_kmer_rate_kernel<<<grid_for(p->host.nkmer, 256, p->sm_count), 256, 0, st>>>(d_owner, d_rate, n, p->host.nkmer,
+                                                                                       d_kmer_rate);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    KP_CUDA(cudaStreamSynchronize(st));   // the scratch is reused by the next call
+    return 0;
+}
+
+int kp_seq_scan(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0,
+                uint64_t pos1, int both, const double *d_kmer_rate, const uint32_t *d_tasks, uint64_t ntask, double *d_sum,
+                int64_t *d_n, float *d_track, const uint32_t *d_count_mask, int64_t *d_counts, void *stream)
+{
+    if (!p) return fail("kp_seq_scan: null plan");
+    const int k = p->host.k, c = k / 2;
+    if (!d_seq || !d_kmer_rate || !d_sum || !d_n) return fail("kp_seq_scan: null argument");
+    if ((uintptr_t)d_seq & 15) return fail("kp_seq_scan: the sequence buffer must be 16-byte aligned");
+    if (both && k % 2 == 0) return fail("kp_seq_scan: both strands need an odd k");
+    if (pos0 % KP_SEQ_PIECE || pos0 > pos1 || pos1 > rec_len) return fail("kp_seq_scan: bad position range");
+    // every window of [pos0, pos1) that lies in the record must lie in the given bytes
+    const uint64_t need_lo = pos0 >= (uint64_t)c ? pos0 - c : 0, need_hi = std::min<uint64_t>(rec_len, pos1 + (k - 1 - c));
+    if (pos1 > pos0 && (seq_base > need_lo || seq_base + seq_len < need_hi || seq_base + seq_len > rec_len))
+        return fail("kp_seq_scan: the sequence bytes do not cover the windows of the positions");
+    if (d_tasks && (d_track || d_counts)) return fail("kp_seq_scan: tracks and counts come from the whole-piece pass");
+    if (pos1 == pos0 || (d_tasks && ntask == 0)) return 0;
+    if (!d_tasks && (pos1 - pos0 + KP_SEQ_PIECE - 1) / KP_SEQ_PIECE > 0x7FFFFFFFull) return fail("kp_seq_scan: too many pieces");
+    if (d_tasks && ntask > 0x7FFFFFFFull) return fail("kp_seq_scan: too many tasks");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    KpSeqScan a;
+    a.seq = d_seq;
+    a.seq_base = seq_base;
+    a.seq_len = seq_len;
+    a.rec_len = rec_len;
+    a.pos0 = pos0;
+    a.pos1 = pos1;
+    a.kmer_rate = d_kmer_rate;
+    a.tasks = d_tasks;
+    a.sum = d_sum;
+    a.n = (unsigned long long *)d_n;
+    a.track = d_track;
+    a.count_mask = d_count_mask;
+    a.counts = (unsigned long long *)d_counts;
+    a.k = k;
+    a.c = c;
+    const unsigned grid = (unsigned)(d_tasks ? ntask : (pos1 - pos0 + KP_SEQ_PIECE - 1) / KP_SEQ_PIECE);
+    if (both) kp_seq_scan_kernel<true><<<grid, KP_SEQ_THREADS, 0, st>>>(p->d_tab, p->d_genmask, a);
+    else kp_seq_scan_kernel<false><<<grid, KP_SEQ_THREADS, 0, st>>>(p->d_tab, p->d_genmask, a);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int kp_region_sums(kp_plan *p, const double *d_piece_sum, const int64_t *d_piece_n, const double *d_task_sum,
+                   const int64_t *d_task_n, const int64_t *d_regions, uint64_t n, double *d_sum, int64_t *d_n, void *stream)
+{
+    if (!p) return fail("kp_region_sums: null plan");
+    if (n == 0) return 0;
+    if (!d_piece_sum || !d_piece_n || !d_regions || !d_sum || !d_n) return fail("kp_region_sums: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    kp_region_sum_kernel<<<grid_for(n, 256, p->sm_count), 256, 0, st>>>(
+        d_piece_sum, (const unsigned long long *)d_piece_n, d_task_sum, (const unsigned long long *)d_task_n,
+        (const long long *)d_regions, n, d_sum, (unsigned long long *)d_n);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// ===================================================================================================
 // One DP sharded over the GPUs of a node (SURVEY 8f.3).  The score table is split by the digit of the top high
 // position; every rank runs the same waves on its own tiles and reads the children that live on a peer straight
 // from the peer's memory (NVLink) inside the DP kernel.  The caller puts a barrier between the waves.

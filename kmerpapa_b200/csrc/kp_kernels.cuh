@@ -1833,6 +1833,188 @@ __global__ void kp_part_kmer_rate_kernel(const uint32_t *owner, const double *ra
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Applying a partition along sequences (kp_seq_scan / kp_region_sums, DESIGN §4c).  Position i of a record has the
+// window seq[i - c, i - c + k), c = k / 2.  A window is a context when it lies inside the record and all its bytes are
+// A, C, G or T in either case; it matches when every base lies in the general pattern's letter at its position, and
+// its k-mer index is kp_pack_kernel's.  The reverse context is the reverse complement of the same window.
+//
+// A record is cut into pieces at multiples of KP_SEQ_PIECE in record coordinates.  One block sums the rates of one
+// piece (or of a clipped range of it, a "task") through a fixed tree: thread t adds the positions t + 256 j of the
+// piece in increasing order, then a fixed shuffle tree per warp, then the 8 warp sums in warp order.  A clipped range
+// goes through the same tree with zeros outside it, so a piece's sum is the same bits whichever chunk, grid or call
+// computes it.  The per-k-mer counts are integer atomics.
+// ---------------------------------------------------------------------------------------------------
+#define KP_SEQ_PIECE 65536u      // positions per piece
+#define KP_SEQ_TILE 4096         // positions staged in shared memory at a time (divides KP_SEQ_PIECE)
+#define KP_SEQ_THREADS 256
+#define KP_SEQ_BAD 0xFFFFFFFFu   // base not allowed at a position (bit 31: no valid k-mer index has it)
+
+struct KpSeqScan {
+    const uint8_t *seq;              // record bytes [seq_base, seq_base + seq_len), 16-byte aligned, readable to a multiple of 16
+    unsigned long long seq_base, seq_len, rec_len;
+    unsigned long long pos0, pos1;   // positions of this call [pos0, pos1), pos0 a multiple of KP_SEQ_PIECE
+    const double *kmer_rate;         // [nkmer]
+    const uint32_t *tasks;           // null: block b takes piece pos0 / PIECE + b whole; else [3 b..]: piece, lo, hi in it
+    double *sum;                     // [block] rate sum
+    unsigned long long *n;           // [block] matching (position, strand) pairs
+    float *track;                    // [pos1 - pos0] or null
+    const uint32_t *count_mask;      // bit i - pos0: count position i (null: every position)
+    unsigned long long *counts;      // [nkmer] or null
+    int k, c;
+};
+
+// k-mer index contribution of base code cd (A, C, G, T = 0..3; 4 = not a base) at string position s
+__device__ __forceinline__ uint32_t kp_seq_offset(const KpTables &tb, const uint8_t *gen_mask, int s, int cd)
+{
+    if (cd > 3) return KP_SEQ_BAD;
+    const unsigned m = 1u << cd, g = gen_mask[s];
+    if (!(m & g)) return KP_SEQ_BAD;
+    if (!(g & (g - 1))) return 0;
+    int e = 0;
+    for (int x = 0; x < s; x++) e += (gen_mask[x] & (gen_mask[x] - 1)) != 0;
+    return (uint32_t)tb.mask_digit[e][m] * tb.kw[e];
+}
+
+__device__ __forceinline__ uint8_t kp_seq_code(unsigned byte)
+{
+    const unsigned u = byte | 0x20u;   // lower case; only 'A' and 'a' become 'a', and so on
+    return u == 'a' ? 0 : u == 'c' ? 1 : u == 'g' ? 2 : u == 't' ? 3 : 4;
+}
+
+// one count per lane that wants one, aggregated over the lanes of equal index (every lane of the warp calls it)
+__device__ __forceinline__ void kp_seq_count(unsigned long long *counts, bool want, uint32_t kidx)
+{
+    const unsigned act = __ballot_sync(0xFFFFFFFFu, want);
+    if (want) {
+        const unsigned peers = __match_any_sync(act, kidx);
+        if ((int)(threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(counts + kidx, (unsigned long long)__popc(peers));
+    }
+}
+
+template <bool BOTH>
+__global__ void __launch_bounds__(KP_SEQ_THREADS) kp_seq_scan_kernel(const KpTables *tab, const uint8_t *gen_mask, KpSeqScan a)
+{
+    __shared__ uint32_t s_off[2][KP_MAXK][8];   // [strand][window position][base code]
+    __shared__ uint8_t s_code[KP_SEQ_TILE + KP_MAXK + 16];
+    __shared__ double s_wsum[KP_SEQ_THREADS / 32];
+    __shared__ unsigned long long s_wn[KP_SEQ_THREADS / 32];
+    const KpTables &tb = *tab;
+    const int k = a.k, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int x = tid; x < KP_MAXK * 8; x += blockDim.x) {
+        const int j = x >> 3, cd = x & 7;
+        // reverse strand: window byte j is base k-1-j of the reverse complement (complement of code cd is 3 - cd)
+        s_off[0][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, j, cd) : KP_SEQ_BAD;
+        s_off[1][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, k - 1 - j, cd < 4 ? 3 - cd : cd) : KP_SEQ_BAD;
+    }
+    unsigned long long piece, lo = 0, hi = KP_SEQ_PIECE;
+    if (a.tasks) {
+        piece = a.tasks[3 * blockIdx.x];
+        lo = a.tasks[3 * blockIdx.x + 1];
+        hi = a.tasks[3 * blockIdx.x + 2];
+    } else {
+        piece = a.pos0 / KP_SEQ_PIECE + blockIdx.x;
+    }
+    const unsigned long long pstart = piece * KP_SEQ_PIECE, plo = pstart + lo, phi = min(pstart + hi, a.pos1);
+    const int nb = KP_SEQ_TILE + k - 1;
+    double acc = 0.0;
+    unsigned long long cnt = 0;
+    for (unsigned long long t0 = pstart + lo / KP_SEQ_TILE * KP_SEQ_TILE; t0 < phi; t0 += KP_SEQ_TILE) {
+        __syncthreads();
+        // stage the codes of record bytes [t0 - c, t0 - c + nb) with aligned 16-byte loads; bytes outside the
+        // record (or outside the call's bytes, which no window of [pos0, pos1) reaches) are code 4
+        const long long g0 = (long long)t0 - a.c - (long long)a.seq_base;
+        const long long ga = g0 >= 0 ? (g0 & ~15LL) : -((-g0 + 15) & ~15LL);
+        const int nvec = (int)((g0 + nb - ga + 15) >> 4);
+        for (int v = tid; v < nvec; v += blockDim.x) {
+            const long long gi = ga + 16LL * v;
+            uint4 w = make_uint4(0, 0, 0, 0);
+            if (gi >= 0 && gi < (long long)a.seq_len) w = *(const uint4 *)(a.seq + gi);
+            const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+            for (int b = 0; b < 16; b++) {
+                const long long q = gi + b - g0, g = gi + b;
+                if (q >= 0 && q < nb)
+                    s_code[q] = g >= 0 && g < (long long)a.seq_len ? kp_seq_code((ws[b >> 2] >> (8 * (b & 3))) & 0xFFu) : 4;
+            }
+        }
+        __syncthreads();
+        for (int jj = 0; jj < KP_SEQ_TILE / KP_SEQ_THREADS; jj++) {
+            const int p = jj * KP_SEQ_THREADS + tid;
+            const unsigned long long i = t0 + p;
+            const bool in = i >= plo && i < phi;
+            uint32_t kf = 0, bf = 0, kr = 0, br = 0, cor = 0;
+            if (in) {
+#pragma unroll 4
+                for (int j = 0; j < k; j++) {
+                    const int cd = s_code[p + j];
+                    cor |= cd;
+                    const uint32_t of = s_off[0][j][cd];
+                    kf += of;
+                    bf |= of;
+                    if (BOTH) {
+                        const uint32_t orv = s_off[1][j][cd];
+                        kr += orv;
+                        br |= orv;
+                    }
+                }
+            }
+            const bool ctx = in && !(cor & 4u);
+            const bool mf = ctx && !(bf >> 31), mr = BOTH && ctx && !(br >> 31);
+            const double rf = mf ? a.kmer_rate[kf] : 0.0, rr = mr ? a.kmer_rate[kr] : 0.0;
+            const double r = rf + rr;
+            acc += r;
+            cnt += (unsigned)mf + (unsigned)mr;
+            if (a.track && in) a.track[i - a.pos0] = ctx ? __double2float_rn(r) : __int_as_float(0x7fc00000);
+            if (a.counts) {
+                const bool use = in && (!a.count_mask || ((a.count_mask[(i - a.pos0) >> 5] >> ((i - a.pos0) & 31)) & 1u));
+                kp_seq_count(a.counts, mf && use, kf);
+                if (BOTH) kp_seq_count(a.counts, mr && use, kr);
+            }
+        }
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        acc += __shfl_down_sync(0xFFFFFFFFu, acc, d);
+        cnt += __shfl_down_sync(0xFFFFFFFFu, cnt, d);
+    }
+    if (lane == 0) {
+        s_wsum[warp] = acc;
+        s_wn[warp] = cnt;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double s = 0.0;
+        unsigned long long c = 0;
+        for (int w = 0; w < KP_SEQ_THREADS / 32; w++) {
+            s += s_wsum[w];
+            c += s_wn[w];
+        }
+        a.sum[blockIdx.x] = s;
+        a.n[blockIdx.x] = c;
+    }
+}
+
+// region r = (first piece pa, last piece pb, task of pa or -1, task of pb or -1): the left-to-right float64 sum of its
+// clipped piece sums (a task's sum where the region clips the piece, the piece's own sum where it covers it)
+__global__ void kp_region_sum_kernel(const double *psum, const unsigned long long *pn, const double *tsum,
+                                     const unsigned long long *tn, const long long *reg, unsigned long long n, double *out,
+                                     unsigned long long *out_n)
+{
+    for (unsigned long long r = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; r < n;
+         r += (unsigned long long)gridDim.x * blockDim.x) {
+        const long long pa = reg[4 * r], pb = reg[4 * r + 1], ta = reg[4 * r + 2], tb = reg[4 * r + 3];
+        double s = 0.0;
+        unsigned long long c = 0;
+        for (long long q = pa; q <= pb; q++) {
+            if (q == pa && ta >= 0) { s += tsum[ta]; c += tn[ta]; }
+            else if (q == pb && tb >= 0) { s += tsum[tb]; c += tn[tb]; }
+            else { s += psum[q]; c += pn[q]; }
+        }
+        out[r] = s;
+        out_n[r] = c;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
 // test hooks
 // ---------------------------------------------------------------------------------------------------
 __global__ void kp_debug_log_kernel(const double *x, double *y, unsigned long long n)

@@ -292,6 +292,37 @@ class PartitionPlan:
                                           M.ctypes.data, U.ctypes.data, t.ctypes.data, self._stream()), "kp_partition_score")
         return (M, U, t) if owner is None else (M, U, t, kmer_rate[: self.nkmer])
 
+    # -- applying a partition along sequences (DESIGN §4c) ---------------------------------------
+    SEQ_PIECE = 1 << 16   # positions per piece of a record (kp_seq_scan)
+
+    def kmer_rates(self, owner, rates, name="apply"):
+        """float64 device tensor: the rate of every k-mer's owner (kp_kmer_rates)."""
+        torch = _torch()
+        rates = np.ascontiguousarray(rates, dtype=np.float64)
+        out = self._buffer(name + "_kmer_rate", self.nkmer, torch.float64)
+        check(self.lib.kp_kmer_rates(self.handle, owner.data_ptr(), rates.ctypes.data, rates.size, out.data_ptr(),
+                                     self._stream()), "kp_kmer_rates")
+        return out[: self.nkmer]
+
+    def seq_scan(self, seq, seq_base, seq_len, rec_len, pos0, pos1, kmer_rate, both, out_sum, out_n, tasks=None,
+                 track=None, count_mask=None, counts=None):
+        """One kp_seq_scan call on the stream, without waiting.  seq: uint8 device tensor whose first seq_len bytes are
+        the record bytes from seq_base on (at least 16 more bytes allocated); out_sum (float64) / out_n (int64): device tensors with one entry per piece of [pos0, pos1), or per
+        row of tasks (int32/uint32 device tensor [ntask, 3]); track: float32 device tensor of pos1 - pos0 entries;
+        count_mask: int32 device tensor of bits; counts: int64 device tensor [nkmer]."""
+        ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
+        ntask = 0 if tasks is None else int(tasks.shape[0])
+        check(self.lib.kp_seq_scan(self.handle, seq.data_ptr(), int(seq_base), int(seq_len), int(rec_len), int(pos0),
+                                   int(pos1), int(bool(both)), kmer_rate.data_ptr(), ptr(tasks), ntask, out_sum.data_ptr(),
+                                   out_n.data_ptr(), ptr(track), ptr(count_mask), ptr(counts), self._stream()), "kp_seq_scan")
+
+    def region_sums(self, piece_sum, piece_n, task_sum, task_n, regions, out_sum, out_n):
+        """kp_region_sums on the stream, without waiting.  regions: int64 device tensor [n, 4]."""
+        ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
+        check(self.lib.kp_region_sums(self.handle, piece_sum.data_ptr(), piece_n.data_ptr(), ptr(task_sum), ptr(task_n),
+                                      regions.data_ptr(), int(regions.shape[0]), out_sum.data_ptr(), out_n.data_ptr(),
+                                      self._stream()), "kp_region_sums")
+
     # -- dense views (tests, exports) ------------------------------------------------------------
     def gather(self, table, first=0, n=None):
         """float32 values of patterns first..first+n-1 (dense numbering) from a device table."""

@@ -108,16 +108,13 @@ class PartitionScore:
         self.__dict__.update(kw)
 
 
-def score(patterns, rates, contextD, device=None, per_kmer=False):
-    """Check that `patterns` partition their general pattern and score the counts contextD {kmer: (n_pos, n_neg)}.
-    Longer k-mers are collapsed around their centre to the patterns' length (as kmerpapa --test_smaller_k does);
-    k-mers of the partition that contextD lacks count as zero.  Raises PartitionError naming the first k-mer that is
-    covered twice or not at all, or a test k-mer outside the general pattern."""
-    from .algorithms.bottum_up_array_w_numba import kmer_arrays
+def assign(patterns, device=None):
+    """Check on the GPU that `patterns` partition their general pattern (their LCA).  Returns (gen_pat, plan, patnums,
+    owner): the lite plan of the general pattern, the dense pattern numbers and the device owner table of
+    PartitionPlan.partition_assign.  Raises PartitionError naming the first k-mer that is covered twice or not at all."""
     from .engine import get_plan
 
     gen_pat = iupac.lca_pattern(patterns)
-    k = len(gen_pat)
     plan = get_plan(gen_pat, device, lite=True)
     patnums = pattern_numbers(patterns, gen_pat)
     owner, conflict, uncovered = plan.partition_assign(patnums)
@@ -129,6 +126,18 @@ def score(patterns, rates, contextD, device=None, per_kmer=False):
     if uncovered is not None:
         raise PartitionError(f"the patterns leave a gap: k-mer {iupac.kmer_of_index(gen_pat, uncovered)} of their general "
                              f"pattern {gen_pat} is in none of them")
+    return gen_pat, plan, patnums, owner
+
+
+def score(patterns, rates, contextD, device=None, per_kmer=False):
+    """Check that `patterns` partition their general pattern and score the counts contextD {kmer: (n_pos, n_neg)}.
+    Longer k-mers are collapsed around their centre to the patterns' length (as kmerpapa --test_smaller_k does);
+    k-mers of the partition that contextD lacks count as zero.  Raises PartitionError naming the first k-mer that is
+    covered twice or not at all, or a test k-mer outside the general pattern."""
+    from .algorithms.bottum_up_array_w_numba import kmer_arrays
+
+    gen_pat, plan, patnums, owner = assign(patterns, device)
+    k = len(gen_pat)
     if not contextD:
         raise PartitionError("the input has no k-mers")
     have = len(next(iter(contextD)))
