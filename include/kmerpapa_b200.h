@@ -233,8 +233,10 @@ int kp_pattern_offset(const kp_plan *plan, uint64_t patnum, uint64_t *table_elem
 
 /* Number of kernel launches issued through this plan so far (for bench.py's gpu_launches). */
 uint64_t kp_plan_launch_count(const kp_plan *plan);
-/* Name of the kernel family kp_dp_single / kp_dp_cv_job launch for this plan (reports, bench.py's roofline.kernel). */
-const char *kp_dp_kernel_name(const kp_plan *plan);
+/* Name of the kernel family kp_dp_single / kp_dp_cv_job launch for this plan at one count width (reports, bench.py's
+ * roofline.kernel): wide = 0 for a max_count of at most 2^32 - 1 (32-bit on-chip counts), wide != 0 above.  The fiber
+ * kernel needs more shared memory for 64-bit counts, so the two widths can run different families. */
+const char *kp_dp_kernel_name(const kp_plan *plan, int wide);
 
 /* ---------------------------------------------------------------------------------------------------
  * One DP sharded over the GPUs of a node (SURVEY 8f.3: pattern-space sharding; the reference has no

@@ -67,7 +67,7 @@ SYMBOLS = {
     "kp_region_sums": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _vp, _vp]),
     "kp_pattern_offset":(_int, [_vp, _u64, ctypes.POINTER(_u64), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_uint32)]),
     "kp_plan_launch_count": (_u64, [_vp]),
-    "kp_dp_kernel_name": (_cp, [_vp]),
+    "kp_dp_kernel_name": (_cp, [_vp, _int]),
     "kp_shard_assignment": (_int, [_vp, _int, _vp, _vp]),
     "kp_shard_create": (_int, [_vp, _int, _int, _int, ctypes.POINTER(_vp)]),
     "kp_shard_destroy": (_int, [_vp]),

@@ -292,9 +292,9 @@ int kp_plan_get_info(const kp_plan *p, kp_plan_info *o)
 
 uint64_t kp_plan_launch_count(const kp_plan *p) { return p ? p->launches : 0; }
 
-const char *kp_dp_kernel_name(const kp_plan *p)
+const char *kp_dp_kernel_name(const kp_plan *p, int wide)
 {
-    return p && p->use_fiber && p->fiber_smem[0] ? "kp_dp_fiber_kernel" : "kp_dp_rows_kernel";
+    return p && p->use_fiber && p->fiber_smem[wide != 0] ? "kp_dp_fiber_kernel" : "kp_dp_rows_kernel";
 }
 
 int kp_pattern_offset(const kp_plan *p, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit)
@@ -1542,7 +1542,7 @@ int kp_greedy(kp_plan *p, const int64_t *d_kmerM, const int64_t *d_kmerU, const 
     for (int d = 0; d < levels && d < 64; d++) {
         kp_greedy_marginals_kernel<<<grid, 256, 0, st>>>(p->d_tab, (const long long *)d_kmerM, (const long long *)d_kmerU,
                                                          (const long long *)d_testM, (const long long *)d_testU, d,
-                                                         (d & 1) ? fb : fa, (d & 1) ? sb : sa, ctr, big, acc);
+                                                         (d & 1) ? fb : fa, (d & 1) ? sb : sa, ctr, big, cap, acc);
         kp_greedy_decide_kernel<<<grid, 256, 0, st>>>(p->d_tab, d_testM != nullptr, alpha, beta, penalty, d, (d & 1) ? fb : fa,
                                                       (d & 1) ? sb : sa, (d & 1) ? fa : fb, (d & 1) ? sa : sb, leaves, cap, ctr,
                                                       acc);

@@ -1227,7 +1227,7 @@ __global__ void __launch_bounds__(256) kp_backtrack_level_kernel(const KpTables 
                                                                  KpBtNode *leaves, unsigned long long cap,
                                                                  unsigned long long *ctr)
 {
-    kp_backtrack_level(*tab, rowtab, vw, depth, cur, nxt, leaves, cap, ctr, ctr[2 + depth]);
+    kp_backtrack_level(*tab, rowtab, vw, depth, cur, nxt, leaves, cap, ctr, ctr[2 + depth] < cap ? ctr[2 + depth] : cap);
 }
 
 // All depths in one launch (cooperative launch: every CTA is resident), a grid-wide barrier between depths:
@@ -1306,13 +1306,15 @@ __global__ void __launch_bounds__(256) kp_greedy_marginals_kernel(const KpTables
                                                                   const long long *testM, const long long *testU, int depth,
                                                                   const KpBtNode *cur, const unsigned long long *cur_size,
                                                                   const unsigned long long *ctr, unsigned long long big,
-                                                                  unsigned long long *acc)
+                                                                  unsigned long long cap, unsigned long long *acc)
 {
     const KpTables &tb = *tab;
     __shared__ unsigned long long marg[KP_GREEDY_ACC];
     __shared__ uint8_t s_bases[KP_MAXPOS][4];
     __shared__ uint32_t s_n[KP_MAXPOS];
-    const unsigned long long ncur = ctr[2 + depth];
+    // the frontier counter keeps counting past cap when a depth overflows (ctr[1] is set, the host retries with a larger
+    // workspace): only the first cap nodes exist
+    const unsigned long long ncur = ctr[2 + depth] < cap ? ctr[2 + depth] : cap;
     const int npos = tb.npos;
     for (unsigned long long ni = 0; ni < ncur; ni++) {
         const unsigned long long total = cur_size[ni];   // k-mers of the node
@@ -1376,7 +1378,7 @@ __global__ void __launch_bounds__(256) kp_greedy_decide_kernel(const KpTables *t
     for (int i = threadIdx.x; i < 128; i += blockDim.x) logtab[i] = make_double2(kpc_logTab[2 * i], kpc_logTab[2 * i + 1]);
     __syncthreads();
     const KpLogK K = kp_logk_load();
-    const unsigned long long ncur = ctr[2 + depth];
+    const unsigned long long ncur = ctr[2 + depth] < cap ? ctr[2 + depth] : cap;   // as in kp_greedy_marginals_kernel
     const int npos = tb.npos, lane = threadIdx.x & 31;
     const unsigned long long nw = (unsigned long long)gridDim.x * (blockDim.x >> 5);
     for (unsigned long long ni = (unsigned long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); ni < ncur; ni += nw) {

@@ -80,9 +80,10 @@ class PartitionPlan:
         if prefix is None or prefix == "cv":
             self._cv_state = None
 
-    def dp_kernel_name(self):
-        """Name of the kernel family kp_dp_single / kp_dp_cv_job launch for this plan (for reports)."""
-        return self.lib.kp_dp_kernel_name(self.handle).decode()
+    def dp_kernel_name(self, wide=False):
+        """Name of the kernel family kp_dp_single / kp_dp_cv_job launch for this plan (for reports), for a max_count of
+        at most 2^32 - 1 or, with wide=True, above it."""
+        return self.lib.kp_dp_kernel_name(self.handle, int(bool(wide))).decode()
 
     @property
     def launches(self):

@@ -20,7 +20,7 @@ def _plan(gen_pat, kernel, monkeypatch):
 
     monkeypatch.setenv("KP_DP_KERNEL", kernel)
     plan = PartitionPlan(gen_pat)
-    assert plan.dp_kernel_name() == f"kp_dp_{kernel}_kernel", (gen_pat, plan.dp_kernel_name())
+    assert plan.dp_kernel_name(wide=False) == f"kp_dp_{kernel}_kernel", (gen_pat, plan.dp_kernel_name())
     return plan
 
 
@@ -47,29 +47,39 @@ def _codes(gen_pat):
     return np.array([iupac.kmer_code(k) for k in iupac.matches(gen_pat)], dtype=np.uint64)
 
 
-@pytest.mark.parametrize("regime", ["dense", "sparse", "ties", "negative_penalty"])
+@pytest.mark.parametrize("regime", ["dense", "sparse", "ties", "negative_penalty", "narrow_top", "wide_edge", "wide"])
 @pytest.mark.parametrize("gen_pat", SHAPES)
 def test_fiber_kernel_against_oracle(oracle, monkeypatch, gen_pat, regime):
-    M, U = _counts(gen_pat, 77 + len(gen_pat), "dense" if regime == "negative_penalty" else regime)
-    alpha, penalty = {"ties": (1.0, 0.5), "negative_penalty": (10.0, -3.0)}.get(regime, (0.8, 4.0))
+    """The count bands of test_gpu_count_scale (totals 2^32 - 1, 2^32 and 2^33..2^40) run with max_count = the true
+    total, so the band selects the count width; the fiber kernel runs at both widths on every shape."""
+    from test_gpu_count_scale import GRID, band_counts
+
+    if regime in ("narrow_top", "wide_edge", "wide"):
+        M, U, _ = band_counts(regime, len(_codes(gen_pat)), 77 + len(gen_pat))
+        grid = GRID
+    else:
+        M, U = _counts(gen_pat, 77 + len(gen_pat), "dense" if regime == "negative_penalty" else regime)
+        grid = ({"ties": (1.0, 0.5), "negative_penalty": (10.0, -3.0)}.get(regime, (0.8, 4.0)),)
     mc = int(M.sum() + U.sum())
-    mu = max(int(M.sum()), 1) / max(mc, 2)
-    beta = alpha * (1.0 - mu) / mu
     plan = _plan(gen_pat, "fiber", monkeypatch)
+    assert plan.dp_kernel_name(wide=True) == "kp_dp_fiber_kernel", gen_pat
     kM, kU = plan.pack_counts(_codes(gen_pat), M, U)
     eM, eU = plan.expand(kM, kU)
-    best, kept = plan.dp_single(eM, eU, mc, alpha, beta, penalty)
-    ref = oracle.single_dp(gen_pat, M, U, alpha, beta, penalty)
-    got = plan.gather(best)
-    bad = np.flatnonzero(_bits(got) != _bits(ref["score"]))
-    assert bad.size == 0, f"{bad.size} of {got.size} scores differ, first {bad[:8]}"
-    codes = plan.split_codes(best, kept, np.arange(plan.npat, dtype=np.uint64))
-    assert np.array_equal(codes, ref["split"])
-    assert np.array_equal(plan.gather_kept(kept) == 1, ref["split"] == 0xFF)
-    assert np.array_equal(plan.backtrack(best, kept), oracle.backtrack(gen_pat, ref["split"]))
-    # the 64-bit on-chip count path (selected by max_count) gives the same table
-    best64, _ = plan.dp_single(eM, eU, 1 << 40, alpha, beta, penalty)
-    assert np.array_equal(_bits(plan.gather(best64)), _bits(ref["score"]))
+    for alpha, penalty in grid:
+        mu = max(int(M.sum()), 1) / max(mc, 2)
+        beta = alpha * (1.0 - mu) / mu
+        best, kept = plan.dp_single(eM, eU, mc, alpha, beta, penalty)
+        ref = oracle.single_dp(gen_pat, M, U, alpha, beta, penalty)
+        got = plan.gather(best)
+        bad = np.flatnonzero(_bits(got) != _bits(ref["score"]))
+        assert bad.size == 0, f"{bad.size} of {got.size} scores differ, first {bad[:8]}"
+        codes = plan.split_codes(best, kept, np.arange(plan.npat, dtype=np.uint64))
+        assert np.array_equal(codes, ref["split"])
+        assert np.array_equal(plan.gather_kept(kept) == 1, ref["split"] == 0xFF)
+        assert np.array_equal(plan.backtrack(best, kept), oracle.backtrack(gen_pat, ref["split"]))
+        # the 64-bit on-chip count path (selected by max_count) gives the same table
+        best64, _ = plan.dp_single(eM, eU, 1 << 40, alpha, beta, penalty)
+        assert np.array_equal(_bits(plan.gather(best64)), _bits(ref["score"]))
 
 
 @pytest.mark.parametrize("gen_pat", ["NNNNN", "RNNNNY", "NNNNNN"])

@@ -75,6 +75,13 @@ def test_device_leaf_score_is_scipy(eng):
     M = rng.binomial(U, rng.random(n) * 0.6)
     M[:1000] = 0
     U[500:1500] = 0
+    # genome-scale counts up to 2^50, a quarter of them with M >= 2^32
+    Ub = (2.0 ** rng.uniform(31, 50, n // 2)).astype(np.int64)
+    Mb = rng.binomial(Ub, np.exp(rng.uniform(np.log(1e-4), np.log(0.6), n // 2)))
+    Mb[: n // 8] = (2.0 ** rng.uniform(32, 50, n // 8)).astype(np.int64)
+    U, M = np.concatenate([U, Ub]), np.concatenate([M, Mb])
+    n = U.size
+    assert (M >= 2 ** 32).sum() >= n // 8 and max(M.max(), U.max()) < 2 ** 50
     alpha, beta, pen = 0.8, 1234.5, 5.0
     out = np.empty(n, dtype=np.float64)
     M64, U64 = M.astype(np.int64), U.astype(np.int64)
@@ -177,18 +184,23 @@ def test_random_against_oracle(eng, oracle, gen_pat, seed):
 
 
 @pytest.mark.parametrize("regime", ["rate_near_one", "half", "tiny_counts", "huge_counts", "zeros", "penalty_ties", "low_rates",
-                                    "kept_whole", "negative_penalty"])
+                                    "kept_whole", "negative_penalty", "narrow_top", "wide_edge", "wide"])
 @pytest.mark.parametrize("gen_pat", ["NNNNN", "NNMNNN", "NNNNNN"])
 def test_count_regimes_against_oracle(eng, oracle, gen_pat, regime):
     """Regimes that stress the score filter (a float32 bound decides whether the exact FP64 score is computed): rates
     near 1 (absolute error of the fast log), rates around 1/2, counts of a few units, counts near 2^31, mostly empty
     tables, penalties that make many self-scores tie with split sums, and negative penalties (the filter's estimate
-    pen + t1 + t2 then cancels).  Full table + split codes vs the oracle."""
+    pen + t1 + t2 then cancels).  The count bands of test_gpu_count_scale (totals 2^32 - 1, 2^32 and 2^33..2^40) run with
+    max_count = the true total, so the band selects the count width.  Full table + split codes vs the oracle."""
     import zlib
+
+    from test_gpu_count_scale import GRID, band_counts
 
     rng = np.random.default_rng(zlib.crc32((gen_pat + regime).encode()))
     _, nk, _ = oracle.plan_info(gen_pat)
-    if regime == "rate_near_one":
+    if regime in ("narrow_top", "wide_edge", "wide"):
+        M, U, _ = band_counts(regime, nk, zlib.crc32((gen_pat + regime).encode()))
+    elif regime == "rate_near_one":
         M = rng.integers(10 ** 5, 10 ** 6, size=nk)
         U = rng.integers(0, 30, size=nk) * (rng.random(nk) < 0.5)
     elif regime == "half":
@@ -216,7 +228,8 @@ def test_count_regimes_against_oracle(eng, oracle, gen_pat, regime):
         M = np.full(nk, 10)
     U[0], M[0] = max(U[0], 5), max(M[0], 1)
     grid = {"penalty_ties": ((1.0, 0.0), (1.0, 2.0)), "kept_whole": ((1.0, 1e6), (0.01, 3e3)),
-            "negative_penalty": ((1.0, -0.5), (10.0, -3.0))}.get(regime, ((1.0, 4.0), (0.5, 0.0)))
+            "negative_penalty": ((1.0, -0.5), (10.0, -3.0)), "narrow_top": GRID, "wide_edge": GRID,
+            "wide": GRID}.get(regime, ((1.0, 4.0), (0.5, 0.0)))
     for alpha, pen in grid:
         mu = M.sum() / (M.sum() + U.sum())
         beta = alpha * (1 - mu) / mu
@@ -310,9 +323,12 @@ def test_pack_counts_sums_duplicates_and_rejects_bad_codes(eng):
                                           ("A", 7), ("NTNBN", 8)])
 def test_greedy_against_oracle(eng, oracle, gen_pat, seed):
     """kp_greedy (one launch per depth, one CTA per pattern) against the plain-Python restatement of the reference's
-    greedy recursion: same leaves in the same order, float64 losses / held-out LLs / score bit for bit."""
+    greedy recursion: same leaves in the same order, float64 losses / held-out LLs / score bit for bit, at small counts
+    and at totals on both sides of 2^32."""
     from kmerpapa_b200 import iupac
     from kmerpapa_b200.algorithms import greedy_penalty_plus_pseudo as gr
+
+    from test_gpu_count_scale import band_counts
 
     rng = np.random.default_rng(seed)
     km = oracle.kmers_of(gen_pat)
@@ -320,20 +336,22 @@ def test_greedy_against_oracle(eng, oracle, gen_pat, seed):
     M = rng.binomial(np.maximum(U, 1), 0.03)
     if M.sum() == 0:
         M[0] = 3
-    Mt, Ut = rng.binomial(M, 0.3), rng.binomial(U, 0.3)
     plan = eng.get_plan(gen_pat)
     PE = iupac.PatternEnumeration(gen_pat)
-    for alpha, pen in ((0.8, 4.0), (10.0, 0.5), (1.0, 30.0)):
-        mu = M.sum() / (M.sum() + U.sum())
-        beta = (alpha * (1.0 - mu)) / mu
-        kM, kU = plan.upload_kmer_tables(M - Mt, U - Ut, name="g_tr")
-        tM, tU = plan.upload_kmer_tables(Mt, Ut, name="g_te")
-        pats, loss, tst, score = gr._greedy(plan, kM, kU, alpha, beta, pen, test=(tM, tU))
-        rscore, rnames, rloss, rtest = oracle.greedy(gen_pat, M - Mt, U - Ut, alpha, beta, pen, Mt, Ut)
-        assert [PE.num2pattern(p) for p in pats] == rnames
-        assert np.array_equal(loss.view(np.uint64), np.array(rloss, dtype=np.float64).view(np.uint64))
-        assert np.array_equal(tst.view(np.uint64), np.array(rtest, dtype=np.float64).view(np.uint64))
-        assert np.float64(score).tobytes() == np.float64(rscore).tobytes()
+    # the same shapes at genome-scale counts: a total of 2^32 - 1 and one of 2^33..2^40 (test_gpu_count_scale's bands)
+    for M, U in [(M, U)] + [band_counts(band, len(km), seed)[:2] for band in ("narrow_top", "wide")]:
+        Mt, Ut = rng.binomial(M, 0.3), rng.binomial(U, 0.3)
+        for alpha, pen in ((0.8, 4.0), (10.0, 0.5), (1.0, 30.0)):
+            mu = M.sum() / (M.sum() + U.sum())
+            beta = (alpha * (1.0 - mu)) / mu
+            kM, kU = plan.upload_kmer_tables(M - Mt, U - Ut, name="g_tr")
+            tM, tU = plan.upload_kmer_tables(Mt, Ut, name="g_te")
+            pats, loss, tst, score = gr._greedy(plan, kM, kU, alpha, beta, pen, test=(tM, tU))
+            rscore, rnames, rloss, rtest = oracle.greedy(gen_pat, M - Mt, U - Ut, alpha, beta, pen, Mt, Ut)
+            assert [PE.num2pattern(p) for p in pats] == rnames
+            assert np.array_equal(loss.view(np.uint64), np.array(rloss, dtype=np.float64).view(np.uint64))
+            assert np.array_equal(tst.view(np.uint64), np.array(rtest, dtype=np.float64).view(np.uint64))
+            assert np.float64(score).tobytes() == np.float64(rscore).tobytes()
 
 
 def test_lattice_free_plan(eng):
