@@ -228,6 +228,32 @@ int kp_seq_scan(kp_plan *plan, const uint8_t *d_seq, uint64_t seq_base, uint64_t
 int kp_region_sums(kp_plan *plan, const double *d_piece_sum, const int64_t *d_piece_n, const double *d_task_sum,
                    const int64_t *d_task_n, const int64_t *d_regions, uint64_t n, double *d_sum, int64_t *d_n, void *stream);
 
+/* Counting the contexts of SNVs (DESIGN §4d; kmerpapa_b200/count_mutations.py), with the windows, matching and k-mer
+ * index of kp_seq_scan.  d_seq, seq_base, seq_len, rec_len, pos0, pos1 and both are as in kp_seq_scan, except that pos0
+ * need not be a multiple of 65536 and d_seq need not be aligned.  SNV t is at record position d_pos[t] (int64, in
+ * [pos0, pos1)) with d_ref_alt[t] = REF code | ALT code << 2 (A, C, G, T = 0..3).  d_status[t] gets the first that
+ * applies of:
+ *   KP_SNV_REF_MISMATCH     the genome byte is a base (either case) other than REF;
+ *   KP_SNV_OUTSIDE_REGIONS  bit pos - pos0 of d_count_mask (uint32 words; NULL: every position) is clear;
+ *   KP_SNV_NO_CONTEXT       the window leaves the record or holds a byte that is not a base;
+ *   KP_SNV_NO_MATCH         neither the forward window nor (both != 0) the reverse one matches;
+ *   KP_SNV_ALT_NOT_SELECTED alt_slot[a] < 0, where a is ALT when the forward window matches, else complement(ALT);
+ *   KP_SNV_COUNTED          d_counts[alt_slot[a] * nkmer + kidx] += 1 (int64, not zeroed here), with kidx the index of
+ *                           the forward window when it matches, else of the reverse one.
+ * A d_pos outside [pos0, pos1) gets KP_SNV_BAD_POSITION and touches nothing else.  alt_slot: 4 host ints, each -1..3.
+ * The counts are integer atomics, so they are the same whatever the thread order and the split into calls.  Does not
+ * synchronise. */
+#define KP_SNV_REF_MISMATCH 0
+#define KP_SNV_OUTSIDE_REGIONS 1
+#define KP_SNV_NO_CONTEXT 2
+#define KP_SNV_NO_MATCH 3
+#define KP_SNV_ALT_NOT_SELECTED 4
+#define KP_SNV_COUNTED 5
+#define KP_SNV_BAD_POSITION 255
+int kp_snv_counts(kp_plan *plan, const uint8_t *d_seq, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0,
+                  uint64_t pos1, int both, const int64_t *d_pos, const uint8_t *d_ref_alt, uint64_t n, const int *alt_slot,
+                  const uint32_t *d_count_mask, int64_t *d_counts, uint8_t *d_status, void *stream);
+
 /* Where a dense pattern number lives in the device layout: element of a float table, element and bit of d_kept. */
 int kp_pattern_offset(const kp_plan *plan, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit);
 

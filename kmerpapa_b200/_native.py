@@ -65,6 +65,7 @@ SYMBOLS = {
     "kp_kmer_rates": (_int, [_vp, _vp, _vp, _u64, _vp, _vp]),
     "kp_seq_scan": (_int, [_vp, _vp, _u64, _u64, _u64, _u64, _u64, _int, _vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "kp_region_sums": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _vp, _vp]),
+    "kp_snv_counts": (_int, [_vp, _vp, _u64, _u64, _u64, _u64, _u64, _int, _vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp]),
     "kp_pattern_offset":(_int, [_vp, _u64, ctypes.POINTER(_u64), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_uint32)]),
     "kp_plan_launch_count": (_u64, [_vp]),
     "kp_dp_kernel_name": (_cp, [_vp, _int]),

@@ -209,8 +209,12 @@ class Applier:
         self.ev = [None, None]
         self.nchunks = 0
 
-    def record(self, name, seq):
-        """Scan one record.  Returns its float32 track (numpy) when tracks are asked for, else None."""
+    def record(self, name, seq, on_chunk=None):
+        """Scan one record.  Returns its float32 track (numpy) when tracks are asked for, else None.  A record that has
+        no region, when regions are given and tracks are not asked for, is not scanned.  on_chunk(dseq, b0, b1, pos0,
+        pos1, mask) is called after the scan of each chunk is enqueued, on the same stream: dseq holds the record bytes
+        [b0, b1), which cover the windows of the positions [pos0, pos1), and mask is the region-union bit mask of those
+        positions (None without regions).  Work it enqueues on that stream may read both until it ends."""
         torch = self.torch
         if isinstance(seq, str):
             seq = seq.encode("ascii")
@@ -231,7 +235,7 @@ class Applier:
         else:
             starts, ends = np.zeros(1, np.int64), np.array([L], np.int64)
         with torch.cuda.device(self.dev):
-            out = self._scan(seq, L, starts, ends)
+            out = self._scan(seq, L, starts, ends, on_chunk)
         if self.regions is not None:
             if len(idx):
                 self.n_contexts[idx], self.expected[idx] = out[0], out[1]
@@ -239,7 +243,7 @@ class Applier:
             self.rows.append((name, 0, L, int(out[0][0]), float(out[1][0])))
         return out[2]
 
-    def _scan(self, seq, L, starts, ends):
+    def _scan(self, seq, L, starts, ends, on_chunk):
         torch, plan, P = self.torch, self.plan, PIECE
         stream = torch.cuda.current_stream(self.dev)
         npieces = (L + P - 1) // P
@@ -277,6 +281,8 @@ class Applier:
             if t1 > t0:
                 plan.seq_scan(self.dseq[slot], b0, b1 - b0, L, pos0, pos1, self.kmer_rate, self.both, tsum[t0:], tn[t0:],
                               tasks=dtasks[t0:t1])
+            if on_chunk is not None:
+                on_chunk(self.dseq[slot], b0, b1, pos0, pos1, mask)
             ev = torch.cuda.Event()
             ev.record(stream)
             self.ev[slot] = ev

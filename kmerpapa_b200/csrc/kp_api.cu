@@ -986,6 +986,50 @@ int kp_seq_scan(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t se
     return 0;
 }
 
+int kp_snv_counts(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0,
+                  uint64_t pos1, int both, const int64_t *d_pos, const uint8_t *d_ref_alt, uint64_t n, const int *alt_slot,
+                  const uint32_t *d_count_mask, int64_t *d_counts, uint8_t *d_status, void *stream)
+{
+    if (!p) return fail("kp_snv_counts: null plan");
+    const int k = p->host.k, c = k / 2;
+    if (!alt_slot) return fail("kp_snv_counts: null argument");
+    for (int a = 0; a < 4; a++)
+        if (alt_slot[a] < -1 || alt_slot[a] > 3) return fail("kp_snv_counts: an alt slot must be -1..3");
+    if (both && k % 2 == 0) return fail("kp_snv_counts: both strands need an odd k");
+    if (pos0 > pos1 || pos1 > rec_len) return fail("kp_snv_counts: bad position range");
+    if (n == 0) return 0;
+    if (!d_seq || !d_pos || !d_ref_alt || !d_counts || !d_status) return fail("kp_snv_counts: null argument");
+    if (((uintptr_t)d_pos & 7) || ((uintptr_t)d_counts & 7)) return fail("kp_snv_counts: d_pos and d_counts must be 8-byte aligned");
+    const uint64_t need_lo = pos0 >= (uint64_t)c ? pos0 - c : 0, need_hi = std::min<uint64_t>(rec_len, pos1 + (k - 1 - c));
+    if (pos1 > pos0 && (seq_base > need_lo || seq_base + seq_len < need_hi || seq_base + seq_len > rec_len))
+        return fail("kp_snv_counts: the sequence bytes do not cover the windows of the positions");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    KpSnvCount a;
+    a.seq = d_seq;
+    a.seq_base = seq_base;
+    a.seq_len = seq_len;
+    a.rec_len = rec_len;
+    a.pos0 = pos0;
+    a.pos1 = pos1;
+    a.pos = (const long long *)d_pos;
+    a.ref_alt = d_ref_alt;
+    a.n = n;
+    a.nkmer = p->host.nkmer;
+    for (int x = 0; x < 4; x++) a.alt_slot[x] = alt_slot[x];
+    a.count_mask = d_count_mask;
+    a.counts = (unsigned long long *)d_counts;
+    a.status = d_status;
+    a.k = k;
+    a.c = c;
+    const int grid = grid_for(n, 256, p->sm_count);
+    if (both) kp_snv_count_kernel<true><<<grid, 256, 0, st>>>(p->d_tab, p->d_genmask, a);
+    else kp_snv_count_kernel<false><<<grid, 256, 0, st>>>(p->d_tab, p->d_genmask, a);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
 int kp_region_sums(kp_plan *p, const double *d_piece_sum, const int64_t *d_piece_n, const double *d_task_sum,
                    const int64_t *d_task_n, const int64_t *d_regions, uint64_t n, double *d_sum, int64_t *d_n, void *stream)
 {

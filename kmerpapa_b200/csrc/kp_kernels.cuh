@@ -1883,6 +1883,38 @@ __device__ __forceinline__ uint8_t kp_seq_code(unsigned byte)
     return u == 'a' ? 0 : u == 'c' ? 1 : u == 'g' ? 2 : u == 't' ? 3 : 4;
 }
 
+// off[strand][j][code] for a window of k bases: the k-mer index contribution of base code (0..3; 4 = not a base) at
+// window position j, KP_SEQ_BAD where the pattern does not allow it.  Reverse strand: window byte j is base k-1-j of the
+// reverse complement (the complement of code cd is 3 - cd).  Every thread of the block calls it; the caller syncs.
+__device__ __forceinline__ void kp_seq_fill_offsets(uint32_t (*off)[KP_MAXK][8], const KpTables &tb, const uint8_t *gen_mask,
+                                                    int k, int tid)
+{
+    for (int x = tid; x < KP_MAXK * 8; x += blockDim.x) {
+        const int j = x >> 3, cd = x & 7;
+        off[0][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, j, cd) : KP_SEQ_BAD;
+        off[1][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, k - 1 - j, cd < 4 ? 3 - cd : cd) : KP_SEQ_BAD;
+    }
+}
+
+// The sum over a window of the offset table off[strand][j][code] of kp_seq_fill_offsets, for the window whose byte j has
+// base code CODE(j): kf (kr) becomes the forward (reverse, BOTH only) k-mer index, bf (br) the OR of the offsets (bit 31
+// set: a base the pattern does not allow) and cor the OR of the codes (bit 2 set: a byte that is not a base).  The
+// caller zeroes the five.  A macro rather than a function: written out this way it compiles to the same scan kernel as
+// the loop it replaced, where an inlined function changed the forward scan's instruction schedule.
+#define KP_SEQ_WINDOW(BOTH, off, k, CODE, kf, bf, kr, br, cor)                                                        \
+    _Pragma("unroll 4") for (int j = 0; j < (k); j++) {                                                                \
+        const int cd = CODE(j);                                                                                        \
+        cor |= cd;                                                                                                     \
+        const uint32_t of = off[0][j][cd];                                                                             \
+        kf += of;                                                                                                      \
+        bf |= of;                                                                                                      \
+        if (BOTH) {                                                                                                    \
+            const uint32_t orv = off[1][j][cd];                                                                        \
+            kr += orv;                                                                                                 \
+            br |= orv;                                                                                                 \
+        }                                                                                                              \
+    }
+
 // one count per lane that wants one, aggregated over the lanes of equal index (every lane of the warp calls it)
 __device__ __forceinline__ void kp_seq_count(unsigned long long *counts, bool want, uint32_t kidx)
 {
@@ -1902,12 +1934,7 @@ __global__ void __launch_bounds__(KP_SEQ_THREADS) kp_seq_scan_kernel(const KpTab
     __shared__ unsigned long long s_wn[KP_SEQ_THREADS / 32];
     const KpTables &tb = *tab;
     const int k = a.k, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int x = tid; x < KP_MAXK * 8; x += blockDim.x) {
-        const int j = x >> 3, cd = x & 7;
-        // reverse strand: window byte j is base k-1-j of the reverse complement (complement of code cd is 3 - cd)
-        s_off[0][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, j, cd) : KP_SEQ_BAD;
-        s_off[1][j][cd] = j < k ? kp_seq_offset(tb, gen_mask, k - 1 - j, cd < 4 ? 3 - cd : cd) : KP_SEQ_BAD;
-    }
+    kp_seq_fill_offsets(s_off, tb, gen_mask, k, tid);
     unsigned long long piece, lo = 0, hi = KP_SEQ_PIECE;
     if (a.tasks) {
         piece = a.tasks[3 * blockIdx.x];
@@ -1946,19 +1973,9 @@ __global__ void __launch_bounds__(KP_SEQ_THREADS) kp_seq_scan_kernel(const KpTab
             const bool in = i >= plo && i < phi;
             uint32_t kf = 0, bf = 0, kr = 0, br = 0, cor = 0;
             if (in) {
-#pragma unroll 4
-                for (int j = 0; j < k; j++) {
-                    const int cd = s_code[p + j];
-                    cor |= cd;
-                    const uint32_t of = s_off[0][j][cd];
-                    kf += of;
-                    bf |= of;
-                    if (BOTH) {
-                        const uint32_t orv = s_off[1][j][cd];
-                        kr += orv;
-                        br |= orv;
-                    }
-                }
+#define KP_SCAN_CODE(j) s_code[p + (j)]
+                KP_SEQ_WINDOW(BOTH, s_off, k, KP_SCAN_CODE, kf, bf, kr, br, cor)
+#undef KP_SCAN_CODE
             }
             const bool ctx = in && !(cor & 4u);
             const bool mf = ctx && !(bf >> 31), mr = BOTH && ctx && !(br >> 31);
@@ -1992,6 +2009,72 @@ __global__ void __launch_bounds__(KP_SEQ_THREADS) kp_seq_scan_kernel(const KpTab
         }
         a.sum[blockIdx.x] = s;
         a.n[blockIdx.x] = c;
+    }
+}
+
+// Counting the contexts of SNVs (kp_snv_counts, DESIGN §4d).  One thread per SNV reads its window from the record bytes
+// that kp_seq_scan reads for the same positions, so the genome is uploaded once for both tables.
+struct KpSnvCount {
+    const uint8_t *seq;              // as KpSeqScan
+    unsigned long long seq_base, seq_len, rec_len;
+    unsigned long long pos0, pos1;   // the SNVs' positions lie in [pos0, pos1)
+    const long long *pos;            // [n] record positions
+    const uint8_t *ref_alt;          // [n] REF code | ALT code << 2 (A, C, G, T = 0..3)
+    unsigned long long n, nkmer;
+    int alt_slot[4];                 // ALT code -> table of counts, -1: not counted
+    const uint32_t *count_mask;      // bit i - pos0: position i is in the regions (null: every position)
+    unsigned long long *counts;      // [slot][nkmer]
+    uint8_t *status;                 // [n] KP_SNV_*
+    int k, c;
+};
+
+template <bool BOTH>
+__global__ void __launch_bounds__(256) kp_snv_count_kernel(const KpTables *tab, const uint8_t *gen_mask, KpSnvCount a)
+{
+    __shared__ uint32_t s_off[2][KP_MAXK][8];
+    kp_seq_fill_offsets(s_off, *tab, gen_mask, a.k, threadIdx.x);
+    __syncthreads();
+    for (unsigned long long t = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; t < a.n;
+         t += (unsigned long long)gridDim.x * blockDim.x) {
+        const long long i = a.pos[t];
+        uint8_t st;
+        if (i < (long long)a.pos0 || i >= (long long)a.pos1) {
+            st = KP_SNV_BAD_POSITION;
+        } else {
+            const unsigned ra = a.ref_alt[t], ref = ra & 3u, alt = (ra >> 2) & 3u;
+            const unsigned g = kp_seq_code(a.seq[i - (long long)a.seq_base]);
+            const unsigned long long d = (unsigned long long)i - a.pos0;
+            if (g < 4 && g != ref) {
+                st = KP_SNV_REF_MISMATCH;
+            } else if (a.count_mask && !((a.count_mask[d >> 5] >> (d & 31)) & 1u)) {
+                st = KP_SNV_OUTSIDE_REGIONS;
+            } else if (i < a.c || (unsigned long long)(i - a.c + a.k) > a.rec_len) {
+                st = KP_SNV_NO_CONTEXT;
+            } else {
+                const uint8_t *w = a.seq + (i - a.c - (long long)a.seq_base);
+                uint32_t kf = 0, bf = 0, kr = 0, br = 0, cor = 0;
+#define KP_SNV_CODE(j) kp_seq_code(w[j])
+                KP_SEQ_WINDOW(BOTH, s_off, a.k, KP_SNV_CODE, kf, bf, kr, br, cor)
+#undef KP_SNV_CODE
+                const bool mf = !(bf >> 31), mr = BOTH && !(br >> 31);
+                if (cor & 4u) {
+                    st = KP_SNV_NO_CONTEXT;
+                } else if (!mf && !mr) {
+                    st = KP_SNV_NO_MATCH;
+                } else {
+                    // the reverse window reads the complement strand, where the ALT base is its complement
+                    const unsigned x = mf ? alt : 3u - alt;   // selects, not an indexed load that puts `a` on the stack
+                    const int slot = x == 0 ? a.alt_slot[0] : x == 1 ? a.alt_slot[1] : x == 2 ? a.alt_slot[2] : a.alt_slot[3];
+                    if (slot < 0) {
+                        st = KP_SNV_ALT_NOT_SELECTED;
+                    } else {
+                        atomicAdd(a.counts + (unsigned long long)slot * a.nkmer + (mf ? kf : kr), 1ull);
+                        st = KP_SNV_COUNTED;
+                    }
+                }
+            }
+        }
+        a.status[t] = st;
     }
 }
 

@@ -317,6 +317,23 @@ class PartitionPlan:
                                    int(pos1), int(bool(both)), kmer_rate.data_ptr(), ptr(tasks), ntask, out_sum.data_ptr(),
                                    out_n.data_ptr(), ptr(track), ptr(count_mask), ptr(counts), self._stream()), "kp_seq_scan")
 
+    def snv_counts(self, seq, seq_base, seq_len, rec_len, pos0, pos1, both, pos, ref_alt, alt_slot, counts, status,
+                   count_mask=None):
+        """One kp_snv_counts call on the stream, without waiting.  seq, seq_base, seq_len, rec_len, pos0, pos1, both and
+        count_mask as in seq_scan; pos: int64 device tensor of record positions in [pos0, pos1); ref_alt: uint8 device
+        tensor (REF code | ALT code << 2); alt_slot: 4 ints (-1: not counted); counts: int64 device tensor
+        [slots, nkmer]; status: uint8 device tensor with one entry per SNV."""
+        n = int(pos.shape[0])
+        if ref_alt.shape[0] != n or status.shape[0] != n:
+            raise ValueError("pos, ref_alt and status need one entry per SNV")
+        if counts.numel() < (max(alt_slot) + 1) * self.nkmer:
+            raise ValueError("counts needs nkmer entries for every slot")
+        slots = (ctypes.c_int * 4)(*[int(x) for x in alt_slot])
+        check(self.lib.kp_snv_counts(self.handle, seq.data_ptr(), int(seq_base), int(seq_len), int(rec_len), int(pos0),
+                                     int(pos1), int(bool(both)), pos.data_ptr(), ref_alt.data_ptr(), n, slots,
+                                     count_mask.data_ptr() if count_mask is not None else None, counts.data_ptr(),
+                                     status.data_ptr(), self._stream()), "kp_snv_counts")
+
     def region_sums(self, piece_sum, piece_n, task_sum, task_n, regions, out_sum, out_n):
         """kp_region_sums on the stream, without waiting.  regions: int64 device tensor [n, 4]."""
         ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
