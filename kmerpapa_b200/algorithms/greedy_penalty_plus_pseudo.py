@@ -12,8 +12,8 @@ import ctypes
 import numpy as np
 
 from .. import CV_tools, iupac
-from .._native import KP_ERR_CAPACITY, KpError
-from ..engine import _torch, get_plan
+from .._native import KpError
+from ..engine import _torch, get_plan, grow_capacity
 from ..score_utils import get_betas
 
 
@@ -28,7 +28,8 @@ def _kmer_table(genpat, contextD):
 def _greedy(plan, kM, kU, alpha, beta, penalty, test=None, cap=65536):
     """(pattern numbers in the reference's order, float64 losses, float64 held-out LLs or None, float64 score)."""
     torch = _torch()
-    while True:
+
+    def run(cap):
         ws = plan._buffer("greedy_ws", int(plan.lib.kp_greedy_ws_bytes(cap)), torch.uint8)
         pats = np.empty(cap, dtype=np.uint64)
         loss = np.empty(cap, dtype=np.float64)
@@ -38,13 +39,10 @@ def _greedy(plan, kM, kU, alpha, beta, penalty, test=None, cap=65536):
                                 test[1].data_ptr() if test else None, float(alpha), float(beta), float(penalty), ws.data_ptr(),
                                 cap, pats.ctypes.data, loss.ctypes.data, tst.ctypes.data, ctypes.byref(n), ctypes.byref(total),
                                 plan._stream())
-        if rc == 0:
-            k = n.value
-            return pats[:k].copy(), loss[:k].copy(), (tst[:k].copy() if test else None), total.value
-        if rc == KP_ERR_CAPACITY and cap < (1 << 24):
-            cap *= 8
-            continue
-        raise KpError("kp_greedy: " + plan.lib.kp_last_error().decode())
+        return rc, (pats, loss, tst, n.value, total.value)
+
+    pats, loss, tst, k, total = grow_capacity(plan.lib, "kp_greedy", cap, 1 << 24, run)
+    return pats[:k].copy(), loss[:k].copy(), (tst[:k].copy() if test else None), total
 
 
 def greedy_partition(genpat, contextD, alpha, beta, penalty, args):

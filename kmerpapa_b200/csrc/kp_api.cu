@@ -90,7 +90,7 @@ struct kp_plan {
 #endif
 
 template <bool WIDE>
-static const void *dp_kernel_for_radix(int r0, int rp)
+static const void *dp_kernel_r0(int r0, int rp)
 {
     switch (r0) {
     case 1: return (const void *)kp_dp_rows_kernel<1, WIDE, 0, 0>;
@@ -102,19 +102,32 @@ static const void *dp_kernel_for_radix(int r0, int rp)
     }
 }
 
-template <int R0, int RP, int SHARD>
-static void launch_dp_r0(bool wide, int grid, int threads, size_t smem, cudaStream_t st, const KpDpParams &prm)
-{
-    if (wide) kp_dp_rows_kernel<R0, true, RP, SHARD><<<grid, threads, smem, st>>>(prm);
-    else kp_dp_rows_kernel<R0, false, RP, SHARD><<<grid, threads, smem, st>>>(prm);
-}
-
-// the sharded DP exists for the register radix 15 only (a pattern without an N position is far too small to shard)
 template <bool WIDE, int SHARD>
-static const void *dp_kernel_sharded(int rp)
+static const void *dp_kernel_rp(int rp)
 {
     return rp == KP_RP_NN ? (const void *)kp_dp_rows_kernel<15, WIDE, KP_RP_NN, SHARD>
                           : (const void *)kp_dp_rows_kernel<15, WIDE, 0, SHARD>;
+}
+
+template <int RP, int SHARD>
+static const void *dp_kernel_w(bool wide)
+{
+    return wide ? (const void *)kp_dp_rows_kernel<15, true, RP, SHARD> : (const void *)kp_dp_rows_kernel<15, false, RP, SHARD>;
+}
+
+// The kp_dp_rows_kernel that runs (register radix, row pitch, shard mode) at a count width.  The shard modes 1..4
+// (sharded, sharded and replicated, one launch, cooperative tail) exist for the register radix 15 only: a pattern
+// without an N position is far too small for them.  The order of the cases is the order of the kernels in the
+// library; keep it, so that the SASS dumps of two builds can be compared byte for byte.
+static const void *dp_kernel(int r0, int rp, int shard, bool wide)
+{
+    switch (shard) {
+    case 0: return wide ? dp_kernel_r0<true>(r0, rp) : dp_kernel_r0<false>(r0, rp);
+    case 3: return wide ? dp_kernel_rp<true, 3>(rp) : dp_kernel_rp<false, 3>(rp);
+    case 4: return rp == KP_RP_NN ? dp_kernel_w<KP_RP_NN, 4>(wide) : dp_kernel_w<0, 4>(wide);
+    case 1: return wide ? dp_kernel_rp<true, 1>(rp) : dp_kernel_rp<false, 1>(rp);
+    default: return wide ? dp_kernel_rp<true, 2>(rp) : dp_kernel_rp<false, 2>(rp);
+    }
 }
 
 // a view of one unsharded table
@@ -147,15 +160,18 @@ static KpView single_view(const kp_plan *p, const float *best, const uint16_t *f
     return v;
 }
 
+// element of pattern `patnum` in an unsharded score table
+static uint64_t table_elem(const KpHostPlan &h, uint64_t patnum)
+{
+    uint64_t tile; uint32_t srow, d0;
+    kp_locate(h, patnum, &tile, &srow, &d0);
+    return tile * h.t.tile_stride + ((uint64_t)(d0 >> 2) * h.t.rp + srow) * 4 + (d0 & 3);
+}
+
 extern "C" {
 
 const char *kp_last_error(void) { return g_err.c_str(); }
 int kp_version(void) { return 100; }
-
-static const void *dp_kernel_ptr(int r0, int rp, bool wide)
-{
-    return wide ? dp_kernel_for_radix<true>(r0, rp) : dp_kernel_for_radix<false>(r0, rp);
-}
 
 static int plan_create(const char *gen_pat, int device, bool lattice, kp_plan **out);
 
@@ -231,11 +247,11 @@ static int plan_create(const char *gen_pat, int device, bool lattice, kp_plan **
         if (nw > KP_MAX_WARPS) nw = KP_MAX_WARPS;
         p->nwarps[wide] = nw;
         // the attribute is per function, not per plan: always raise it to the device maximum
-        KP_CUDA(cudaFuncSetAttribute(dp_kernel_ptr(t.r0, t.rp, wide), cudaFuncAttributeMaxDynamicSharedMemorySize,
+        KP_CUDA(cudaFuncSetAttribute(dp_kernel(t.r0, t.rp, 0, wide), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)prop.sharedMemPerBlockOptin));
         if (t.r0 == 15)
-            KP_CUDA(cudaFuncSetAttribute(wide ? dp_kernel_sharded<true, 3>(t.rp) : dp_kernel_sharded<false, 3>(t.rp),
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+            KP_CUDA(cudaFuncSetAttribute(dp_kernel(t.r0, t.rp, 3, wide), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)prop.sharedMemPerBlockOptin));
     }
     *out = p;
     return 0;
@@ -297,16 +313,15 @@ const char *kp_dp_kernel_name(const kp_plan *p, int wide)
     return p && p->use_fiber && p->fiber_smem[wide != 0] ? "kp_dp_fiber_kernel" : "kp_dp_rows_kernel";
 }
 
-int kp_pattern_offset(const kp_plan *p, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit)
+int kp_pattern_offset(const kp_plan *p, uint64_t patnum, uint64_t *table_out, uint64_t *kept_elem, uint32_t *kept_bit)
 {
     if (p && !p->host.lattice) return fail("kp_pattern_offset: this plan was created without the tile lattice (kp_plan_create_lite)");
     if (!p) return fail("kp_pattern_offset: null plan");
     if (patnum >= p->host.npat) return fail("kp_pattern_offset: pattern number out of range");
     uint64_t tile; uint32_t srow, d0;
     kp_locate(p->host, patnum, &tile, &srow, &d0);
-    const KpTables &t = p->host.t;
-    if (table_elem) *table_elem = tile * t.tile_stride + ((uint64_t)(d0 >> 2) * t.rp + srow) * 4 + (d0 & 3);
-    if (kept_elem) *kept_elem = tile * (uint64_t)t.rp + srow;
+    if (table_out) *table_out = table_elem(p->host, patnum);
+    if (kept_elem) *kept_elem = tile * (uint64_t)p->host.t.rp + srow;
     if (kept_bit) *kept_bit = d0;
     return 0;
 }
@@ -388,6 +403,52 @@ int kp_expand_counts(kp_plan *p, const int64_t *d_kmerM, const int64_t *d_kmerU,
     return 0;
 }
 
+// launch shape of a DP wave of `ntile` tiles: nwarps tiles in flight per CTA, or fewer to spread a small wave over all SMs
+struct DpGeom {
+    int grid, threads;
+    size_t smem;
+};
+
+static DpGeom wave_geom(const kp_plan *p, bool wide, uint64_t ntile)
+{
+    const KpTables &t = p->host.t;
+    int warps = p->nwarps[wide];
+    if (ntile < (uint64_t)p->sm_count * warps) {
+        warps = (int)((ntile + p->sm_count - 1) / p->sm_count);
+        if (warps < 1) warps = 1;
+    }
+    const uint64_t grid = std::min<uint64_t>((ntile + warps - 1) / warps, (uint64_t)p->sm_count);
+    return {(int)grid, warps * 32, 2048 + t.rt_bytes + (size_t)warps * t.warp_smem_bytes[wide]};
+}
+
+// one kp_dp_rows_kernel launch; like a <<<>>> launch, an error surfaces at the caller's cudaGetLastError
+static void launch_rows(kp_plan *p, int shard, bool wide, const DpGeom &g, const KpDpParams &prm, cudaStream_t st)
+{
+    void *args[] = {(void *)&prm};
+    cudaLaunchKernel(dp_kernel(p->host.t.r0, p->host.t.rp, shard, wide), dim3(g.grid), dim3(g.threads), args, g.smem, st);
+    p->launches++;
+}
+
+// the KpDpParams fields of every DP launch: tables, the counts d_exp - d_sub (d_sub*: null for none), score parameters
+// and output tables
+static KpDpParams dp_params(const kp_plan *p, const int64_t *d_expM, const int64_t *d_expU, const int64_t *d_subM,
+                            const int64_t *d_subU, double alpha, double beta, double penalty, float *d_best, uint16_t *d_kept)
+{
+    KpDpParams prm;
+    memset(&prm, 0, sizeof prm);
+    prm.tab = p->d_tab;
+    prm.rowtab = p->d_rowtab;
+    prm.e0 = (const long long *)d_expM;
+    prm.e1 = (const long long *)d_expU;
+    prm.s0 = (const long long *)d_subM;
+    prm.s1 = (const long long *)d_subU;
+    prm.alpha = alpha; prm.beta = beta; prm.penalty = penalty;
+    prm.best = d_best;
+    prm.flags = d_kept;
+    prm.pf_dist = p->pf_dist;
+    return prm;
+}
+
 static int launch_dp(kp_plan *p, bool wide, KpDpParams prm, cudaStream_t st)
 {
     if (!p->host.lattice) return fail("this plan was created without the tile lattice (kp_plan_create_lite): no DP");
@@ -436,10 +497,7 @@ static int launch_dp(kp_plan *p, bool wide, KpDpParams prm, cudaStream_t st)
         prm.wave_done = p->d_counters + 64;
         prm.err = p->d_err;
         for (size_t l = 0; l < 64; l++) prm.wave_size[l] = l < nhl ? (uint32_t)(p->host.hl_off[l + 1] - p->host.hl_off[l]) : 0;
-        const size_t sm = 2048 + t.rt_bytes + (size_t)nw * t.warp_smem_bytes[wide];
-        if (t.rp == KP_RP_NN) launch_dp_r0<15, KP_RP_NN, 3>(wide, p->sm_count, nw * 32, sm, st, prm);
-        else launch_dp_r0<15, 0, 3>(wide, p->sm_count, nw * 32, sm, st, prm);
-        p->launches++;
+        launch_rows(p, 3, wide, wave_geom(p, wide, t.ntiles), prm, st);   // one CTA of nw warps per SM
         KP_CUDA(cudaGetLastError());
         return 0;
     }
@@ -455,42 +513,13 @@ static int launch_dp(kp_plan *p, bool wide, KpDpParams prm, cudaStream_t st)
         if (p->coop_tail && t.r0 == 15 && ntile <= (uint64_t)p->sm_count && nchunk <= KP_MAX_WARPS) {
             // at most one tile per SM (the last waves of a big lattice, every wave of a small one): a CTA per tile, every
             // warp streams one 32-row chunk of it, warp 0 runs the rounds - the wave costs a fraction of a tile latency
-            const size_t smc = 2048 + t.rt_bytes + (size_t)t.warp_smem_bytes[wide];
-            if (t.rp == KP_RP_NN) launch_dp_r0<15, KP_RP_NN, 4>(wide, (int)ntile, nchunk * 32, smc, st, prm);
-            else launch_dp_r0<15, 0, 4>(wide, (int)ntile, nchunk * 32, smc, st, prm);
-            p->launches++;
+            launch_rows(p, 4, wide, {(int)ntile, nchunk * 32, 2048 + t.rt_bytes + (size_t)t.warp_smem_bytes[wide]}, prm, st);
             continue;
         }
-        int warps = nw;
-        if (ntile < (uint64_t)p->sm_count * nw) {  // small wave: spread the tiles over all SMs
-            warps = (int)((ntile + p->sm_count - 1) / p->sm_count);
-            if (warps < 1) warps = 1;
-        }
-        uint64_t grid = (ntile + warps - 1) / warps;
-        if (grid > (uint64_t)p->sm_count) grid = p->sm_count;
-        size_t sm = 2048 + t.rt_bytes + (size_t)warps * t.warp_smem_bytes[wide];
-        switch (t.r0) {
-        case 1: launch_dp_r0<1, 0, 0>(wide, (int)grid, warps * 32, sm, st, prm); break;
-        case 3: launch_dp_r0<3, 0, 0>(wide, (int)grid, warps * 32, sm, st, prm); break;
-        case 7: launch_dp_r0<7, 0, 0>(wide, (int)grid, warps * 32, sm, st, prm); break;
-        default:
-            if (t.rp == KP_RP_NN) launch_dp_r0<15, KP_RP_NN, 0>(wide, (int)grid, warps * 32, sm, st, prm);
-            else launch_dp_r0<15, 0, 0>(wide, (int)grid, warps * 32, sm, st, prm);
-            break;
-        }
-        p->launches++;
+        launch_rows(p, 0, wide, wave_geom(p, wide, ntile), prm, st);
     }
     KP_CUDA(cudaGetLastError());
     return 0;
-}
-
-static int dp_counts(kp_plan *p, const int64_t *d_expM, const int64_t *d_expU, const int64_t *d_subM, const int64_t *d_subU,
-                     uint64_t max_count, double alpha, double beta, double penalty, float *d_best, uint16_t *d_kept, void *stream);
-
-int kp_dp_single(kp_plan *p, const int64_t *d_expM, const int64_t *d_expU, uint64_t max_count, double alpha, double beta,
-                 double penalty, float *d_best, uint16_t *d_kept, void *stream)
-{
-    return dp_counts(p, d_expM, d_expU, nullptr, nullptr, max_count, alpha, beta, penalty, d_best, d_kept, stream);
 }
 
 // the DP on the counts d_expM - d_subM, d_expU - d_subU (d_sub*: null for none)
@@ -499,35 +528,48 @@ static int dp_counts(kp_plan *p, const int64_t *d_expM, const int64_t *d_expU, c
 {
     if (!p) return fail("kp_dp_single: null plan");
     KP_CUDA(cudaSetDevice(p->device));
-    bool wide = max_count > 0xFFFFFFFFull;
-    KpDpParams prm;
-    memset(&prm, 0, sizeof prm);
-    prm.tab = p->d_tab;
-    prm.rowtab = p->d_rowtab;
-    prm.e0 = (const long long *)d_expM;
-    prm.e1 = (const long long *)d_expU;
-    prm.s0 = (const long long *)d_subM;
-    prm.s1 = (const long long *)d_subU;
-    prm.alpha = alpha; prm.beta = beta; prm.penalty = penalty;
-    prm.best = d_best;
-    prm.flags = d_kept;
-    prm.pf_dist = p->pf_dist;
+    KpDpParams prm = dp_params(p, d_expM, d_expU, d_subM, d_subU, alpha, beta, penalty, d_best, d_kept);
     prm.evict_top = p->evict_top < p->host.t.nhigh ? p->evict_top : 0;
     prm.pf_top = p->pf_top;
     prm.pf_bulk = p->pf_bulk;
-    return launch_dp(p, wide, prm, (cudaStream_t)stream);
+    return launch_dp(p, max_count > 0xFFFFFFFFull, prm, (cudaStream_t)stream);
 }
 
-// breadth-first backtrack from `root`; leaves end up sorted by path key in the workspace
-static int backtrack_device(kp_plan *p, const KpView &vw, void *d_ws, uint64_t cap, uint64_t root,
-                            cudaStream_t st, unsigned long long **sorted_out, unsigned long long **keys_out, float **vals_out,
-                            unsigned long long **ctr_out)
+int kp_dp_single(kp_plan *p, const int64_t *d_expM, const int64_t *d_expU, uint64_t max_count, double alpha, double beta,
+                 double penalty, float *d_best, uint16_t *d_kept, void *stream)
 {
-    KpBtNode *fa = (KpBtNode *)d_ws, *fb = fa + cap, *leaves = fb + cap;
-    unsigned long long *sorted = (unsigned long long *)(leaves + cap);
-    unsigned long long *keys = sorted + cap;
-    unsigned long long *ctr = keys + cap;   // [0] leaves, [1] overflow, [2 + d] nodes at depth d
-    float *vals = (float *)(ctr + 80);
+    return dp_counts(p, d_expM, d_expU, nullptr, nullptr, max_count, alpha, beta, penalty, d_best, d_kept, stream);
+}
+
+// the backtrack workspace (kp_backtrack_ws_bytes): two frontiers and the leaves, then the leaves' pattern numbers and
+// path keys sorted by key, the counters ([0] leaves, [1] overflow, [2 + d] nodes at depth d) and the leaves' held-out losses
+struct BtWs {
+    KpBtNode *fa, *fb, *leaves;
+    unsigned long long *sorted, *keys, *ctr;
+    float *vals;
+};
+
+static BtWs bt_layout(void *d_ws, uint64_t cap)
+{
+    BtWs L;
+    L.fa = (KpBtNode *)d_ws;
+    L.fb = L.fa + cap;
+    L.leaves = L.fb + cap;
+    L.sorted = (unsigned long long *)(L.leaves + cap);
+    L.keys = L.sorted + cap;
+    L.ctr = L.keys + cap;
+    L.vals = (float *)(L.ctr + 80);
+    return L;
+}
+
+// breadth-first backtrack from `root` on a view; leaves end up sorted by path key in the workspace
+static int backtrack_device(kp_plan *p, const KpView &vw, const BtWs &L, uint64_t cap, uint64_t root, cudaStream_t st,
+                            const char *what)
+{
+    if (p->host.t.total_level > 64) return fail(std::string(what) + ": more than 64 levels");
+    KP_CUDA(cudaSetDevice(p->device));
+    KpBtNode *fa = L.fa, *fb = L.fb, *leaves = L.leaves;
+    unsigned long long *ctr = L.ctr;
     kp_backtrack_init_kernel<<<1, 128, 0, st>>>(fa, root, ctr);
     const int levels = (int)p->host.t.total_level + 1;
     int grid = (int)((cap + 7) / 8);
@@ -554,10 +596,74 @@ static int backtrack_device(kp_plan *p, const KpView &vw, void *d_ws, uint64_t c
                                                         (d & 1) ? fa : fb, leaves, cap, ctr);
         p->launches++;
     }
-    kp_backtrack_sort_kernel<<<p->sm_count, 256, 0, st>>>(leaves, ctr, cap, sorted, keys);
+    kp_backtrack_sort_kernel<<<p->sm_count, 256, 0, st>>>(leaves, ctr, cap, L.sorted, L.keys);
     p->launches += 2;
     KP_CUDA(cudaGetLastError());
-    *sorted_out = sorted; *keys_out = keys; *vals_out = vals; *ctr_out = ctr;
+    return 0;
+}
+
+// waits for the stream, then the number of leaves of the backtrack; fails if the DP gave up waiting for a child tile
+static int bt_leaves(kp_plan *p, const BtWs &L, uint64_t cap, cudaStream_t st, const char *what, uint64_t *n)
+{
+    unsigned long long hc[2] = {0, 0};
+    int herr = 0;
+    KP_CUDA(cudaMemcpyAsync(hc, L.ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(&herr, p->d_err, sizeof herr, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    if (herr == 2) return fail(std::string(what) + ": the DP gave up waiting for a child tile (internal error)");
+    *n = hc[0];
+    if (hc[1] || hc[0] > cap) return fail_capacity(std::string(what) + ": partition larger than the workspace capacity");
+    return 0;
+}
+
+// the optimal partition of `root` on a view: its pattern numbers, in the reference's order, to the host
+static int backtrack_host(kp_plan *p, const KpView &vw, void *d_ws, uint64_t cap, uint64_t root, uint64_t *h_patnums,
+                          uint64_t *n_out, cudaStream_t st, const char *what)
+{
+    const BtWs L = bt_layout(d_ws, cap);
+    if (backtrack_device(p, vw, L, cap, root, st, what)) return KP_ERR;
+    if (int rc = bt_leaves(p, L, cap, st, what, n_out)) return rc;
+    KP_CUDA(cudaMemcpyAsync(h_patnums, L.sorted, *n_out * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// queues the backtrack of `root` on a view and the held-out loss of every leaf of it
+static int heldout_enqueue(kp_plan *p, const KpView &vw, const int64_t *d_expMtot, const int64_t *d_expUtot,
+                           const int64_t *d_expMtest, const int64_t *d_expUtest, double alpha, double beta_fold, double penalty,
+                           uint64_t root, const BtWs &L, uint64_t cap, cudaStream_t st, const char *what)
+{
+    if (backtrack_device(p, vw, L, cap, root, st, what)) return KP_ERR;
+    kp_cv_leaf_kernel<<<p->sm_count, 128, 0, st>>>(p->d_tab, p->d_rowtab, (const long long *)d_expMtot, (const long long *)d_expUtot,
+                                                   (const long long *)d_expMtest, (const long long *)d_expUtest, alpha, beta_fold,
+                                                   penalty, L.sorted, L.ctr, cap, L.vals);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// heldout_enqueue, then *h_test = the float32 sum of the leaves' held-out losses in the order of the partition tree; with
+// d_train_top, also *h_train_top = *d_train_top (the root's train loss), read in the same round trip
+static int heldout_sync(kp_plan *p, const KpView &vw, const int64_t *d_expMtot, const int64_t *d_expUtot,
+                        const int64_t *d_expMtest, const int64_t *d_expUtest, double alpha, double beta_fold, double penalty,
+                        uint64_t root, void *d_ws, uint64_t cap, const float *d_train_top, float *h_train_top, float *h_test,
+                        cudaStream_t st, const char *what)
+{
+    const BtWs L = bt_layout(d_ws, cap);
+    if (heldout_enqueue(p, vw, d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold, penalty, root, L, cap, st, what))
+        return KP_ERR;
+    float htrain = 0.f;
+    if (d_train_top) KP_CUDA(cudaMemcpyAsync(&htrain, d_train_top, sizeof htrain, cudaMemcpyDeviceToHost, st));
+    uint64_t n = 0;
+    if (int rc = bt_leaves(p, L, cap, st, what, &n)) return rc;
+    if (n == 0) return fail(std::string(what) + ": the backtrack produced no leaf (internal error)");
+    std::vector<unsigned long long> hk(n);
+    std::vector<float> hv(n);
+    KP_CUDA(cudaMemcpyAsync(hk.data(), L.keys, n * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(hv.data(), L.vals, n * 4, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    if (d_train_top) *h_train_top = htrain;
+    *h_test = tree_sum(hk.data(), hv.data(), 0, n, 0);
     return 0;
 }
 
@@ -565,25 +671,10 @@ int kp_backtrack(kp_plan *p, const float *d_best, const uint16_t *d_kept, void *
                  uint64_t *h_patnums, uint64_t *n_out, void *stream)
 {
     if (!p || !d_ws || !h_patnums || !n_out) return fail("kp_backtrack: null argument");
-    if (p->host.t.total_level > 64) return fail("kp_backtrack: more than 64 levels");
     if (root == UINT64_MAX) root = p->host.npat - 1;
     if (root >= p->host.npat) return fail("kp_backtrack: root out of range");
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    unsigned long long *sorted, *keys, *ctr;
-    float *vals;
-    if (backtrack_device(p, single_view(p, d_best, d_kept), d_ws, cap, root, st, &sorted, &keys, &vals, &ctr)) return 1;
-    unsigned long long hc[2] = {0, 0};
-    int herr = 0;
-    KP_CUDA(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(&herr, p->d_err, sizeof herr, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    if (herr == 2) return fail("kp_backtrack: the DP gave up waiting for a child tile (internal error)");
-    *n_out = hc[0];
-    if (hc[1] || hc[0] > cap) return fail_capacity("kp_backtrack: partition larger than the workspace capacity");
-    KP_CUDA(cudaMemcpyAsync(h_patnums, sorted, hc[0] * 8, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return backtrack_host(p, single_view(p, d_best, d_kept), d_ws, cap, root, h_patnums, n_out, (cudaStream_t)stream,
+                          "kp_backtrack");
 }
 
 int kp_cv_heldout(kp_plan *p, const float *d_train, const uint16_t *d_kept, const int64_t *d_expMtot, const int64_t *d_expUtot,
@@ -593,28 +684,8 @@ int kp_cv_heldout(kp_plan *p, const float *d_train, const uint16_t *d_kept, cons
     if (!p || !d_ws || !h_test) return fail("kp_cv_heldout: null argument");
     if (root == UINT64_MAX) root = p->host.npat - 1;
     if (root >= p->host.npat) return fail("kp_cv_heldout: root out of range");
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    unsigned long long *sorted, *keys, *ctr;
-    float *vals;
-    if (backtrack_device(p, single_view(p, d_train, d_kept), d_ws, cap, root, st, &sorted, &keys, &vals, &ctr)) return 1;
-    kp_cv_leaf_kernel<<<p->sm_count, 128, 0, st>>>(p->d_tab, p->d_rowtab, (const long long *)d_expMtot, (const long long *)d_expUtot,
-                                                   (const long long *)d_expMtest, (const long long *)d_expUtest, alpha, beta_fold,
-                                                   penalty, sorted, ctr, cap, vals);
-    p->launches++;
-    KP_CUDA(cudaGetLastError());
-    unsigned long long hc[2] = {0, 0};
-    KP_CUDA(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    if (hc[1] || hc[0] > cap) return fail_capacity("kp_cv_heldout: partition larger than the workspace capacity");
-    if (hc[0] == 0) return fail("kp_cv_heldout: the backtrack produced no leaf (internal error)");
-    std::vector<unsigned long long> hk(hc[0]);
-    std::vector<float> hv(hc[0]);
-    KP_CUDA(cudaMemcpyAsync(hk.data(), keys, hc[0] * 8, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(hv.data(), vals, hc[0] * 4, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    *h_test = tree_sum(hk.data(), hv.data(), 0, hc[0], 0);
-    return 0;
+    return heldout_sync(p, single_view(p, d_train, d_kept), d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold,
+                        penalty, root, d_ws, cap, nullptr, nullptr, h_test, (cudaStream_t)stream, "kp_cv_heldout");
 }
 
 int kp_dp_cv_job(kp_plan *p, const int64_t *d_expMtot, const int64_t *d_expUtot, const int64_t *d_expMtest,
@@ -622,24 +693,16 @@ int kp_dp_cv_job(kp_plan *p, const int64_t *d_expMtot, const int64_t *d_expUtot,
                  float *d_train, uint16_t *d_kept, void *d_ws, uint64_t cap, float *h_top, void *stream)
 {
     if (!p || !d_expMtest || !d_expUtest) return fail("kp_dp_cv_job: null argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    const KpTables &t = p->host.t;
     // train counts = total - held-out: the subtraction commutes with the sums of the expansion, so it is done by the DP
     // kernel (and the leaf kernel) when they read the tile's base counts; no train table is materialised
     if (dp_counts(p, d_expMtot, d_expUtot, d_expMtest, d_expUtest, max_count, alpha, beta_fold, penalty, d_train, d_kept, stream))
-        return 1;
-    if (h_top) {
-        if (int rc = kp_cv_heldout(p, d_train, d_kept, d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold, penalty,
-                                   UINT64_MAX, d_ws, cap, h_top + 1, stream))
-            return rc;
-        uint64_t tile; uint32_t srow, d0;
-        kp_locate(p->host, p->host.npat - 1, &tile, &srow, &d0);
-        size_t top = (size_t)tile * t.tile_stride + ((size_t)(d0 >> 2) * t.rp + srow) * 4 + (d0 & 3);
-        KP_CUDA(cudaMemcpyAsync(h_top, d_train + top, sizeof(float), cudaMemcpyDeviceToHost, st));
-        KP_CUDA(cudaStreamSynchronize(st));
-    }
-    return 0;
+        return KP_ERR;
+    if (!h_top) return 0;
+    if (!d_ws) return fail("kp_dp_cv_job: null argument");
+    const uint64_t top = p->host.npat - 1;
+    return heldout_sync(p, single_view(p, d_train, d_kept), d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold,
+                        penalty, top, d_ws, cap, d_train + table_elem(p->host, top), h_top, h_top + 1, (cudaStream_t)stream,
+                        "kp_dp_cv_job");
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -647,7 +710,8 @@ int kp_dp_cv_job(kp_plan *p, const int64_t *d_expMtot, const int64_t *d_expUtot,
 // their results into a (pinned) host staging area and returns at once; kp_cv_job_finish, called after the stream has
 // passed that point (an event the caller records), does the host part (the float32 tree sum).  With two train tables
 // in rotation the next job's DP is queued before the previous job's results are read, so the GPU never waits for the host.
-// Staging layout: u64 leaves, u64 overflow, f32 train loss of the general pattern, pad to 32 bytes; u64 keys[cap]; f32 vals[cap].
+// Staging layout: u64 leaves, u64 overflow, f32 train loss of the general pattern, i32 DP error flag (2: the DP gave up
+// waiting for a child tile), pad to 32 bytes; u64 keys[cap]; f32 vals[cap].
 // ---------------------------------------------------------------------------------------------------
 uint64_t kp_cv_stage_bytes(uint64_t cap) { return 32 + cap * 12; }
 
@@ -657,26 +721,19 @@ int kp_cv_job_enqueue(kp_plan *p, const int64_t *d_expMtot, const int64_t *d_exp
 {
     if (!p || !d_expMtest || !d_expUtest || !d_ws || !h_stage) return fail("kp_cv_job_enqueue: null argument");
     cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    const KpTables &t = p->host.t;
     if (dp_counts(p, d_expMtot, d_expUtot, d_expMtest, d_expUtest, max_count, alpha, beta_fold, penalty, d_train, d_kept, stream))
-        return 1;
-    unsigned long long *sorted, *keys, *ctr;
-    float *vals;
-    if (backtrack_device(p, single_view(p, d_train, d_kept), d_ws, cap, p->host.npat - 1, st, &sorted, &keys, &vals, &ctr)) return 1;
-    kp_cv_leaf_kernel<<<p->sm_count, 128, 0, st>>>(p->d_tab, p->d_rowtab, (const long long *)d_expMtot, (const long long *)d_expUtot,
-                                                   (const long long *)d_expMtest, (const long long *)d_expUtest, alpha, beta_fold,
-                                                   penalty, sorted, ctr, cap, vals);
-    p->launches++;
-    KP_CUDA(cudaGetLastError());
+        return KP_ERR;
+    const uint64_t top = p->host.npat - 1;
+    const BtWs L = bt_layout(d_ws, cap);
+    if (heldout_enqueue(p, single_view(p, d_train, d_kept), d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold,
+                        penalty, top, L, cap, st, "kp_cv_job_enqueue"))
+        return KP_ERR;
     unsigned char *h = (unsigned char *)h_stage;
-    uint64_t tile; uint32_t srow, d0;
-    kp_locate(p->host, p->host.npat - 1, &tile, &srow, &d0);
-    const size_t top = (size_t)tile * t.tile_stride + ((size_t)(d0 >> 2) * t.rp + srow) * 4 + (d0 & 3);
-    KP_CUDA(cudaMemcpyAsync(h, ctr, 16, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(h + 16, d_train + top, sizeof(float), cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(h + 32, keys, cap * 8, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(h + 32 + cap * 8, vals, cap * 4, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h, L.ctr, 16, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h + 16, d_train + table_elem(p->host, top), sizeof(float), cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h + 20, p->d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h + 32, L.keys, cap * 8, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaMemcpyAsync(h + 32 + cap * 8, L.vals, cap * 4, cudaMemcpyDeviceToHost, st));
     return 0;
 }
 
@@ -685,7 +742,10 @@ int kp_cv_job_finish(const void *h_stage, uint64_t cap, float *h_top)
     if (!h_stage || !h_top) return fail("kp_cv_job_finish: null argument");
     const unsigned char *h = (const unsigned char *)h_stage;
     unsigned long long hc[2];
+    int herr;
     memcpy(hc, h, 16);
+    memcpy(&herr, h + 20, sizeof herr);
+    if (herr == 2) return fail("kp_cv_job_finish: the DP gave up waiting for a child tile (internal error)");
     if (hc[1] || hc[0] > cap) return fail_capacity("kp_cv_job_finish: partition larger than the workspace capacity");
     if (hc[0] == 0) return fail("kp_cv_job_finish: the backtrack produced no leaf (internal error)");
     memcpy(h_top, h + 16, sizeof(float));
@@ -693,55 +753,49 @@ int kp_cv_job_finish(const void *h_stage, uint64_t cap, float *h_top)
     return 0;
 }
 
+// scores / kept-whole flags / split codes, read through a view, of the patterns h_patnums[0..n) or, without h_patnums, of
+// the patterns first..first+n-1 (split codes need h_patnums); an output that is not asked for is null
+static int gather_view(kp_plan *p, const KpView &vw, const uint64_t *h_patnums, uint64_t first, uint64_t n, float *h_best,
+                       uint8_t *h_kept, uint8_t *h_codes, cudaStream_t st)
+{
+    if (n == 0) return 0;
+    KP_CUDA(cudaSetDevice(p->device));
+    const uint64_t pat_bytes = h_patnums ? n * 8 : 0, best_bytes = h_best ? n * 4 : 0, kept_bytes = h_kept ? n : 0;
+    if (scratch_reserve(p, pat_bytes + best_bytes + kept_bytes + (h_codes ? n : 0), st)) return KP_ERR;
+    unsigned long long *d_pat = h_patnums ? (unsigned long long *)p->d_scratch : nullptr;
+    float *d_val = (float *)(p->d_scratch + pat_bytes);
+    uint8_t *d_k = p->d_scratch + pat_bytes + best_bytes, *d_c = d_k + kept_bytes;
+    if (h_patnums) KP_CUDA(cudaMemcpyAsync(d_pat, h_patnums, n * 8, cudaMemcpyHostToDevice, st));
+    const int grid = grid_for(n, 256, p->sm_count);
+    if (h_best) { kp_gather_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, first, n, d_val); p->launches++; }
+    if (h_kept) { kp_gather_flags_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, first, n, d_k); p->launches++; }
+    if (h_codes) { kp_split_codes_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, n, d_c); p->launches++; }
+    KP_CUDA(cudaGetLastError());
+    if (h_best) KP_CUDA(cudaMemcpyAsync(h_best, d_val, n * 4, cudaMemcpyDeviceToHost, st));
+    if (h_kept) KP_CUDA(cudaMemcpyAsync(h_kept, d_k, n, cudaMemcpyDeviceToHost, st));
+    if (h_codes) KP_CUDA(cudaMemcpyAsync(h_codes, d_c, n, cudaMemcpyDeviceToHost, st));
+    KP_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
 int kp_split_codes(kp_plan *p, const float *d_best, const uint16_t *d_kept, const uint64_t *h_patnums, uint64_t n,
                    uint8_t *h_codes, void *stream)
 {
     if (!p) return fail("kp_split_codes: null plan");
-    if (n == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, n * 9, st)) return 1;
-    unsigned long long *d_pat = (unsigned long long *)p->d_scratch;
-    uint8_t *d_codes = (uint8_t *)(d_pat + n);
-    KP_CUDA(cudaMemcpyAsync(d_pat, h_patnums, n * 8, cudaMemcpyHostToDevice, st));
-    kp_split_codes_kernel<<<grid_for(n, 256, p->sm_count), 256, 0, st>>>(p->d_tab, p->d_rowtab, single_view(p, d_best, d_kept), d_pat, n, d_codes);
-    p->launches++;
-    KP_CUDA(cudaGetLastError());
-    KP_CUDA(cudaMemcpyAsync(h_codes, d_codes, n, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    if (n && !h_patnums) return fail("kp_split_codes: null argument");
+    return gather_view(p, single_view(p, d_best, d_kept), h_patnums, 0, n, nullptr, nullptr, h_codes, (cudaStream_t)stream);
 }
 
 int kp_gather_table(kp_plan *p, const float *d_table, uint64_t first, uint64_t n, float *h_out, void *stream)
 {
     if (!p) return fail("kp_gather_table: null plan");
-    if (n == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, n * 4, st)) return 1;
-    float *d_out = (float *)p->d_scratch;
-    kp_gather_kernel<<<grid_for(n, 256, p->sm_count), 256, 0, st>>>(p->d_tab, p->d_rowtab, single_view(p, d_table, nullptr), nullptr, first, n, d_out);
-    p->launches++;
-    KP_CUDA(cudaGetLastError());
-    KP_CUDA(cudaMemcpyAsync(h_out, d_out, n * 4, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return gather_view(p, single_view(p, d_table, nullptr), nullptr, first, n, h_out, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int kp_gather_kept(kp_plan *p, const uint16_t *d_kept, uint64_t first, uint64_t n, uint8_t *h_out, void *stream)
 {
     if (!p) return fail("kp_gather_kept: null plan");
-    if (n == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, n, st)) return 1;
-    uint8_t *d_out = (uint8_t *)p->d_scratch;
-    kp_gather_flags_kernel<<<grid_for(n, 256, p->sm_count), 256, 0, st>>>(p->d_tab, p->d_rowtab, single_view(p, nullptr, d_kept), nullptr, first, n, d_out);
-    p->launches++;
-    KP_CUDA(cudaGetLastError());
-    KP_CUDA(cudaMemcpyAsync(h_out, d_out, n, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return gather_view(p, single_view(p, nullptr, d_kept), nullptr, first, n, nullptr, h_out, nullptr, (cudaStream_t)stream);
 }
 
 // scores / kept-whole flags / split codes of arbitrary patterns of an unsharded table (any of the outputs may be null)
@@ -752,25 +806,7 @@ int kp_gather_patterns(kp_plan *p, const float *d_table, const uint16_t *d_kept,
     if (!p->host.lattice) return fail("kp_gather_patterns: this plan was created without the tile lattice (kp_plan_create_lite)");
     if ((h_best || h_codes) && !d_table) return fail("kp_gather_patterns: scores and split codes need the score table");
     if ((h_kept || h_codes) && !d_kept) return fail("kp_gather_patterns: kept flags and split codes need the kept-whole table");
-    if (n == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, n * 16, st)) return 1;
-    unsigned long long *d_pat = (unsigned long long *)p->d_scratch;
-    float *d_val = (float *)(d_pat + n);
-    uint8_t *d_k = (uint8_t *)(d_val + n), *d_c = d_k + n;
-    KP_CUDA(cudaMemcpyAsync(d_pat, h_patnums, n * 8, cudaMemcpyHostToDevice, st));
-    const int grid = grid_for(n, 256, p->sm_count);
-    const KpView vw = single_view(p, d_table, d_kept);
-    if (h_best) { kp_gather_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, 0, n, d_val); p->launches++; }
-    if (h_kept) { kp_gather_flags_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, 0, n, d_k); p->launches++; }
-    if (h_codes) { kp_split_codes_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, vw, d_pat, n, d_c); p->launches++; }
-    KP_CUDA(cudaGetLastError());
-    if (h_best) KP_CUDA(cudaMemcpyAsync(h_best, d_val, n * 4, cudaMemcpyDeviceToHost, st));
-    if (h_kept) KP_CUDA(cudaMemcpyAsync(h_kept, d_k, n, cudaMemcpyDeviceToHost, st));
-    if (h_codes) KP_CUDA(cudaMemcpyAsync(h_codes, d_c, n, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return gather_view(p, single_view(p, d_table, d_kept), h_patnums, 0, n, h_best, h_kept, h_codes, (cudaStream_t)stream);
 }
 
 int kp_pattern_counts(kp_plan *p, const int64_t *d_kmerM, const int64_t *d_kmerU, const uint64_t *h_patnums, uint64_t n,
@@ -942,6 +978,14 @@ int kp_kmer_rates(kp_plan *p, const uint32_t *d_owner, const double *h_rate, uin
     return 0;
 }
 
+// the bytes [seq_base, seq_base + seq_len) of a record hold every window of the positions [pos0, pos1) that lies in it
+static bool windows_covered(int k, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0, uint64_t pos1)
+{
+    const int c = k / 2;
+    const uint64_t need_lo = pos0 >= (uint64_t)c ? pos0 - c : 0, need_hi = std::min<uint64_t>(rec_len, pos1 + (k - 1 - c));
+    return pos1 <= pos0 || (seq_base <= need_lo && seq_base + seq_len >= need_hi && seq_base + seq_len <= rec_len);
+}
+
 int kp_seq_scan(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t seq_len, uint64_t rec_len, uint64_t pos0,
                 uint64_t pos1, int both, const double *d_kmer_rate, const uint32_t *d_tasks, uint64_t ntask, double *d_sum,
                 int64_t *d_n, float *d_track, const uint32_t *d_count_mask, int64_t *d_counts, void *stream)
@@ -952,9 +996,7 @@ int kp_seq_scan(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t se
     if ((uintptr_t)d_seq & 15) return fail("kp_seq_scan: the sequence buffer must be 16-byte aligned");
     if (both && k % 2 == 0) return fail("kp_seq_scan: both strands need an odd k");
     if (pos0 % KP_SEQ_PIECE || pos0 > pos1 || pos1 > rec_len) return fail("kp_seq_scan: bad position range");
-    // every window of [pos0, pos1) that lies in the record must lie in the given bytes
-    const uint64_t need_lo = pos0 >= (uint64_t)c ? pos0 - c : 0, need_hi = std::min<uint64_t>(rec_len, pos1 + (k - 1 - c));
-    if (pos1 > pos0 && (seq_base > need_lo || seq_base + seq_len < need_hi || seq_base + seq_len > rec_len))
+    if (!windows_covered(k, seq_base, seq_len, rec_len, pos0, pos1))
         return fail("kp_seq_scan: the sequence bytes do not cover the windows of the positions");
     if (d_tasks && (d_track || d_counts)) return fail("kp_seq_scan: tracks and counts come from the whole-piece pass");
     if (pos1 == pos0 || (d_tasks && ntask == 0)) return 0;
@@ -1000,8 +1042,7 @@ int kp_snv_counts(kp_plan *p, const uint8_t *d_seq, uint64_t seq_base, uint64_t 
     if (n == 0) return 0;
     if (!d_seq || !d_pos || !d_ref_alt || !d_counts || !d_status) return fail("kp_snv_counts: null argument");
     if (((uintptr_t)d_pos & 7) || ((uintptr_t)d_counts & 7)) return fail("kp_snv_counts: d_pos and d_counts must be 8-byte aligned");
-    const uint64_t need_lo = pos0 >= (uint64_t)c ? pos0 - c : 0, need_hi = std::min<uint64_t>(rec_len, pos1 + (k - 1 - c));
-    if (pos1 > pos0 && (seq_base > need_lo || seq_base + seq_len < need_hi || seq_base + seq_len > rec_len))
+    if (!windows_covered(k, seq_base, seq_len, rec_len, pos0, pos1))
         return fail("kp_snv_counts: the sequence bytes do not cover the windows of the positions");
     cudaStream_t st = (cudaStream_t)stream;
     KP_CUDA(cudaSetDevice(p->device));
@@ -1075,7 +1116,6 @@ struct kp_shard {
 static void optimise_cell_owners(const KpTables &t, int e1, int e2, int world, std::vector<uint8_t> &owner)
 {
     const int r1 = t.radix[e1], r2 = t.radix[e2], ncell = r1 * r2;
-    auto pc = [](unsigned m) { return (int)((m & 1) + ((m >> 1) & 1) + ((m >> 2) & 1) + ((m >> 3) & 1)); };
     std::vector<std::vector<int>> sup1(r1), sup2(r2);
     for (int d = 0; d < r1; d++)
         for (int q = 0; q < r1; q++)
@@ -1087,7 +1127,7 @@ static void optimise_cell_owners(const KpTables &t, int e1, int e2, int world, s
     int nlvl = 0;
     for (int d1 = 0; d1 < r1; d1++)
         for (int d2 = 0; d2 < r2; d2++) {
-            lvl[d2 + r2 * d1] = pc(t.digit_mask[e1][d1]) + pc(t.digit_mask[e2][d2]) - 2;
+            lvl[d2 + r2 * d1] = __builtin_popcount(t.digit_mask[e1][d1]) + __builtin_popcount(t.digit_mask[e2][d2]) - 2;
             nlvl = std::max(nlvl, lvl[d2 + r2 * d1] + 1);
         }
     std::vector<int> inb(world), outb(world), wl((size_t)nlvl * world);
@@ -1175,8 +1215,8 @@ static int shard_assignment(const kp_plan *p, int world, uint8_t *owner, uint8_t
     if (world < 1 || world > KP_MAX_SHARDS || world > radix) return fail("sharding: world size must be 1..min(8, radix of the top position)");
     std::vector<int> digits(radix);
     for (int d = 0; d < radix; d++) digits[d] = d;
-    auto lvl = [&](int d) { unsigned m = t.digit_mask[e][d]; return (int)((m & 1) + ((m >> 1) & 1) + ((m >> 2) & 1) + ((m >> 3) & 1)); };
-    std::stable_sort(digits.begin(), digits.end(), [&](int a, int b) { return lvl(a) > lvl(b); });
+    std::stable_sort(digits.begin(), digits.end(),
+                     [&](int a, int b) { return __builtin_popcount(t.digit_mask[e][a]) > __builtin_popcount(t.digit_mask[e][b]); });
     for (int r = 0; r < KP_MAX_SHARDS; r++) nslots_of_rank[r] = 0;
     memset(owner, 0, 16);
     memset(slot, 0, 16);
@@ -1236,8 +1276,9 @@ int kp_shard_create(kp_plan *p, int rank, int world, int replicate, kp_shard **o
                 const int radix = t.radix[pos];
                 std::vector<int> digits(radix);
                 for (int d = 0; d < radix; d++) digits[d] = d;
-                auto lvl = [&](int d) { unsigned m = t.digit_mask[pos][d]; return (int)((m & 1) + ((m >> 1) & 1) + ((m >> 2) & 1) + ((m >> 3) & 1)); };
-                std::stable_sort(digits.begin(), digits.end(), [&](int a, int b) { return lvl(a) > lvl(b); });
+                std::stable_sort(digits.begin(), digits.end(), [&](int a, int b) {
+                    return __builtin_popcount(t.digit_mask[pos][a]) > __builtin_popcount(t.digit_mask[pos][b]);
+                });
                 idx.assign(radix, 0);
                 for (int i = 0; i < radix; i++) idx[digits[i]] = i;
             };
@@ -1306,10 +1347,10 @@ int kp_shard_create(kp_plan *p, int rank, int world, int replicate, kp_shard **o
     KP_CUDA(cudaMemcpy(s->d_tiles, mine.data(), sizeof(uint32_t) * mine.size(), cudaMemcpyHostToDevice));
     s->view.best[rank] = s->d_best;
     s->view.flags[rank] = s->d_kept;
-    KP_CUDA(cudaFuncSetAttribute(dp_kernel_sharded<true, 1>(t.rp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_optin));
-    KP_CUDA(cudaFuncSetAttribute(dp_kernel_sharded<false, 1>(t.rp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_optin));
-    KP_CUDA(cudaFuncSetAttribute(dp_kernel_sharded<true, 2>(t.rp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_optin));
-    KP_CUDA(cudaFuncSetAttribute(dp_kernel_sharded<false, 2>(t.rp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_optin));
+    for (int shard = 1; shard <= 2; shard++)
+        for (int wide = 0; wide < 2; wide++)
+            KP_CUDA(cudaFuncSetAttribute(dp_kernel(t.r0, t.rp, shard, wide), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)p->smem_optin));
     *out = s;
     return 0;
 }
@@ -1385,7 +1426,6 @@ static int shard_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_
 {
     if (!s) return fail(std::string(what) + ": null shard");
     kp_plan *p = s->plan;
-    const KpTables &t = p->host.t;
     if (wave < 0 || wave >= (int)s->hl_off.size() - 1 || wave >= 64) return fail(std::string(what) + ": bad wave");
     for (int r = 0; r < s->world; r++)
         if (!s->view.best[r] || !s->view.flags[r]) return fail(std::string(what) + ": a peer's shard has not been set");
@@ -1395,43 +1435,15 @@ static int shard_wave(kp_shard *s, int wave, const int64_t *d_expM, const int64_
     const uint64_t lo = s->hl_off[wave], hi = s->hl_off[wave + 1];
     if (hi == lo) return 0;
     const bool wide = max_count > 0xFFFFFFFFull;
-    const int nw = p->nwarps[wide];
-    if (nw < 1) return fail("DP kernel does not fit in shared memory for this tile shape");
-    KpDpParams prm;
-    memset(&prm, 0, sizeof prm);
-    prm.tab = p->d_tab;
-    prm.rowtab = p->d_rowtab;
-    prm.e0 = (const long long *)d_expM;
-    prm.e1 = (const long long *)d_expU;
-    prm.s0 = (const long long *)d_subM;
-    prm.s1 = (const long long *)d_subU;
-    prm.alpha = alpha; prm.beta = beta; prm.penalty = penalty;
-    prm.best = s->d_best;
-    prm.flags = s->d_kept;
-    prm.pf_dist = p->pf_dist;
+    if (p->nwarps[wide] < 1) return fail("DP kernel does not fit in shared memory for this tile shape");
+    KpDpParams prm = dp_params(p, d_expM, d_expU, d_subM, d_subU, alpha, beta, penalty, s->d_best, s->d_kept);
     prm.view = s->view;
     prm.my_rank = s->rank;
     prm.tile_list = s->d_tiles + lo;
     prm.ntiles_wave = (uint32_t)(hi - lo);
     prm.counter = s->d_counters + wave;
     prm.leaf_wave = (wave == 0);
-    const uint64_t ntile = hi - lo;
-    int warps = nw;
-    if (ntile < (uint64_t)p->sm_count * nw) {
-        warps = (int)((ntile + p->sm_count - 1) / p->sm_count);
-        if (warps < 1) warps = 1;
-    }
-    uint64_t grid = (ntile + warps - 1) / warps;
-    if (grid > (uint64_t)p->sm_count) grid = p->sm_count;
-    const size_t sm = 2048 + t.rt_bytes + (size_t)warps * t.warp_smem_bytes[wide];
-    if (s->replicate) {
-        if (t.rp == KP_RP_NN) launch_dp_r0<15, KP_RP_NN, 2>(wide, (int)grid, warps * 32, sm, st, prm);
-        else launch_dp_r0<15, 0, 2>(wide, (int)grid, warps * 32, sm, st, prm);
-    } else {
-        if (t.rp == KP_RP_NN) launch_dp_r0<15, KP_RP_NN, 1>(wide, (int)grid, warps * 32, sm, st, prm);
-        else launch_dp_r0<15, 0, 1>(wide, (int)grid, warps * 32, sm, st, prm);
-    }
-    p->launches++;
+    launch_rows(p, s->replicate ? 2 : 1, wide, wave_geom(p, wide, hi - lo), prm, st);
     KP_CUDA(cudaGetLastError());
     return 0;
 }
@@ -1459,40 +1471,16 @@ int kp_shard_cv_heldout(kp_shard *s, const int64_t *d_expMtot, const int64_t *d_
     if (!s || !d_expMtot || !d_expUtot || !d_expMtest || !d_expUtest || !d_ws || !h_top)
         return fail("kp_shard_cv_heldout: null argument");
     kp_plan *p = s->plan;
-    if (p->host.t.total_level > 64) return fail("kp_shard_cv_heldout: more than 64 levels");
     if (root == UINT64_MAX) root = p->host.npat - 1;
     if (root >= p->host.npat) return fail("kp_shard_cv_heldout: root out of range");
     cudaStream_t st = (cudaStream_t)stream;
     KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, sizeof(float), st)) return 1;
+    if (scratch_reserve(p, sizeof(float), st)) return KP_ERR;
     float *d_rootval = (float *)p->d_scratch;
-    unsigned long long *sorted, *keys, *ctr;
-    float *vals;
-    if (backtrack_device(p, s->view, d_ws, cap, root, st, &sorted, &keys, &vals, &ctr)) return 1;
-    kp_cv_leaf_kernel<<<p->sm_count, 128, 0, st>>>(p->d_tab, p->d_rowtab, (const long long *)d_expMtot, (const long long *)d_expUtot,
-                                                   (const long long *)d_expMtest, (const long long *)d_expUtest, alpha, beta_fold,
-                                                   penalty, sorted, ctr, cap, vals);
     kp_gather_kernel<<<1, 32, 0, st>>>(p->d_tab, p->d_rowtab, s->view, nullptr, root, 1, d_rootval);
-    p->launches += 2;
-    KP_CUDA(cudaGetLastError());
-    unsigned long long hc[2] = {0, 0};
-    int herr = 0;
-    float htrain = 0.f;
-    KP_CUDA(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(&herr, p->d_err, sizeof herr, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(&htrain, d_rootval, sizeof htrain, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    if (herr == 2) return fail("kp_shard_cv_heldout: the DP gave up waiting for a child tile (internal error)");
-    if (hc[1] || hc[0] > cap) return fail_capacity("kp_shard_cv_heldout: partition larger than the workspace capacity");
-    if (hc[0] == 0) return fail("kp_shard_cv_heldout: the backtrack produced no leaf (internal error)");
-    std::vector<unsigned long long> hk(hc[0]);
-    std::vector<float> hv(hc[0]);
-    KP_CUDA(cudaMemcpyAsync(hk.data(), keys, hc[0] * 8, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaMemcpyAsync(hv.data(), vals, hc[0] * 4, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    h_top[0] = htrain;
-    h_top[1] = tree_sum(hk.data(), hv.data(), 0, hc[0], 0);
-    return 0;
+    p->launches++;
+    return heldout_sync(p, s->view, d_expMtot, d_expUtot, d_expMtest, d_expUtest, alpha, beta_fold, penalty, root, d_ws, cap,
+                        d_rootval, h_top, h_top + 1, st, "kp_shard_cv_heldout");
 }
 
 int kp_shard_backtrack(kp_shard *s, void *d_ws, uint64_t cap, uint64_t root, uint64_t *h_patnums, uint64_t *n_out, void *stream)
@@ -1501,19 +1489,7 @@ int kp_shard_backtrack(kp_shard *s, void *d_ws, uint64_t cap, uint64_t root, uin
     kp_plan *p = s->plan;
     if (root == UINT64_MAX) root = p->host.npat - 1;
     if (root >= p->host.npat) return fail("kp_shard_backtrack: root out of range");
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    unsigned long long *sorted, *keys, *ctr;
-    float *vals;
-    if (backtrack_device(p, s->view, d_ws, cap, root, st, &sorted, &keys, &vals, &ctr)) return 1;
-    unsigned long long hc[2] = {0, 0};
-    KP_CUDA(cudaMemcpyAsync(hc, ctr, sizeof hc, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    *n_out = hc[0];
-    if (hc[1] || hc[0] > cap) return fail_capacity("kp_shard_backtrack: partition larger than the workspace capacity");
-    KP_CUDA(cudaMemcpyAsync(h_patnums, sorted, hc[0] * 8, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return backtrack_host(p, s->view, d_ws, cap, root, h_patnums, n_out, (cudaStream_t)stream, "kp_shard_backtrack");
 }
 
 // scores / kept-whole flags / split codes of arbitrary patterns, read through the view (any rank's shard)
@@ -1521,25 +1497,7 @@ int kp_shard_gather(kp_shard *s, const uint64_t *h_patnums, uint64_t n, float *h
                     void *stream)
 {
     if (!s || !h_patnums) return fail("kp_shard_gather: null argument");
-    if (n == 0) return 0;
-    kp_plan *p = s->plan;
-    cudaStream_t st = (cudaStream_t)stream;
-    KP_CUDA(cudaSetDevice(p->device));
-    if (scratch_reserve(p, n * 16, st)) return 1;
-    unsigned long long *d_pat = (unsigned long long *)p->d_scratch;
-    float *d_val = (float *)(d_pat + n);
-    uint8_t *d_k = (uint8_t *)(d_val + n), *d_c = d_k + n;
-    KP_CUDA(cudaMemcpyAsync(d_pat, h_patnums, n * 8, cudaMemcpyHostToDevice, st));
-    const int grid = grid_for(n, 256, p->sm_count);
-    if (h_best) kp_gather_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, s->view, d_pat, 0, n, d_val);
-    if (h_kept) kp_gather_flags_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, s->view, d_pat, 0, n, d_k);
-    if (h_codes) kp_split_codes_kernel<<<grid, 256, 0, st>>>(p->d_tab, p->d_rowtab, s->view, d_pat, n, d_c);
-    KP_CUDA(cudaGetLastError());
-    if (h_best) KP_CUDA(cudaMemcpyAsync(h_best, d_val, n * 4, cudaMemcpyDeviceToHost, st));
-    if (h_kept) KP_CUDA(cudaMemcpyAsync(h_kept, d_k, n, cudaMemcpyDeviceToHost, st));
-    if (h_codes) KP_CUDA(cudaMemcpyAsync(h_codes, d_c, n, cudaMemcpyDeviceToHost, st));
-    KP_CUDA(cudaStreamSynchronize(st));
-    return 0;
+    return gather_view(s->plan, s->view, h_patnums, 0, n, h_best, h_kept, h_codes, (cudaStream_t)stream);
 }
 
 // float64 sum of the leaves' losses in the order of the recursion (s1 + s2 at every inner node; keys sorted ascending)

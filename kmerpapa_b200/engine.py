@@ -21,6 +21,19 @@ def _torch():
     return torch
 
 
+def grow_capacity(lib, what, cap, max_cap, run):
+    """run(cap) -> (return code, result) of one C ABI call whose workspace holds `cap` leaves.  While the call reports
+    KP_ERR_CAPACITY and cap < max_cap, runs it again with 8 times the capacity.  Returns the result of the call that
+    succeeded; raises KpError with the library's message otherwise."""
+    while True:
+        rc, res = run(cap)
+        if rc == 0:
+            return res
+        if rc != KP_ERR_CAPACITY or cap >= max_cap:
+            raise KpError(what + ": " + lib.kp_last_error().decode())
+        cap *= 8
+
+
 class PartitionPlan:
     """Tables, launch geometry and reusable device buffers for one general pattern on one GPU."""
 
@@ -147,18 +160,16 @@ class PartitionPlan:
         """Dense pattern numbers of the optimal partition of `root` (default: the general pattern) in the
         reference's emission order."""
         torch = _torch()
-        while True:
+
+        def run(cap):
             ws = self._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
             out = np.empty(cap, dtype=np.uint64)
             n = ctypes.c_uint64(0)
             rc = self.lib.kp_backtrack(self.handle, best.data_ptr(), kept.data_ptr(), ws.data_ptr(), cap,
                                        self.TOP if root is None else int(root), out.ctypes.data, ctypes.byref(n), self._stream())
-            if rc == 0:
-                return out[: n.value].copy()
-            if rc == KP_ERR_CAPACITY and cap < self.MAX_CAP:
-                cap *= 8
-                continue
-            raise KpError("kp_backtrack: " + self.lib.kp_last_error().decode())
+            return rc, out[: n.value]
+
+        return grow_capacity(self.lib, "kp_backtrack", cap, self.MAX_CAP, run).copy()
 
     def split_codes(self, best, kept, patnums):
         """The reference's backtrack pointer as position*8+split codes (0xFF: kept whole)."""
@@ -178,18 +189,15 @@ class PartitionPlan:
         train = self._buffer("cvtrain", n, torch.float32)
         kept = self._buffer("cvkept", int(self.info.kept_elems), torch.int16)
         top = (ctypes.c_float * 2)()
-        while True:
+
+        def run(cap):
             ws = self._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
-            rc = self.lib.kp_dp_cv_job(self.handle, eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(),
-                                       int(max_count), float(alpha), float(beta), float(penalty),
-                                       train.data_ptr(), kept.data_ptr(), ws.data_ptr(), cap,
-                                       ctypes.cast(top, ctypes.c_void_p) if read_top else None, self._stream())
-            if rc == 0:
-                break
-            if rc == KP_ERR_CAPACITY and cap < self.MAX_CAP:
-                cap *= 8
-                continue
-            raise KpError("kp_dp_cv_job: " + self.lib.kp_last_error().decode())
+            return self.lib.kp_dp_cv_job(self.handle, eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(),
+                                         int(max_count), float(alpha), float(beta), float(penalty),
+                                         train.data_ptr(), kept.data_ptr(), ws.data_ptr(), cap,
+                                         ctypes.cast(top, ctypes.c_void_p) if read_top else None, self._stream()), None
+
+        grow_capacity(self.lib, "kp_dp_cv_job", cap, self.MAX_CAP, run)
         self._cv_state = (eMtot, eUtot, eMte, eUte, float(alpha), float(beta), float(penalty))
         if not read_top:
             return train, kept
@@ -239,17 +247,15 @@ class PartitionPlan:
             raise KpError("cv_heldout: no cv_job has run on this plan yet")
         eMtot, eUtot, eMte, eUte, alpha, beta, penalty = self._cv_state
         out = ctypes.c_float(0)
-        while True:
+
+        def run(cap):
             ws = self._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
-            rc = self.lib.kp_cv_heldout(self.handle, self._buf["cvtrain"].data_ptr(), self._buf["cvkept"].data_ptr(),
-                                        eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(), alpha, beta, penalty,
-                                        int(root), ws.data_ptr(), cap, ctypes.byref(out), self._stream())
-            if rc == 0:
-                return np.float32(out.value)
-            if rc == KP_ERR_CAPACITY and cap < self.MAX_CAP:
-                cap *= 8
-                continue
-            raise KpError("kp_cv_heldout: " + self.lib.kp_last_error().decode())
+            return self.lib.kp_cv_heldout(self.handle, self._buf["cvtrain"].data_ptr(), self._buf["cvkept"].data_ptr(),
+                                          eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(), alpha, beta,
+                                          penalty, int(root), ws.data_ptr(), cap, ctypes.byref(out), self._stream()), None
+
+        grow_capacity(self.lib, "kp_cv_heldout", cap, self.MAX_CAP, run)
+        return np.float32(out.value)
 
     # -- output stage ----------------------------------------------------------------------------
     def pattern_counts(self, kM, kU, patnums):

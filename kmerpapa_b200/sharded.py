@@ -16,8 +16,8 @@ import ctypes
 import numpy as np
 
 from . import _native
-from ._native import KP_ERR_CAPACITY, KpError, check
-from .engine import _torch
+from ._native import KpError, check
+from .engine import _torch, grow_capacity
 
 
 def assignment(plan, world):
@@ -201,33 +201,29 @@ class ShardedDP:
         """(train, held-out) loss of `root` after the last wave of a CV job (this rank only, reads the peers' tables)."""
         torch = _torch()
         top = (ctypes.c_float * 2)()
-        while True:
+
+        def run(cap):
             ws = self.plan._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
-            rc = self.lib.kp_shard_cv_heldout(self.handle, eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(), eUte.data_ptr(),
-                                              float(alpha), float(beta), float(penalty),
-                                              self.plan.TOP if root is None else int(root), ws.data_ptr(), cap,
-                                              ctypes.cast(top, ctypes.c_void_p), self.plan._stream())
-            if rc == 0:
-                return np.float32(top[0]), np.float32(top[1])
-            if rc == KP_ERR_CAPACITY and cap < self.plan.MAX_CAP:
-                cap *= 8
-                continue
-            raise KpError("kp_shard_cv_heldout: " + self.lib.kp_last_error().decode())
+            return self.lib.kp_shard_cv_heldout(self.handle, eMtot.data_ptr(), eUtot.data_ptr(), eMte.data_ptr(),
+                                                eUte.data_ptr(), float(alpha), float(beta), float(penalty),
+                                                self.plan.TOP if root is None else int(root), ws.data_ptr(), cap,
+                                                ctypes.cast(top, ctypes.c_void_p), self.plan._stream()), None
+
+        grow_capacity(self.lib, "kp_shard_cv_heldout", cap, self.plan.MAX_CAP, run)
+        return np.float32(top[0]), np.float32(top[1])
 
     def backtrack(self, cap=65536, root=None):
         torch = _torch()
-        while True:
+
+        def run(cap):
             ws = self.plan._buffer("btws", int(self.lib.kp_backtrack_ws_bytes(cap)), torch.uint8)
             out = np.empty(cap, dtype=np.uint64)
             n = ctypes.c_uint64(0)
             rc = self.lib.kp_shard_backtrack(self.handle, ws.data_ptr(), cap, self.plan.TOP if root is None else int(root),
                                              out.ctypes.data, ctypes.byref(n), self.plan._stream())
-            if rc == 0:
-                return out[: n.value].copy()
-            if rc == KP_ERR_CAPACITY and cap < self.plan.MAX_CAP:
-                cap *= 8
-                continue
-            raise KpError("kp_shard_backtrack: " + self.lib.kp_last_error().decode())
+            return rc, out[: n.value]
+
+        return grow_capacity(self.lib, "kp_shard_backtrack", cap, self.plan.MAX_CAP, run).copy()
 
     def gather(self, patnums, codes=False):
         """(scores, kept-whole flags[, split codes]) of arbitrary patterns, wherever they are stored."""

@@ -151,6 +151,12 @@ def test_cv_jobs_against_reference_tables(eng, oracle, path):
                     ref_te = g["last_test_table"][:, f]
                 else:
                     _, ref_te = oracle.cv_job(gp, Mtot, Utot, Mf[:, f], Uf[:, f], alpha, betas[f], pen)
+                ref_top = ref_tr[-1].tobytes(), ref_te[-1].tobytes()
+                # a one-leaf workspace: the synchronous and the pipelined job go through the capacity retry
+                top = plan.cv_job(tot[0], tot[1], fold[0], fold[1], mc, alpha, betas[f], pen, cap=1)
+                assert (top[0].tobytes(), top[1].tobytes()) == ref_top
+                top = plan.cv_job_result(plan.cv_job_submit(tot[0], tot[1], fold[0], fold[1], mc, alpha, betas[f], pen, cap=1))
+                assert (top[0].tobytes(), top[1].tobytes()) == ref_top
                 for wide_mc in (mc, 1 << 40):
                     top = plan.cv_job(tot[0], tot[1], fold[0], fold[1], wide_mc, alpha, betas[f], pen)
                     # train table: every cell; held-out loss: the general pattern (all the reference reads) ...
@@ -160,6 +166,7 @@ def test_cv_jobs_against_reference_tables(eng, oracle, path):
                 rng = np.random.default_rng(gi * 31 + f)
                 for root in rng.choice(plan.npat, size=min(40, plan.npat), replace=False):
                     assert plan.cv_heldout(int(root)).tobytes() == ref_te[root].tobytes()
+                assert plan.cv_heldout(plan.npat - 1, cap=1).tobytes() == ref_te[-1].tobytes()
             gi += 1
 
 

@@ -37,6 +37,7 @@ def test_sharded_equals_unsharded(gen_pat, world, replicate):
     alpha, penalty = 1.0, 4.0
     best, kept = plan.dp_single(eM, eU, mc, alpha, beta, penalty)
     ref_part = plan.backtrack(best, kept)
+    assert np.array_equal(plan.backtrack(best, kept, cap=1), ref_part)   # through the capacity retry
     rng = np.random.default_rng(5)
     pats = np.unique(np.concatenate([rng.integers(0, plan.npat, size=20000, dtype=np.uint64),
                                      np.array([0, plan.npat - 1], dtype=np.uint64), ref_part]))
@@ -58,6 +59,7 @@ def test_sharded_equals_unsharded(gen_pat, world, replicate):
             assert s.top_score() == top
             part = s.backtrack()
             assert np.array_equal(part, ref_part)
+            assert np.array_equal(s.backtrack(cap=1), ref_part)
             vals, flags, codes = s.gather(pats, codes=True)
             assert np.array_equal(codes, ref_codes)
             assert np.array_equal(vals[:50], ref_vals)
