@@ -254,6 +254,18 @@ int kp_snv_counts(kp_plan *plan, const uint8_t *d_seq, uint64_t seq_base, uint64
                   uint64_t pos1, int both, const int64_t *d_pos, const uint8_t *d_ref_alt, uint64_t n, const int *alt_slot,
                   const uint32_t *d_count_mask, int64_t *d_counts, uint8_t *d_status, void *stream);
 
+/* Counting the SNVs of several models per region (DESIGN §4e; kmerpapa_b200/burden.py).  The n SNVs of one record are
+ * at d_pos (int64, sorted ascending) and d_model[t] (uint8) is the model that counts SNV t; an id >= nmodels (255: none)
+ * counts for no model.  nmodels is 1..255.  For region r = d_regions[2r..2r+1] = (start, end), half-open in the
+ * coordinates of d_pos, d_observed[r * nmodels + m] (int64) = the SNVs t with start <= d_pos[t] < end and d_model[t] = m.
+ * Regions may overlap and come in any order; one with end <= start counts nothing.  A per-model prefix count over the
+ * SNVs (a three-pass block scan) makes each region cost two binary searches and nmodels differences, whatever its
+ * length.  d_ws: device workspace of kp_snv_region_ws_bytes(n, nmodels) bytes; d_pos, d_regions, d_ws and d_observed
+ * are 8-byte aligned.  The counts are integers, the same on every run.  Does not synchronise. */
+uint64_t kp_snv_region_ws_bytes(uint64_t n, int nmodels);
+int kp_snv_region_counts(kp_plan *plan, const int64_t *d_pos, const uint8_t *d_model, uint64_t n, int nmodels,
+                         const int64_t *d_regions, uint64_t nreg, void *d_ws, int64_t *d_observed, void *stream);
+
 /* Where a dense pattern number lives in the device layout: element of a float table, element and bit of d_kept. */
 int kp_pattern_offset(const kp_plan *plan, uint64_t patnum, uint64_t *table_elem, uint64_t *kept_elem, uint32_t *kept_bit);
 

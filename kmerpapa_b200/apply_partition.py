@@ -159,15 +159,17 @@ def region_tasks(starts, ends, rec_len):
 
 class ApplyResult:
     """Per region (input order; per record without regions): chrom, start, end, n_contexts (int64), expected
-    (float64).  tracks: {name: float32 array} when asked for; counts: int64 per k-mer of gen_pat in k-mer index order
-    when asked for."""
+    (float64); model_n_contexts and model_expected hold them for every model of Applier.add_model, [model, region],
+    the first model's row being n_contexts / expected.  tracks: {name: float32 array} when asked for; counts: int64 per
+    k-mer of gen_pat in k-mer index order when asked for."""
 
     def __init__(self, **kw):
         self.__dict__.update(kw)
 
 
 class Applier:
-    """Streams records through the scan: one plan, the device rate table, double-buffered pinned uploads."""
+    """Streams records through the scan: a plan and a device rate table per model (one model unless add_model is
+    called), double-buffered pinned uploads."""
 
     def __init__(self, patterns, rates, regions=None, strand="forward", track=False, kmer_counts=False, device=None,
                  chunk_bases=CHUNK_BASES):
@@ -188,6 +190,7 @@ class Applier:
         self.k, self.c, self.both, self.track, self.chunk = k, k // 2, strand == "both", bool(track), int(chunk_bases)
         self.torch, self.dev = torch, self.plan.device
         self.kmer_rate = self.plan.kmer_rates(owner, rates)
+        self.scans = [(self.plan, self.kmer_rate)]   # (plan, device rate table) per model
         self.counts = torch.zeros(self.plan.nkmer, dtype=torch.int64, device=self.dev) if kmer_counts else None
         self.regions = None
         if regions is not None:
@@ -197,7 +200,7 @@ class Applier:
             for i, r in enumerate(regions):
                 self.by_chrom.setdefault(r[0], []).append(i)
             n = len(regions)
-            self.n_contexts, self.expected = np.zeros(n, np.int64), np.zeros(n, np.float64)
+            self.n_contexts, self.expected = np.zeros((1, n), np.int64), np.zeros((1, n), np.float64)
         else:
             self.rows = []
         self.names = set()
@@ -208,6 +211,29 @@ class Applier:
         self.dmask = [torch.empty(self.chunk // 32, dtype=torch.int32, device=self.dev) for _ in range(2)]
         self.ev = [None, None]
         self.nchunks = 0
+
+    def add_model(self, patterns, rates):
+        """Scan one more partition of the same k with the first, from the same uploaded bytes: kp_seq_scan and
+        kp_region_sums run once per model on its own plan (shared by models of one general pattern) and rate table.
+        Returns (model index, general pattern, plan).  Call it before the first record, on an Applier without tracks
+        and k-mer counts.  Raises PartitionError as the constructor does."""
+        if self.track or self.counts is not None:
+            raise InputError("tracks and k-mer counts are of one partition only")
+        if self.nchunks or self.names:
+            raise InputError("add every model before the first record")
+        rates = np.ascontiguousarray(rates, dtype=np.float64)
+        if len(rates) != len(patterns):
+            raise InputError("one rate per pattern")
+        if len(patterns[0]) != self.k:
+            raise InputError(f"every partition needs the same k ({self.k}), not {len(patterns[0])}")
+        gen_pat, plan, _, owner = assign(patterns, self.dev.index)
+        m = len(self.scans)
+        self.scans.append((plan, plan.kmer_rates(owner, rates, name=f"apply{m}")))
+        if self.regions is not None:
+            n = len(self.regions)
+            self.n_contexts = np.concatenate([self.n_contexts, np.zeros((1, n), np.int64)])
+            self.expected = np.concatenate([self.expected, np.zeros((1, n), np.float64)])
+        return m, gen_pat, plan
 
     def record(self, name, seq, on_chunk=None):
         """Scan one record.  Returns its float32 track (numpy) when tracks are asked for, else None.  A record that has
@@ -238,21 +264,21 @@ class Applier:
             out = self._scan(seq, L, starts, ends, on_chunk)
         if self.regions is not None:
             if len(idx):
-                self.n_contexts[idx], self.expected[idx] = out[0], out[1]
+                self.n_contexts[:, idx], self.expected[:, idx] = out[0], out[1]
         else:
-            self.rows.append((name, 0, L, int(out[0][0]), float(out[1][0])))
+            self.rows.append((name, 0, L, out[0][:, 0], out[1][:, 0]))
         return out[2]
 
     def _scan(self, seq, L, starts, ends, on_chunk):
-        torch, plan, P = self.torch, self.plan, PIECE
+        torch, P, nm = self.torch, PIECE, len(self.scans)
         stream = torch.cuda.current_stream(self.dev)
         npieces = (L + P - 1) // P
-        psum = torch.empty(max(npieces, 1), dtype=torch.float64, device=self.dev)
-        pn = torch.empty(max(npieces, 1), dtype=torch.int64, device=self.dev)
+        psum = torch.empty((nm, max(npieces, 1)), dtype=torch.float64, device=self.dev)
+        pn = torch.empty((nm, max(npieces, 1)), dtype=torch.int64, device=self.dev)
         tasks, reg = region_tasks(starts, ends, L) if len(starts) else (np.zeros((0, 3), np.uint32), np.zeros((0, 4), np.int64))
         dtasks = torch.from_numpy(tasks.view(np.int32)).to(self.dev) if len(tasks) else None
-        tsum = torch.empty(max(len(tasks), 1), dtype=torch.float64, device=self.dev)
-        tn = torch.empty(max(len(tasks), 1), dtype=torch.int64, device=self.dev)
+        tsum = torch.empty((nm, max(len(tasks), 1)), dtype=torch.float64, device=self.dev)
+        tn = torch.empty((nm, max(len(tasks), 1)), dtype=torch.int64, device=self.dev)
         track = torch.empty(L, dtype=torch.float32, device=self.dev) if self.track else None
         masked = self.counts is not None and self.regions is not None
         if masked:
@@ -274,13 +300,14 @@ class Applier:
                 self.pmask[slot].numpy()[: len(words)] = words.view(np.int32)
                 mask = self.dmask[slot][: len(words)]
                 mask.copy_(self.pmask[slot][: len(words)], non_blocking=True)
-            plan.seq_scan(self.dseq[slot], b0, b1 - b0, L, pos0, pos1, self.kmer_rate, self.both, psum[pos0 // P:],
-                          pn[pos0 // P:], track=track[pos0:pos1] if track is not None else None, count_mask=mask,
-                          counts=self.counts)
             t0, t1 = np.searchsorted(tpiece, pos0 // P), np.searchsorted(tpiece, (pos1 + P - 1) // P)
-            if t1 > t0:
-                plan.seq_scan(self.dseq[slot], b0, b1 - b0, L, pos0, pos1, self.kmer_rate, self.both, tsum[t0:], tn[t0:],
-                              tasks=dtasks[t0:t1])
+            for m, (plan, kmer_rate) in enumerate(self.scans):
+                plan.seq_scan(self.dseq[slot], b0, b1 - b0, L, pos0, pos1, kmer_rate, self.both, psum[m, pos0 // P:],
+                              pn[m, pos0 // P:], track=track[pos0:pos1] if track is not None else None, count_mask=mask,
+                              counts=self.counts)
+                if t1 > t0:
+                    plan.seq_scan(self.dseq[slot], b0, b1 - b0, L, pos0, pos1, kmer_rate, self.both, tsum[m, t0:],
+                                  tn[m, t0:], tasks=dtasks[t0:t1])
             if on_chunk is not None:
                 on_chunk(self.dseq[slot], b0, b1, pos0, pos1, mask)
             ev = torch.cuda.Event()
@@ -289,9 +316,11 @@ class Applier:
         res_n = res_s = None
         if len(reg):
             dreg = torch.from_numpy(reg).to(self.dev)
-            osum = torch.empty(len(reg), dtype=torch.float64, device=self.dev)
-            on = torch.empty(len(reg), dtype=torch.int64, device=self.dev)
-            plan.region_sums(psum, pn, tsum if len(tasks) else None, tn if len(tasks) else None, dreg, osum, on)
+            osum = torch.empty((nm, len(reg)), dtype=torch.float64, device=self.dev)
+            on = torch.empty((nm, len(reg)), dtype=torch.int64, device=self.dev)
+            for m, (plan, _) in enumerate(self.scans):
+                plan.region_sums(psum[m], pn[m], tsum[m] if len(tasks) else None, tn[m] if len(tasks) else None, dreg,
+                                 osum[m], on[m])
             res_n, res_s = on.cpu().numpy(), osum.cpu().numpy()
         return res_n, res_s, track.cpu().numpy() if track is not None else None
 
@@ -310,11 +339,12 @@ class Applier:
             chrom = [r[0] for r in self.rows]
             start = np.array([r[1] for r in self.rows], np.int64)
             end = np.array([r[2] for r in self.rows], np.int64)
-            n_contexts = np.array([r[3] for r in self.rows], np.int64)
-            expected = np.array([r[4] for r in self.rows], np.float64)
+            nm = len(self.scans)
+            n_contexts = np.ascontiguousarray(np.array([r[3] for r in self.rows], np.int64).reshape(-1, nm).T)
+            expected = np.ascontiguousarray(np.array([r[4] for r in self.rows], np.float64).reshape(-1, nm).T)
         counts = self.counts.cpu().numpy() if self.counts is not None else None
-        return ApplyResult(gen_pat=self.gen_pat, k=self.k, chrom=chrom, start=start, end=end, n_contexts=n_contexts,
-                           expected=expected, counts=counts)
+        return ApplyResult(gen_pat=self.gen_pat, k=self.k, chrom=chrom, start=start, end=end, n_contexts=n_contexts[0],
+                           expected=expected[0], model_n_contexts=n_contexts, model_expected=expected, counts=counts)
 
 
 def apply(patterns, rates, records, regions=None, strand="forward", track=False, kmer_counts=False, device=None,

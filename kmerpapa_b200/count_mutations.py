@@ -221,13 +221,13 @@ class CountResult:
 
 
 class _Counter:
-    """The per-record SNV state of count_mutations: the record's SNVs sorted by position on the device and the
-    on_chunk hook that counts those of each chunk."""
+    """The per-record SNV state of count_mutations (a snv_pass hook): the record's SNVs sorted by position on the
+    device and the on_chunk hook that counts those of each chunk."""
 
     def __init__(self, ap, snvs, slot, counts):
         self.ap, self.snvs, self.slot, self.counts = ap, snvs, slot, counts
 
-    def start(self, idx, L):
+    def start(self, name, idx, L):
         torch, dev = self.ap.torch, self.ap.dev
         self.L = L
         self.pos = self.snvs.pos[idx]
@@ -244,17 +244,19 @@ class _Counter:
             self.ap.plan.snv_counts(dseq, b0, b1 - b0, self.L, pos0, pos1, self.ap.both, self.dpos[lo:hi], self.dra[lo:hi],
                                     self.slot, self.counts, self.dstatus[lo:hi], count_mask=mask)
 
+    def finish(self, name):
+        return self.dstatus.cpu().numpy()
 
-def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts=None, device=None,
-                    chunk_bases=CHUNK_BASES):
-    """Background and positive k-mer counts of gen_pat over records, an iterable of (name, bytes) pairs, and the SNVs
-    snvs (Snvs, as read_vcf returns).  regions: None (whole records) or (chrom, start, end[, where]) tuples; alts: None
-    (one table of every SNV) or ALT letters (one table each).  chunk_bases (a multiple of 65536) changes no result.
-    Returns a CountResult; see the module docstring for the conventions.  Raises InputError on bad input."""
-    labels, slot = check_args(gen_pat, strand, alts)
-    ap = Applier([gen_pat], [0.0], regions, strand, kmer_counts=True, device=device, chunk_bases=chunk_bases)
-    torch = ap.torch
-    counts = torch.zeros((len(labels), ap.plan.nkmer), dtype=torch.int64, device=ap.dev)
+
+def snv_pass(ap, records, snvs, hook):
+    """The record loop of count_mutations and burden: stream records, an iterable of (name, bytes) pairs, through the
+    Applier ap with the SNV alleles snvs (Snvs).  Per record, hook.start(name, idx, L) gets the indices of the record's
+    SNVs that lie inside it, sorted by position; ap.record(name, seq, on_chunk=hook) scans the record, and the hook sets
+    hook.scanned when a chunk was scanned; then hook.finish(name) returns the uint8 status of those SNVs.  The status
+    codes are the caller's, except that REF_MISMATCH, OUTSIDE_REGIONS and BAD_POSITION mean what they mean in STATUS:
+    SNVs of a record that is not scanned are OUTSIDE_REGIONS.  Returns (status of every SNV, ap.finish()).  Raises
+    InputError after the pass for an unknown CHROM, a POS past the end of its record and a REF mismatch, in that order,
+    and AssertionError when a scanned SNV is left BAD_POSITION."""
     n = len(snvs)
     status = np.full(n, BAD_POSITION, np.uint8)
     dc = np.diff(snvs.chrom)
@@ -264,7 +266,6 @@ def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts
         order = np.lexsort((snvs.pos, snvs.chrom))
     bounds = np.searchsorted(snvs.chrom[order], np.arange(len(snvs.chroms) + 1))
     chrom_of = {nm: i for i, nm in enumerate(snvs.chroms)}
-    cnt = _Counter(ap, snvs, slot, counts)
     past_end, mismatch, seen = [], [], set()
     for name, seq in records:
         if isinstance(seq, str):
@@ -277,12 +278,12 @@ def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts
         if over.any():
             past_end.append(idx[over])
             idx = idx[~over]
-        cnt.start(idx, L)
-        ap.record(name, seq, on_chunk=cnt)
-        if not cnt.scanned:
+        hook.start(name, idx, L)
+        ap.record(name, seq, on_chunk=hook)
+        if not hook.scanned:
             status[idx] = OUTSIDE_REGIONS
             continue
-        st = cnt.dstatus.cpu().numpy()
+        st = hook.finish(name)
         if (st == BAD_POSITION).any():
             raise AssertionError("kp_snv_counts left an SNV of a scanned record uncounted")
         status[idx] = st
@@ -290,7 +291,7 @@ def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts
         if len(bad):
             j = bad[np.argmin(snvs.line[bad])]
             mismatch.append((int(snvs.line[j]), name, int(snvs.pos[j]), seq[snvs.pos[j]: snvs.pos[j] + 1].decode(), j))
-    bg = ap.finish().counts
+    res = ap.finish()
     where = snvs.name
     lost = [i for i in range(len(snvs.chroms)) if i not in seen]
     if lost:   # every CHROM of the VCF, also one whose lines have no SNV allele
@@ -306,8 +307,22 @@ def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts
         total = int((status == REF_MISMATCH).sum())
         raise InputError(f"{where}:{line}: REF {'ACGT'[snvs.ref[j]]} does not match the genome base {base} at "
                          f"{name}:{pos + 1}; {total} SNV alleles mismatch in all (is the VCF from another genome build?)")
+    return status, res
+
+
+def count_mutations(gen_pat, records, snvs, regions=None, strand="forward", alts=None, device=None,
+                    chunk_bases=CHUNK_BASES):
+    """Background and positive k-mer counts of gen_pat over records, an iterable of (name, bytes) pairs, and the SNVs
+    snvs (Snvs, as read_vcf returns).  regions: None (whole records) or (chrom, start, end[, where]) tuples; alts: None
+    (one table of every SNV) or ALT letters (one table each).  chunk_bases (a multiple of 65536) changes no result.
+    Returns a CountResult; see the module docstring for the conventions.  Raises InputError on bad input."""
+    labels, slot = check_args(gen_pat, strand, alts)
+    ap = Applier([gen_pat], [0.0], regions, strand, kmer_counts=True, device=device, chunk_bases=chunk_bases)
+    torch = ap.torch
+    counts = torch.zeros((len(labels), ap.plan.nkmer), dtype=torch.int64, device=ap.dev)
+    status, res = snv_pass(ap, records, snvs, _Counter(ap, snvs, slot, counts))
     hist = np.bincount(status, minlength=len(STATUS))
-    return CountResult(gen_pat=gen_pat, k=len(gen_pat), alts=labels, background=bg, positive=counts.cpu().numpy(),
+    return CountResult(gen_pat=gen_pat, k=len(gen_pat), alts=labels, background=res.counts, positive=counts.cpu().numpy(),
                        status=status, status_counts={s: int(hist[i]) for i, s in enumerate(STATUS)},
                        skipped=snvs.skipped)
 

@@ -1087,6 +1087,46 @@ int kp_region_sums(kp_plan *p, const double *d_piece_sum, const int64_t *d_piece
     return 0;
 }
 
+// blocks of scan passes 1 and 3 for n SNVs
+static uint64_t snv_scan_blocks(uint64_t n)
+{
+    return std::max<uint64_t>(1, std::min<uint64_t>(KP_SNV_SCAN_BLOCKS, (n + 255) / 256));
+}
+
+uint64_t kp_snv_region_ws_bytes(uint64_t n, int nmodels)
+{
+    if (nmodels < 1) return 0;
+    return ((n + 1) * nmodels + (snv_scan_blocks(n) + 1) * nmodels) * 8;
+}
+
+int kp_snv_region_counts(kp_plan *p, const int64_t *d_pos, const uint8_t *d_model, uint64_t n, int nmodels,
+                         const int64_t *d_regions, uint64_t nreg, void *d_ws, int64_t *d_observed, void *stream)
+{
+    if (!p) return fail("kp_snv_region_counts: null plan");
+    if (nmodels < 1 || nmodels > 255) return fail("kp_snv_region_counts: nmodels must be 1..255");
+    if (nreg == 0) return 0;
+    if (!d_regions || !d_observed || !d_ws || (n && (!d_pos || !d_model))) return fail("kp_snv_region_counts: null argument");
+    if (((uintptr_t)d_pos & 7) || ((uintptr_t)d_regions & 7) || ((uintptr_t)d_ws & 7) || ((uintptr_t)d_observed & 7))
+        return fail("kp_snv_region_counts: d_pos, d_regions, d_ws and d_observed must be 8-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    KP_CUDA(cudaSetDevice(p->device));
+    unsigned long long *pre = (unsigned long long *)d_ws, *bsum = pre + (n + 1) * nmodels, *tot = bsum + snv_scan_blocks(n) * nmodels;
+    KP_CUDA(cudaMemsetAsync(pre, 0, nmodels * 8, st));
+    if (n) {
+        const uint64_t nb = snv_scan_blocks(n), per = (n + nb - 1) / nb;
+        kp_snv_prefix_prep_kernel<<<(unsigned)nb, 256, 0, st>>>(d_model, n, nmodels, per, bsum);
+        for (int m = 0; m < nmodels; m++) kp_part_scan_kernel<<<1, 256, 0, st>>>(bsum + m * nb, (unsigned)nb, tot + m, 0);
+        kp_snv_prefix_kernel<<<(unsigned)nb, 256, 0, st>>>(d_model, n, nmodels, per, bsum, pre);
+        p->launches += 2 + nmodels;
+    }
+    kp_snv_region_kernel<<<grid_for(nreg, 256, p->sm_count), 256, 0, st>>>((const long long *)d_pos, n, nmodels, pre,
+                                                                           (const long long *)d_regions, nreg,
+                                                                           (unsigned long long *)d_observed);
+    p->launches++;
+    KP_CUDA(cudaGetLastError());
+    return 0;
+}
+
 // ===================================================================================================
 // One DP sharded over the GPUs of a node (SURVEY 8f.3).  The score table is split by the digit of the top high
 // position; every rank runs the same waves on its own tiles and reads the children that live on a peer straight

@@ -2099,6 +2099,91 @@ __global__ void kp_region_sum_kernel(const double *psum, const unsigned long lon
     }
 }
 
+// Counting the SNVs of several models per region (kp_snv_region_counts, DESIGN §4e).  The SNVs of one record are sorted
+// by position and carry a model id; pre[j][m] (int64 [n + 1][nm]) = the SNVs among the first j with id m, built by a
+// three-pass block scan (pass 2 is kp_part_scan_kernel, once per model).  A region [start, end) holds the SNVs
+// [lower_bound(start), lower_bound(end)), so its count of model m is the difference of two rows of pre, whatever its
+// length.  Every value is an integer: the same on every run.
+#define KP_SNV_SCAN_BLOCKS 2048   // most blocks of scan passes 1 and 3
+
+// scan pass 1: bsum[m * nb + b] = the SNVs of model m among [b * per, (b + 1) * per); an id >= nm counts for no model
+__global__ void __launch_bounds__(256) kp_snv_prefix_prep_kernel(const uint8_t *model, unsigned long long n, int nm,
+                                                                 unsigned long long per, unsigned long long *bsum)
+{
+    __shared__ unsigned int s_cnt[256];
+    s_cnt[threadIdx.x] = 0;
+    __syncthreads();
+    const unsigned long long lo = blockIdx.x * per, hi = min(n, lo + per);
+    for (unsigned long long base = lo; base < hi; base += blockDim.x) {
+        const unsigned long long j = base + threadIdx.x;
+        const unsigned id = j < hi ? model[j] : 255u;
+        const unsigned peers = __match_any_sync(0xFFFFFFFFu, id);   // one shared atomic per id present in the warp
+        if (id < (unsigned)nm && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&s_cnt[id], __popc(peers));
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < nm) bsum[threadIdx.x * (unsigned long long)gridDim.x + blockIdx.x] = s_cnt[threadIdx.x];
+}
+
+// scan pass 3: rows 1..n of pre (row 0 is zeroed by the caller); bsum holds pass 2's exclusive sums over the blocks.
+// Per 256-SNV tile: each warp counts every model with a ballot, thread m turns the 8 warp counts into exclusive prefixes
+// plus the running carry of model m, and each SNV's row adds the count of its own warp's lanes up to it.
+__global__ void __launch_bounds__(256) kp_snv_prefix_kernel(const uint8_t *model, unsigned long long n, int nm,
+                                                            unsigned long long per, const unsigned long long *bsum,
+                                                            unsigned long long *pre)
+{
+    __shared__ unsigned int s_warp[8][256];
+    __shared__ unsigned long long s_pre[8][256];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const unsigned upto = 0xFFFFFFFFu >> (31 - lane);
+    unsigned long long carry = (int)threadIdx.x < nm ? bsum[threadIdx.x * (unsigned long long)gridDim.x + blockIdx.x] : 0;
+    const unsigned long long lo = blockIdx.x * per, hi = min(n, lo + per);
+    for (unsigned long long base = lo; base < hi; base += blockDim.x) {
+        const unsigned long long j = base + threadIdx.x;
+        const unsigned id = j < hi ? model[j] : 255u;
+        for (int m = 0; m < nm; m++) {
+            const unsigned b = __ballot_sync(0xFFFFFFFFu, id == (unsigned)m);
+            if (lane == 0) s_warp[w][m] = __popc(b);
+        }
+        __syncthreads();
+        if ((int)threadIdx.x < nm) {
+            for (int x = 0; x < 8; x++) {
+                s_pre[x][threadIdx.x] = carry;
+                carry += s_warp[x][threadIdx.x];
+            }
+        }
+        __syncthreads();
+        for (int m = 0; m < nm; m++) {
+            const unsigned b = __ballot_sync(0xFFFFFFFFu, id == (unsigned)m);
+            if (j < hi) pre[(j + 1) * nm + m] = s_pre[w][m] + __popc(b & upto);
+        }
+        // the next tile writes s_warp before its first barrier and s_pre after it, when every row above is stored
+    }
+}
+
+// first j in [0, n) with pos[j] >= x, n when there is none
+__device__ __forceinline__ unsigned long long kp_lower_bound(const long long *pos, unsigned long long n, long long x)
+{
+    unsigned long long lo = 0, hi = n;
+    while (lo < hi) {
+        const unsigned long long mid = lo + (hi - lo) / 2;
+        if (pos[mid] < x) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// region r = (start, end) of reg[2r..2r+1]: out[r * nm + m] = the SNVs of model m with start <= pos < end
+__global__ void __launch_bounds__(256) kp_snv_region_kernel(const long long *pos, unsigned long long n, int nm,
+                                                            const unsigned long long *pre, const long long *reg,
+                                                            unsigned long long nreg, unsigned long long *out)
+{
+    for (unsigned long long r = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; r < nreg;
+         r += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned long long a = kp_lower_bound(pos, n, reg[2 * r]);
+        const unsigned long long b = max(a, kp_lower_bound(pos, n, reg[2 * r + 1]));
+        for (int m = 0; m < nm; m++) out[r * nm + m] = pre[b * nm + m] - pre[a * nm + m];
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // test hooks
 // ---------------------------------------------------------------------------------------------------

@@ -340,6 +340,21 @@ class PartitionPlan:
                                      count_mask.data_ptr() if count_mask is not None else None, counts.data_ptr(),
                                      status.data_ptr(), self._stream()), "kp_snv_counts")
 
+    def snv_region_counts(self, pos, model, nmodels, regions, observed):
+        """One kp_snv_region_counts call on the stream, without waiting.  pos: int64 device tensor of one record's SNV
+        positions, sorted; model: uint8 device tensor, the model id of each SNV (>= nmodels: none); regions: int64 device
+        tensor [r, 2] of (start, end); observed: int64 device tensor [r, nmodels], overwritten."""
+        torch = _torch()
+        n, nreg = int(pos.shape[0]), int(regions.shape[0])
+        if model.shape[0] != n:
+            raise ValueError("pos and model need one entry per SNV")
+        if tuple(observed.shape) != (nreg, nmodels) or not observed.is_contiguous() or not regions.is_contiguous():
+            raise ValueError("observed must be a contiguous [regions, nmodels] tensor and regions contiguous")
+        ws = self._buffer("snv_region_ws", int(self.lib.kp_snv_region_ws_bytes(n, int(nmodels))), torch.uint8)
+        check(self.lib.kp_snv_region_counts(self.handle, pos.data_ptr() if n else None, model.data_ptr() if n else None, n,
+                                            int(nmodels), regions.data_ptr(), nreg, ws.data_ptr(), observed.data_ptr(),
+                                            self._stream()), "kp_snv_region_counts")
+
     def region_sums(self, piece_sum, piece_n, task_sum, task_n, regions, out_sum, out_n):
         """kp_region_sums on the stream, without waiting.  regions: int64 device tensor [n, 4]."""
         ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
